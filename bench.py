@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W           # this framework, one rank per GPU
   python bench.py --impl reference --gpus N ...            # the reference's own CPU code on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write a fixed sample of the last timed step's outputs
 
 A "step" is one full denoising of the light field: hard-threshold step then Wiener step. The noisy input is produced on the
 host by the reference's generator (mt19937ar + Box-Muller, utilities.cpp:154-185; the product's own restatement in
@@ -38,6 +39,7 @@ WORKLOAD = "configs[2]: Stanford-shaped synthetic LF 17x17 SAIs 1024x1024 RGB, s
 METRIC = "LF Mpix/s (both steps) 17x17x1024^2 RGB"
 N_PASSES = 64            # window passes per step at 17x17 with an = 1 (SURVEY.md A1)
 SEED0 = 20171016
+DUMP_SAMPLES = 1 << 22   # elements kept per dumped output: 16 MB of float32 each, three outputs at most
 
 
 def config_dict(world):
@@ -137,6 +139,15 @@ def clean_lf(aw, ah, H, W, C, seed=12345):
     return lfdata.synth_lf(aw, ah, H, W, C, seed=seed)
 
 
+def sample_outputs(torch, arrays):
+    """Host copies of the same fixed DUMP_SAMPLES flat positions (drawn without replacement from seed 0, ascending) of each
+    equally shaped device array, so that the outputs of two builds can be compared element for element."""
+    n = next(iter(arrays.values())).numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLES), replace=False, shuffle=False))
+    idx = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    return {name: t.reshape(-1)[idx].cpu().numpy() for name, t in arrays.items()}
+
+
 def host_ptrs(t, asize):
     each = t[0].numel()
     return (Cc.POINTER(Cc.c_float) * asize)(*[Cc.cast(t.data_ptr() + 4 * each * i, Cc.POINTER(Cc.c_float)) for i in range(asize)])
@@ -214,6 +225,11 @@ def run_ours(args):
     e1.record(stream)
     e1.synchronize()
     barrier()
+    # what a caller of the timed path holds after its last step, taken before the profile run below overwrites it. The team
+    # path leaves basic and the round-tripped noisy LF band-resident; only the gathered result is complete on a rank.
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = sample_outputs(torch, {"denoised": out, "basic": basic, "noisy_roundtrip": work} if team is None else {"denoised": out})
     ms = e0.elapsed_time(e1)
     st = eng.stats()
     launches = int(st.kernel_launches)
@@ -335,6 +351,10 @@ def run_ours(args):
                 "e2e": e2e, "gpu_launches": launches, "clocks": sampler.summary(), "roofline": roof, "roofline_other": roof_other, "roofline_bm": roof_bm,
                 "phases": phases, "team": team_info, "team_phases": team_phases, "cpu_baseline": cpu, "parity": parity, "psnr": psnr}
         print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if team is not None:
         team.close()
     if world > 1:
@@ -573,7 +593,15 @@ def main():
                     help="N > 1: independent windows of a plan level run concurrently, one per lane (own pass buffers, ~22 GB each)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample (%d elements each) of the outputs of the last timed step as DIR/<name>.npy, float32; "
+                         "--impl ours only (the reference arm times a smaller CPU sample, not this workload)" % DUMP_SAMPLES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        # the reference arm times a bounded, extrapolated CPU sample of another size, not the 17x17x1024^2 light field
+        ap.error("--dump-outputs writes the outputs of the 17x17x1024^2 workload, which only --impl ours computes")
     if args.impl == "reference":
         run_reference(args)
     else:

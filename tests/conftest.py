@@ -29,8 +29,9 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
+    """The unmodified reference's values: live from oracle/_ref where it is built, stored digests elsewhere (refapi.Pinned)."""
     import refapi
-    if not refapi.available():
-        pytest.skip("oracle/_ref not built (reference sources not mounted)")
-    refapi.lib()
-    return refapi
+    pins = refapi.Pinned()
+    yield pins
+    if pins.record:
+        pins.save()

@@ -1,8 +1,20 @@
 """Re-creates the inputs the golden vectors (tests/make_golden.py) were generated from."""
+import os
+
 import numpy as np
 
 import lfdata
 import oracleapi as O
+
+FIXTURE_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sourceLF")
+
+
+def config1_fixture():
+    """The reference's fixture `testing/sourceLF` (3x3 SAIs 256x256 RGB) as [9, 3, 256, 256] uint8, row-major SAI order, read
+    from its lossless copy tests/golden/sourceLF/SAI_<s>_<t>.png (s, t from 1)."""
+    from PIL import Image
+    return np.stack([np.asarray(Image.open(os.path.join(FIXTURE_DIR, "SAI_%02d_%02d.png" % (s + 1, t + 1))).convert("RGB")).transpose(2, 0, 1)
+                     for s in range(3) for t in range(3)])
 
 
 def pad_inputs(H, W, sigma, n=24):

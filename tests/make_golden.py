@@ -1,6 +1,6 @@
 """Generates tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref) in the build container.
 Inputs are re-creatable anywhere from tests/lfdata.py + the oracle's mt19937ar noise, so only outputs are stored.
-Run:  python tests/make_golden.py      (needs /root/reference mounted; see oracle/Makefile)"""
+Run:  python tests/make_golden.py      (needs oracle/_ref built from the reference's sources; see oracle/Makefile)"""
 import os
 import sys
 
@@ -64,16 +64,15 @@ def main():
     rn3, rd3 = R.pass_step1(sym, z, z, mask, proc, 4, 4, 3, 25.0, 2.7, 18, 6, 16, 1, 4, R.BIOR, R.SADCT, R.HAAR)
     out["p1bior_num"], out["p1bior_den"] = rn3[crop], rd3[crop]
     np.savez_compressed(os.path.join(GOLD, "pass_40x48.npz"), **out)
-    # 3. complete runs: 3x3 (one window pass per step) and 5x5 (five passes per step), README parameters
-    out = {}
+    # 3. complete runs: 3x3 (one window pass per step) and 5x5 (five passes per step), README parameters; one file per run
     for tag, (aw, H, W) in {"3x3": (3, 32, 40), "5x5": (5, 24, 28)}.items():
         clean = lfdata.synth_lf(aw, aw, H, W)
         noisy = O.add_noise(clean, 25.0)
         mask = np.ones(aw * aw)
         b, nrt = R.run_step1(noisy, mask, 25.0, 2.7, aw, aw, 1, 8, 18, 6, 16, 4, R.ID, R.SADCT, R.HAAR)
         d, b2, _ = R.run_step2(nrt, b, mask, 25.0, aw, aw, 1, 16, 18, 6, 8, 4, R.DCT, R.SADCT, R.HAAR)
-        out["basic_" + tag], out["noisy_rt_" + tag], out["denoised_" + tag], out["basic_rt_" + tag] = b, nrt, d, b2
-    np.savez_compressed(os.path.join(GOLD, "runs.npz"), **out)
+        out = {"basic_" + tag: b, "noisy_rt_" + tag: nrt, "denoised_" + tag: d, "basic_rt_" + tag: b2}
+        np.savez_compressed(os.path.join(GOLD, "runs_%s.npz" % tag), **out)
     # 4. partial-window branch (pst != cst): one call per step on accumulators with holes, and complete grayscale runs
     #    (several core calls per window: LF_denoised_percent stays below 100 after the first SAI when C == 1)
     _, _, sym = pad_inputs(32, 40, 25.0)

@@ -5,12 +5,16 @@ build container; it is not available where /root/reference was never mounted unl
 prebuilt .so travelled with the snapshot.
 """
 import ctypes as C
+import hashlib
+import json
 import os
+import sys
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libref_lfbm5d.so")
+PINS = os.path.join(HERE, "golden", "ref_pins.json")
 
 YUV, YCBCR, OPP, RGB, ID, DCT, SADCT, BIOR, HADAMARD, HAAR, NONE, ROWMAJOR, COLMAJOR = range(13)
 
@@ -29,6 +33,53 @@ def lib():
         _lib.ref_mt_res53.restype = C.c_double
         _lib.ref_ind_initialize.restype = C.c_uint
     return _lib
+
+
+def _values(x):
+    return tuple(x) if isinstance(x, (tuple, list)) else (x,)
+
+
+def digest(values):
+    """SHA-256 over dtype, shape and bytes of each value: equal digests mean bit-identical values."""
+    h = hashlib.sha256()
+    for v in _values(values):
+        a = np.ascontiguousarray(np.asarray(v))
+        h.update(("%s%s" % (a.dtype.str, a.shape)).encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
+class Pinned:
+    """The reference's side of the oracle-vs-reference comparisons. Where oracle/_ref is built, `check` compares with the
+    reference live. Elsewhere it compares the SHA-256 of the values under test with the digest stored in
+    tests/golden/ref_pins.json, which holds the reference's values on the same seeded inputs. With LFBM5D_RECORD_REF_PINS=1
+    the digests of the checked values are written back to that file: python -m pytest tests/test_oracle_vs_ref.py
+    tests/test_host_io.py -k "not gpu"."""
+
+    def __init__(self):
+        self.live = available()
+        self.record = os.environ.get("LFBM5D_RECORD_REF_PINS") == "1"
+        self.pins = {}
+        if os.path.exists(PINS):
+            with open(PINS) as f:
+                self.pins = json.load(f)
+
+    def check(self, key, got, want):
+        """got: the values under test (an array or a tuple of them); want(refapi): the same values computed by the reference."""
+        if self.live:
+            w = _values(want(sys.modules[__name__]))
+            g = _values(got)
+            assert len(g) == len(w) and all(np.array_equal(a, b) for a, b in zip(g, w)), key
+        if self.record:
+            self.pins[key] = digest(got)
+        elif not self.live:
+            assert key in self.pins, "no stored reference values for %s (tests/golden/ref_pins.json)" % key
+            assert digest(got) == self.pins[key], key
+
+    def save(self):
+        with open(PINS, "w") as f:
+            json.dump(self.pins, f, indent=0, sort_keys=True)
+            f.write("\n")
 
 
 def fp(a):

@@ -38,8 +38,8 @@ def test_pass_golden(oracle):
 
 
 def test_runs_golden(oracle):
-    g = np.load(os.path.join(GOLD, "runs.npz"))
     for tag, npass in (("3x3", 1), ("5x5", 5)):
+        g = np.load(os.path.join(GOLD, "runs_%s.npz" % tag))
         aw, clean, noisy = gi.run_inputs(tag)
         mask = np.ones(aw * aw)
         b, nrt, sch = oracle.run_step1(noisy, mask, 25.0, 2.7, aw, aw, 1, 8, 18, 6, 16, 4, oracle.ID, oracle.SADCT, oracle.HAAR)
@@ -88,9 +88,10 @@ def test_schedule_pass_counts(oracle):
 
 def test_config1_fixture_golden(oracle):
     """BASELINE.json configs[0] (the reference's fixture, README.md:50 parameters): the oracle reproduces the unmodified reference's
-    basic and denoised estimates bit for bit (tiles + PSNRs of tests/golden/config1.npz, tests/make_golden_config1.py)."""
+    basic and denoised estimates bit for bit (tiles + PSNRs of tests/golden/config1.npz, tests/make_golden_config1.py). The fixture's
+    pixels are stored losslessly as tests/golden/sourceLF/SAI_<s>_<t>.png."""
     g = np.load(os.path.join(GOLD, "config1.npz"))
-    clean = g["clean_u8"].astype(np.float32)
+    clean = gi.config1_fixture().astype(np.float32)
     noisy = oracle.add_noise(clean, 25.0)
     mask = np.ones(9)
     b, nrt, sched = oracle.run_step1(noisy, mask, 25.0, 2.7, 3, 3, 1, 8, 18, 6, 16, 4, oracle.ID, oracle.SADCT, oracle.HAAR)

@@ -120,9 +120,10 @@ def test_config1_fixture_against_reference(eng, oracle):
     """BASELINE.json configs[0]: the reference's fixture testing/sourceLF with mt19937ar noise (seed 20171016 + st), README.md:50
     parameters, through the host-buffer entry points; against tiles and PSNRs produced by the unmodified reference
     (tests/make_golden_config1.py)."""
+    import golden_inputs as gi
     import lfbm5d_b200 as L
     g = np.load(os.path.join(GOLD, "config1.npz"))
-    clean = g["clean_u8"].astype(np.float32)
+    clean = gi.config1_fixture().astype(np.float32)
     noisy = oracle.add_noise(clean, 25.0)
     mask = np.ones(9, np.uint32)
     p1 = L.make_params(25.0, 2.7, 3, 3, 1, 256, 256, 3, 8, 18, 6, 16, 4, L.ID, L.SADCT, L.HAAR)

@@ -1,7 +1,8 @@
 """Host glue of the command lines (SURVEY.md 8(f) rank 1-2), CPU only: the PNG codec of lfbm5d_b200/csrc/lf_io.h against an
 independent decoder (Pillow) — every colour type, bit depth and interlace method read_png_f32 accepts (io_png.c:116-260), the
 writer's rounding (io_png.c:648-650) — and the metrics / difference images / PSNR report against the UNMODIFIED reference
-functions (compute_psnr_LF, compute_diff_LF, write_psnr_LF; utilities_LF.cpp:639-869) compiled into oracle/_ref."""
+functions (compute_psnr_LF, compute_diff_LF, write_psnr_LF; utilities_LF.cpp:639-869): live where oracle/_ref is built, else
+against the stored digests of their results (tests/golden/ref_pins.json)."""
 import ctypes as C
 import os
 import struct
@@ -129,11 +130,10 @@ def test_png_reader_every_format(tmp_path, ctype, depth, interlace):
 
 
 def test_png_reader_on_the_reference_fixture():
-    """The nine SAIs of /root/reference/testing/sourceLF (config 1): same pixels as Pillow."""
+    """The nine SAIs of the reference's fixture `testing/sourceLF` (config 1), stored losslessly as 8-bit RGB PNGs under
+    tests/golden/sourceLF: same pixels as Pillow."""
     from PIL import Image
-    d = "/root/reference/testing/sourceLF"
-    if not os.path.isdir(d):
-        pytest.skip("reference fixture not mounted")
+    d = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sourceLF")
     names = sorted(f for f in os.listdir(d) if f.endswith(".png"))
     assert len(names) == 9
     for f in names:
@@ -172,7 +172,6 @@ def test_png_writer_rounding_and_round_trip(tmp_path, c):
 def test_metrics_and_report_equal_the_reference(tmp_path, ref, major):
     """PSNR / RMSE per SAI with their averages and standard deviations, difference images, and the report file, byte for byte."""
     h = host()
-    r = ref.lib()
     aw, ah, each = 4, 3, 3 * 20 * 24
     asize = aw * ah
     rng = np.random.default_rng(11)
@@ -181,8 +180,8 @@ def test_metrics_and_report_equal_the_reference(tmp_path, ref, major):
     mask = np.ones(asize, np.uint32)
     mask[5] = 0
     fp, up = (lambda x: x.ctypes.data_as(C.POINTER(C.c_float))), (lambda x: x.ctypes.data_as(C.POINTER(C.c_uint)))
-    res = {}
-    for name, lib, pre in (("ours", h, "lfio_"), ("ref", r, "ref_compute_")):
+
+    def metrics(lib, pre):
         ps, rm, st = np.zeros(asize, np.float32), np.zeros(asize, np.float32), np.zeros(4, np.float32)
         f = getattr(lib, pre + "psnr_LF")
         f.argtypes = [C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint), C.c_uint, C.c_size_t, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]
@@ -191,20 +190,22 @@ def test_metrics_and_report_equal_the_reference(tmp_path, ref, major):
         g = getattr(lib, pre + "diff_LF")
         g.argtypes = [C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint), C.c_uint, C.c_size_t, C.c_float, C.POINTER(C.c_float)]
         assert g(fp(a), fp(b), up(mask), asize, each, 10.0, fp(d)) == 0
-        res[name] = (ps, rm, st, d)
-    for x, y in zip(res["ours"], res["ref"]):
-        assert np.array_equal(x, y)
-    ps, rm, st, _ = res["ours"]
-    files = {}
-    for name, f in (("ours", h.lfio_write_psnr_LF), ("ref", r.ref_write_psnr_LF)):
+        return ps, rm, st, d
+    ours = metrics(h, "lfio_")
+    ref.check("metrics_LF", ours, lambda R: metrics(R.lib(), "ref_compute_"))
+    ps, rm, st, _ = ours
+
+    def report(f, name):
         f.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(C.c_uint), C.c_uint, C.c_uint, C.c_uint, C.POINTER(C.c_float), C.c_float, C.c_float,
                       C.POINTER(C.c_float), C.c_float, C.c_float]
         path = tmp_path / (name + ".txt")
         for label in (b"noisy", b"denoised"):          # the report is appended to
-            assert f(str(path).encode(), label, up(mask), ref.ROWMAJOR if major == "row" else ref.COLMAJOR, aw, ah, fp(ps), float(st[0]), float(st[1]),
+            assert f(str(path).encode(), label, up(mask), L.ROWMAJOR if major == "row" else L.COLMAJOR, aw, ah, fp(ps), float(st[0]), float(st[1]),
                      fp(rm), float(st[2]), float(st[3])) == 0
-        files[name] = path.read_bytes()
-    assert files["ours"] == files["ref"] and b"No SAI" in files["ours"]
+        return np.frombuffer(path.read_bytes(), np.uint8)
+    text = report(h.lfio_write_psnr_LF, "ours")
+    ref.check("write_psnr_LF_" + major, text, lambda R: report(R.lib().ref_write_psnr_LF, "ref"))
+    assert b"No SAI" in text.tobytes()
 
 
 def _write_lf(tmp_path, arr, s_start=1, t_start=1, gray=False):
