@@ -29,7 +29,9 @@ typedef struct lfbm5d_params {
     float    lambda;        /* lambdaHard5D; ignored by step 2 */
     unsigned ang_major;     /* LFBM5D_ROWMAJOR / LFBM5D_COLMAJOR */
     unsigned awidth, aheight;
-    unsigned an;            /* anHard / anWien: half size of the angular search window */
+    unsigned an;            /* anHard / anWien: half size of the angular search window, 0, 1 or 2 ((2an+1)^2 SAIs per group).
+                             * an = 2 needs N * k^2 <= 2048 in step 1 and 2 * N * k^2 <= 2048 in step 2 (one channel of the
+                             * 25-SAI group in the shared memory of one CTA): k = 16 with N <= 8 / N <= 4, k = 8 with N <= 32 / N <= 16 */
     unsigned width, height, chnls;
     unsigned N;             /* NHard / NWien */
     unsigned nSim, nDisp;

@@ -6,8 +6,12 @@
 #include <stdint.h>
 
 #define LF_MAXK      16      // largest patch side handled by the transform kernels
-#define LF_MAXASW    3       // angular window side (2*an+1), an <= 1
+#define LF_MAXASW    5       // angular window side (2*an+1), an <= 2
 #define LF_MAXA      (LF_MAXASW * LF_MAXASW)
+// windows up to 3x3 (an <= 1): SA-DCT shapes from a host table of 2^A entries, 16-bit group masks, and the group kernels
+// k_groups / k_groups_id16 / k_groups_w8 with their shared arrays sized for 9 SAIs; 5x5 windows take k_groups25
+#define LF_LUTASW    3
+#define LF_LUTA      (LF_LUTASW * LF_LUTASW)
 #define LF_MAXN      32      // largest number of similar patches
 #define LF_MAXNS2    169     // (2*nDisp+1)^2, nDisp <= 6
 #define LF_SQRT2_INV_F ((float) 0.7071067811865475)
@@ -21,12 +25,12 @@ struct LfTables {
     float dct2i[LF_MAXK * LF_MAXK];      // [kk*k + j] = j ? (float)(2 cos(pi j (kk+1/2) / k)) : 1
     float cn2[LF_MAXK * LF_MAXK], cni2[LF_MAXK * LF_MAXK], kaiser[LF_MAXK * LF_MAXK];
     float coef2inv;                      // 1 / (2k)
-    float dctaf[LF_MAXASW][LF_MAXASW * LF_MAXASW];   // [n-1][kk*n + j], 1-D tables for lengths 1..asw
-    float dctai[LF_MAXASW][LF_MAXASW * LF_MAXASW];
-    float cn4[LF_MAXA], cni4[LF_MAXA];
+    float dctaf[LF_LUTASW][LF_LUTASW * LF_LUTASW];   // [n-1][kk*n + j], 1-D tables for lengths 1..asw (windows up to 3x3)
+    float dctai[LF_LUTASW][LF_LUTASW * LF_LUTASW];
+    float cn4[LF_LUTA], cni4[LF_LUTA];
     float coef4inv;                      // 1 / (sqrt(aw) sqrt(ah) 2)
-    float cnsa[LF_MAXASW][LF_MAXASW], cnisa[LF_MAXASW][LF_MAXASW];   // [n-2][t]
-    float coefsa_inv[LF_MAXASW + 1];     // [n] = 0.5 (float)SQRT2_INV / sqrt(n)
+    float cnsa[LF_LUTASW][LF_LUTASW], cnisa[LF_LUTASW][LF_LUTASW];   // [n-2][t]
+    float coefsa_inv[LF_LUTASW + 1];     // [n] = 0.5 (float)SQRT2_INV / sqrt(n)
     float lpd[10], hpd[10], lpr[10], hpr[10];
     float sigma[3], sigma2[3];
     float thr[3][8];                     // hard threshold per channel and log2(nSx)
@@ -36,6 +40,12 @@ struct LfTables {
     float dct5f[1365], dct5i[1365];
     float cn5_0[6], cn5_c[6], coef5inv[6];
     float thr_dct[3];
+    // the angular tables above for 5x5 windows (lengths 1..5, k_groups25). Kept apart: the 3x3 group kernels read theirs at
+    // the offsets and strides they were tuned with (a 5x5 layout of the same arrays costs k_groups_id16 16 registers).
+    float dctaf5[LF_MAXASW][LF_MAXASW * LF_MAXASW], dctai5[LF_MAXASW][LF_MAXASW * LF_MAXASW];
+    float cn4_5[LF_MAXA], cni4_5[LF_MAXA];
+    float cnsa5[LF_MAXASW][LF_MAXASW], cnisa5[LF_MAXASW][LF_MAXASW];
+    float coefsa_inv5[LF_MAXASW + 1];
 };
 
 __constant__ LfTables c_tab;
@@ -62,6 +72,14 @@ struct LfWindow {
     int      st[LF_MAXA];        // global SAI index of each window slot
     unsigned mask[LF_MAXA];
     unsigned proc[LF_MAXA];
+    int      A;
+};
+// The window as the group kernels of windows up to 3x3 receive it: their parameter block keeps its 3x3 size (a larger one
+// costs k_groups_id16 16 registers)
+struct LfWindow9 {
+    int      st[LF_LUTA];
+    unsigned mask[LF_LUTA];
+    unsigned proc[LF_LUTA];
     int      A;
 };
 

@@ -6,7 +6,9 @@
 #pragma once
 #include "common.cuh"
 
-struct GroupArgs {
+template <int SW> struct GroupShapeT;
+
+struct GroupArgsBase {
     int C, asw, A, k, log2k, N, w, h, pst, nc;
     int r0;                           // first reference patch of the launch (blockIdx.x + r0; row bands of the multi-GPU path)
     int RS, PS;                       // shared-memory row stride / patch stride (floats)
@@ -20,23 +22,56 @@ struct GroupArgs {
     // staging for the ordered aggregation kernel (k_aggregate): filtered patches, weights, positions, flags
     float *zbuf;                                  // [R][N][A][C][k2]
     float *wbuf;                                  // [R][C]
-    const unsigned short *gmask;                  // [R] bit st = SAI st takes part in the group's angular shape (k_group_masks)
-    const struct GroupShape *shape_lut;           // [2^A] SA-DCT index tables per shape (host-built, core:300-330)
+    const unsigned short *gmask;                  // [R] bit st = SAI st takes part in the group's angular shape (k_group_masks), A <= 9
+    const struct GroupShapeT<LF_LUTASW> *shape_lut;   // [2^A] SA-DCT index tables per shape (host-built, core:300-330), A <= 9
     const unsigned char *act;                     // partial-window branch: [R] 1 = reference patch still to be processed; nullptr = all
     int use_sd;                                   // 1: weight = 1 / sample std of the filtered group (core:3140-3173); 2: BM3D's variant (bm3d.cpp:1345)
     int partial;                                  // pst != cst: local 2-D variants (no zero column, core:1735)
     unsigned *ent;                                // [A][R*N] (y << 16 | x) of every patch that is aggregated, else LF_NOENT
     int R;
+};
+struct GroupArgs : GroupArgsBase {                // k_groups, k_groups_id16, k_groups_w8: windows up to 3x3
+    LfWindow9 win;
+};
+struct GroupArgs25 : GroupArgsBase {              // k_groups25: 5x5 windows
     LfWindow win;
+    const unsigned *gmask32;                      // [R] 25-bit angular shape masks (k_group_masks32); the SA-DCT tables are built per group
 };
 
 #define LF_NOENT 0xffffffffu
 
-struct GroupShape {
-    unsigned mask[LF_MAXA], idx[LF_MAXA], idx_col[LF_MAXA], mask_dct[LF_MAXA];
-    unsigned row_size[LF_MAXASW], col_size[LF_MAXASW];
+// SA-DCT index tables of one angular shape of a window of side up to SW
+template <int SW> struct GroupShapeT {
+    unsigned mask[SW * SW], idx[SW * SW], idx_col[SW * SW], mask_dct[SW * SW];
+    unsigned row_size[SW], col_size[SW];
     int use_sadct;
 };
+typedef GroupShapeT<LF_LUTASW> GroupShape;        // the host table's entries (windows up to 3x3)
+
+// The tables of the shape `bits` (bit st: SAI st takes part) of an asw x asw window, as sadct_4d_process builds them
+// (core:1969-2010); ensure_shape_lut runs the same construction on the host for every shape of a window up to 3x3.
+template <int SW>
+__host__ __device__ inline void lf_shape_build(GroupShapeT<SW> &sh, unsigned bits, unsigned asw)
+{
+    const unsigned A = asw * asw;
+    unsigned size = 0;
+    for (unsigned st = 0; st < SW * SW; st++) { sh.mask[st] = st < A ? (bits >> st) & 1u : 0u; sh.idx[st] = sh.idx_col[st] = sh.mask_dct[st] = 0; size += sh.mask[st]; }
+    sh.use_sadct = size != A;
+    unsigned mask_col[SW * SW] = { 0 };
+    for (unsigned s = 0; s < asw; s++) {
+        unsigned rr = 0;
+        for (unsigned t = 0; t < asw; t++) if (sh.mask[s * asw + t]) sh.idx[s * asw + rr++] = t;
+        sh.row_size[s] = rr;
+        for (unsigned t = 0; t < rr; t++) mask_col[s * asw + t] = 1;
+    }
+    for (unsigned t = 0; t < asw; t++) {
+        unsigned rr = 0;
+        for (unsigned s = 0; s < asw; s++) if (mask_col[s * asw + t]) sh.idx_col[(rr++) * asw + t] = s;
+        sh.col_size[t] = rr;
+        for (unsigned s = 0; s < rr; s++) sh.mask_dct[s * asw + t] = 1;
+    }
+    for (unsigned s = asw; s < SW; s++) sh.row_size[s] = sh.col_size[s] = 0;
+}
 
 // ---- 1-D transforms along the similar patches (lib_transforms.cpp:290-321, :403-471), fully unrolled ----
 template <int NS> __device__ __forceinline__ void lf_haar_fwd(float *v)
@@ -213,10 +248,34 @@ __device__ __forceinline__ float lf_filter5d(float *X, float *E, int base, int n
     return wsum;
 }
 
+// ---- angular tables of windows up to TW x TW (LfTables: windows up to 3x3 and 5x5 windows have their own) ----
+template <int TW> __device__ __forceinline__ const float *lf_tab_dcta(int n, bool fwd)      // 1-D DCT of length n
+{
+    if constexpr (TW > LF_LUTASW) return fwd ? c_tab.dctaf5[n - 1] : c_tab.dctai5[n - 1];
+    else return fwd ? c_tab.dctaf[n - 1] : c_tab.dctai[n - 1];
+}
+template <int TW> __device__ __forceinline__ const float *lf_tab_cn4(bool fwd)
+{
+    if constexpr (TW > LF_LUTASW) return fwd ? c_tab.cn4_5 : c_tab.cni4_5;
+    else return fwd ? c_tab.cn4 : c_tab.cni4;
+}
+template <int TW> __device__ __forceinline__ const float *lf_tab_cnsa(int n, bool fwd)
+{
+    if constexpr (TW > LF_LUTASW) return fwd ? c_tab.cnsa5[n - 2] : c_tab.cnisa5[n - 2];
+    else return fwd ? c_tab.cnsa[n - 2] : c_tab.cnisa[n - 2];
+}
+template <int TW> __device__ __forceinline__ float lf_tab_coefsa_inv(int n)
+{
+    if constexpr (TW > LF_LUTASW) return c_tab.coefsa_inv5[n];
+    else return c_tab.coefsa_inv[n];
+}
+
 // ---- angular transforms of one (n, pq) vector v[A] (st fastest) ----
 template <int ASW> __device__ __forceinline__ void lf_dct4_fwd(float *v)
 {
-    const float *T = c_tab.dctaf[ASW - 1];
+    constexpr int TW = ASW > LF_LUTASW ? LF_MAXASW : LF_LUTASW;
+    const float *T = lf_tab_dcta<TW>(ASW, true);
+    const float *cn4 = lf_tab_cn4<TW>(true);
     float y[ASW * ASW];
 #pragma unroll
     for (int s = 0; s < ASW; ++s)
@@ -234,15 +293,17 @@ template <int ASW> __device__ __forceinline__ void lf_dct4_fwd(float *v)
             float acc = 0.f;
 #pragma unroll
             for (int s = 0; s < ASW; ++s) acc = fmaf(y[s * ASW + t], T[kk * ASW + s], acc);
-            v[kk * ASW + t] = acc * c_tab.cn4[kk * ASW + t];
+            v[kk * ASW + t] = acc * cn4[kk * ASW + t];
         }
 }
 template <int ASW> __device__ __forceinline__ void lf_dct4_inv(float *v)
 {
-    const float *T = c_tab.dctai[ASW - 1];
+    constexpr int TW = ASW > LF_LUTASW ? LF_MAXASW : LF_LUTASW;
+    const float *T = lf_tab_dcta<TW>(ASW, false);
+    const float *cni4 = lf_tab_cn4<TW>(false);
     float a[ASW * ASW], y[ASW * ASW];
 #pragma unroll
-    for (int st = 0; st < ASW * ASW; ++st) a[st] = v[st] * c_tab.cni4[st];
+    for (int st = 0; st < ASW * ASW; ++st) a[st] = v[st] * cni4[st];
 #pragma unroll
     for (int s = 0; s < ASW; ++s)
 #pragma unroll
@@ -262,10 +323,10 @@ template <int ASW> __device__ __forceinline__ void lf_dct4_inv(float *v)
             v[kk * ASW + t] = acc * c_tab.coef4inv;
         }
 }
-// generic 1-D r2r of length n (1..ASW) on a small array
-__device__ __forceinline__ void lf_r2r_small(const float *in, float *out, int n, bool fwd)
+// generic 1-D r2r of length n (1..SW) on a small array
+template <int SW> __device__ __forceinline__ void lf_r2r_small(const float *in, float *out, int n, bool fwd)
 {
-    const float *T = fwd ? c_tab.dctaf[n - 1] : c_tab.dctai[n - 1];
+    const float *T = lf_tab_dcta<SW>(n, fwd);
     for (int kk = 0; kk < n; ++kk) {
         float acc = 0.f;
         for (int j = 0; j < n; ++j) acc = fmaf(in[j], T[kk * n + j], acc);
@@ -273,16 +334,16 @@ __device__ __forceinline__ void lf_r2r_small(const float *in, float *out, int n,
     }
 }
 // shape-adaptive variants (core:1969-2116, :2131-2264); rare path, generic code
-__device__ __noinline__ void lf_sadct_fwd(float *v, const GroupShape &sh, int asw)
+template <int SW> __device__ __noinline__ void lf_sadct_fwd(float *v, const GroupShapeT<SW> &sh, int asw)
 {
-    float a[LF_MAXASW], b[LF_MAXASW];
+    float a[SW], b[SW];
     for (int s = 0; s < asw; ++s) {
         const int n = sh.row_size[s];
         if (n == 1) v[s * asw] = v[s * asw + sh.idx[s * asw]];
         else if (n > 1) {
             for (int t = 0; t < n; ++t) a[t] = v[s * asw + sh.idx[s * asw + t]];
-            lf_r2r_small(a, b, n, true);
-            for (int t = 0; t < n; ++t) v[s * asw + t] = b[t] * c_tab.cnsa[n - 2][t];
+            lf_r2r_small<SW>(a, b, n, true);
+            for (int t = 0; t < n; ++t) v[s * asw + t] = b[t] * lf_tab_cnsa<SW>(n, true)[t];
         }
     }
     for (int t = 0; t < asw; ++t) {
@@ -290,24 +351,24 @@ __device__ __noinline__ void lf_sadct_fwd(float *v, const GroupShape &sh, int as
         if (n == 1) v[t] = v[sh.idx_col[t] * asw + t];
         else if (n > 1) {
             for (int s = 0; s < n; ++s) a[s] = v[sh.idx_col[s * asw + t] * asw + t];
-            lf_r2r_small(a, b, n, true);
-            for (int s = 0; s < n; ++s) v[s * asw + t] = b[s] * c_tab.cnsa[n - 2][s];
+            lf_r2r_small<SW>(a, b, n, true);
+            for (int s = 0; s < n; ++s) v[s * asw + t] = b[s] * lf_tab_cnsa<SW>(n, true)[s];
         }
     }
     const float coef = 0.5f * LF_SQRT2_INV_F;
     for (int st = 0; st < asw * asw; ++st) v[st] *= (float) sh.mask_dct[st] * coef;
 }
-__device__ __noinline__ void lf_sadct_inv(float *v, const GroupShape &sh, int asw)
+template <int SW> __device__ __noinline__ void lf_sadct_inv(float *v, const GroupShapeT<SW> &sh, int asw)
 {
-    float a[LF_MAXASW], b[LF_MAXASW];
+    float a[SW], b[SW];
     const float c2 = 2.0f * LF_SQRT2_F;
     for (int t = 0; t < asw; ++t) {
         const int n = sh.col_size[t];
         if (n == 1) v[sh.idx_col[t] * asw + t] = v[t] * c2;
         else if (n > 1) {
-            for (int s = 0; s < n; ++s) a[s] = v[s * asw + t] * c_tab.cnisa[n - 2][s] * c2;
-            lf_r2r_small(a, b, n, false);
-            const float coef = c_tab.coefsa_inv[n];
+            for (int s = 0; s < n; ++s) a[s] = v[s * asw + t] * lf_tab_cnsa<SW>(n, false)[s] * c2;
+            lf_r2r_small<SW>(a, b, n, false);
+            const float coef = lf_tab_coefsa_inv<SW>(n);
             for (int s = 0; s < n; ++s) v[sh.idx_col[s * asw + t] * asw + t] = b[s] * coef;
         }
     }
@@ -315,9 +376,9 @@ __device__ __noinline__ void lf_sadct_inv(float *v, const GroupShape &sh, int as
         const int n = sh.row_size[s];
         if (n == 1) v[s * asw + sh.idx[s * asw]] = v[s * asw];
         else if (n > 1) {
-            for (int t = 0; t < n; ++t) a[t] = v[s * asw + t] * c_tab.cnisa[n - 2][t];
-            lf_r2r_small(a, b, n, false);
-            const float coef = c_tab.coefsa_inv[n];
+            for (int t = 0; t < n; ++t) a[t] = v[s * asw + t] * lf_tab_cnsa<SW>(n, false)[t];
+            lf_r2r_small<SW>(a, b, n, false);
+            const float coef = lf_tab_coefsa_inv<SW>(n);
             for (int t = 0; t < n; ++t) v[s * asw + sh.idx[s * asw + t]] = b[t] * coef;
         }
     }
@@ -452,10 +513,11 @@ __device__ __forceinline__ void lf_t2d(float *B, int npatch, const GroupArgs &g,
 // gathered patch (ZB: patches that read as zeros point at the zero block behind the window buffers, else szero marks them),
 // and the aggregation entries: (y << 16 | x) of every patch that k_aggregate has to add, LF_NOENT otherwise.
 // Returns false (after marking the group's entries empty) for reference patches the partial-window branch skips.
-template <bool ZB>
-__device__ __forceinline__ bool lf_group_setup(const GroupArgs &g, int r, int nSx, GroupShape &sh, unsigned *sofs, unsigned char *szero)
+// SW: window side the shared arrays are sized for; windows up to 3x3 copy their shape from the host table, 5x5 ones build it.
+template <bool ZB, int SW = LF_LUTASW, class GA = GroupArgs>
+__device__ __forceinline__ bool lf_group_setup(const GA &g, int r, int nSx, GroupShapeT<SW> &sh, unsigned *sofs, unsigned char *szero)
 {
-    __shared__ unsigned s_yx[LF_MAXN * LF_MAXA];
+    __shared__ unsigned s_yx[LF_MAXN * SW * SW];
     const int A = g.A, w = g.w, k = g.k;
     const int tid = threadIdx.x, nt = blockDim.x;
     const unsigned plane = (unsigned) g.w * (unsigned) g.h;
@@ -466,11 +528,13 @@ __device__ __forceinline__ bool lf_group_setup(const GroupArgs &g, int r, int nS
         }
         return false;
     }
-    if (tid >= nt - 32) {        // the last warp copies the group's SA-DCT tables, beside the offset loop of the first warps
-        const unsigned *src = reinterpret_cast<const unsigned *>(g.shape_lut + g.gmask[r]);
-        unsigned *dst = reinterpret_cast<unsigned *>(&sh);
-        for (int i = tid - (nt - 32); i < (int) (sizeof(GroupShape) / 4); i += 32) dst[i] = src[i];
-    }
+    if constexpr (SW == LF_LUTASW) {
+        if (tid >= nt - 32) {        // the last warp copies the group's SA-DCT tables, beside the offset loop of the first warps
+            const unsigned *src = reinterpret_cast<const unsigned *>(g.shape_lut + g.gmask[r]);
+            unsigned *dst = reinterpret_cast<unsigned *>(&sh);
+            for (int i = tid - (nt - 32); i < (int) (sizeof(GroupShape) / 4); i += 32) dst[i] = src[i];
+        }
+    } else if (tid == nt - 32) lf_shape_build<SW>(sh, g.gmask32[r], (unsigned) g.asw);     // 2^25 shapes: no table, built per group
     for (int t = tid; t < nSx * A; t += nt) {
         const int n = t / A, st = t - n * A;
         const unsigned ind = g.bm_idx[(size_t) r * (g.N + 1) + n];
@@ -512,8 +576,9 @@ __global__ void k_active_refs(const float *__restrict__ den0, const int *__restr
 }
 
 // bit st of gmask[r]: SAI st belongs to the angular shape of reference patch r (core:300-312)
-__global__ void k_group_masks(const int *__restrict__ rows, const int *__restrict__ cols, int nc, int r0, int r1, int w, unsigned plane, int A, int pst,
-                              LfWindow win, const unsigned char *__restrict__ shape, unsigned short *__restrict__ gmask)
+template <typename M>
+__device__ __forceinline__ void lf_group_mask(const int *__restrict__ rows, const int *__restrict__ cols, int nc, int r0, int r1, int w, unsigned plane,
+                                              int A, int pst, const LfWindow &win, const unsigned char *__restrict__ shape, M *__restrict__ gmask)
 {
     const int r = r0 + blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= r1) return;
@@ -523,7 +588,18 @@ __global__ void k_group_masks(const int *__restrict__ rows, const int *__restric
         const unsigned b = (st == pst) ? 1u : (win.mask[st] ? (unsigned) shape[(size_t) st * plane + k_r] : 0u);
         m |= (b ? 1u : 0u) << st;
     }
-    gmask[r] = (unsigned short) m;
+    gmask[r] = (M) m;
+}
+__global__ void k_group_masks(const int *__restrict__ rows, const int *__restrict__ cols, int nc, int r0, int r1, int w, unsigned plane, int A, int pst,
+                              LfWindow win, const unsigned char *__restrict__ shape, unsigned short *__restrict__ gmask)
+{
+    lf_group_mask(rows, cols, nc, r0, r1, w, plane, A, pst, win, shape, gmask);
+}
+// 5x5 windows: 25 bits
+__global__ void k_group_masks32(const int *__restrict__ rows, const int *__restrict__ cols, int nc, int r0, int r1, int w, unsigned plane, int A, int pst,
+                                LfWindow win, const unsigned char *__restrict__ shape, unsigned *__restrict__ gmask)
+{
+    lf_group_mask(rows, cols, nc, r0, r1, w, plane, A, pst, win, shape, gmask);
 }
 
 template <int STEP, int ASW>
@@ -532,8 +608,8 @@ __global__ void __launch_bounds__(256) k_groups(GroupArgs g)
     extern __shared__ float smem[];
     __shared__ GroupShape sh;
     __shared__ float red[8];
-    __shared__ unsigned sofs[LF_MAXN * LF_MAXA];          // per gathered patch: st*C*plane + position
-    __shared__ unsigned char szero[LF_MAXN * LF_MAXA];    // patch reads as zeros (empty SAI, or column w-k: core:1697)
+    __shared__ unsigned sofs[LF_MAXN * LF_LUTA];          // per gathered patch: st*C*plane + position
+    __shared__ unsigned char szero[LF_MAXN * LF_LUTA];    // patch reads as zeros (empty SAI, or column w-k: core:1697)
     constexpr int A = ASW * ASW;
     const int tid = threadIdx.x;
     const int r = blockIdx.x + g.r0;

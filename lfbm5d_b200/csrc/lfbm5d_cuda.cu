@@ -7,6 +7,7 @@
 #include "block_matching.cuh"
 #include "groups.cuh"
 #include "groups_wiener8.cuh"
+#include "groups25.cuh"
 
 #include <cmath>
 #include <cstdio>
@@ -226,7 +227,7 @@ int validate(const lfbm5d_params *p, int step)
     const unsigned asw = 2 * p->an + 1;
     if (asw > p->aheight || asw > p->awidth)   // bm5d.cpp:120-124
         return fail("Wrong size of angular search window, the angular search window must be smaller than the light field angular size.");
-    if (asw > LF_MAXASW) return fail("angular half window > 1 is not supported by this build");
+    if (asw > LF_MAXASW) return fail("angular half window an > 2 is not supported by this build (an must be 0, 1 or 2)");
     if (p->k != 8 && p->k != 16) return fail("patch size must be 8 or 16 in this build");
     if (p->N == 0 || p->N > LF_MAXN || (p->N & (p->N - 1))) return fail("N must be a power of two <= 32");
     if (p->nDisp > 6) return fail("nDisp > 6 is not supported by this build");
@@ -240,7 +241,9 @@ int validate(const lfbm5d_params *p, int step)
     if (p->height < p->k || p->width < p->k) return fail("image smaller than a patch");
     // the mirror padding of nSim + nDisp pixels (utilities.cpp:215-263) reflects once
     if (p->height < p->nSim + p->nDisp || p->width < p->nSim + p->nDisp) return fail("image smaller than the padding nSim + nDisp");
-    (void) step;
+    // 5x5 windows: one channel of the group (twice that in step 2) has to fit into the shared memory of one CTA (k_groups25)
+    if (asw == 5 && p->N * p->k * p->k * (step == 2 ? 2 : 1) > 2048)
+        return fail("an = 2 needs N * k^2 <= 2048 in step 1 and 2 * N * k^2 <= 2048 in step 2 (k = 16: N <= 8 / N <= 4; k = 8: N <= 32 / N <= 16)");
     return 0;
 }
 
@@ -286,24 +289,31 @@ int setup_tables(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, unsigned tau
             }
         T.coef2inv = 1.0f / (float) (k * 2);
     }
-    for (int n = 1; n <= asw; n++) dct_tables(T.dctaf[n - 1], T.dctai[n - 1], n);
+    // angular tables: windows up to 3x3 and 5x5 windows have their own arrays (row length AW)
+    const bool a5 = asw > LF_LUTASW;
+    const int AW = a5 ? LF_MAXASW : LF_LUTASW;
+    float *dctaf = a5 ? &T.dctaf5[0][0] : &T.dctaf[0][0], *dctai = a5 ? &T.dctai5[0][0] : &T.dctai[0][0];
+    float *cn4 = a5 ? T.cn4_5 : T.cn4, *cni4 = a5 ? T.cni4_5 : T.cni4;
+    float *cnsa = a5 ? &T.cnsa5[0][0] : &T.cnsa[0][0], *cnisa = a5 ? &T.cnisa5[0][0] : &T.cnisa[0][0];
+    float *coefsa_inv = a5 ? T.coefsa_inv5 : T.coefsa_inv;
+    for (int n = 1; n <= asw; n++) dct_tables(dctaf + (n - 1) * AW * AW, dctai + (n - 1) * AW * AW, n);
     {   // core:3191-3216
         const float coef = 0.5f / (sqrtf((float) asw) * sqrtf((float) asw));
         for (int i = 0; i < asw; i++)
             for (int j = 0; j < asw; j++) {
-                if (i == 0 && j == 0) { T.cn4[i * asw + j] = (float) (0.5f * coef); T.cni4[i * asw + j] = 2.0f; }
-                else if (i * j == 0) { T.cn4[i * asw + j] = (float) (SQRT2_INV_D * coef); T.cni4[i * asw + j] = (float) SQRT2_D; }
-                else { T.cn4[i * asw + j] = (float) (1.0f * coef); T.cni4[i * asw + j] = 1.0f; }
+                if (i == 0 && j == 0) { cn4[i * asw + j] = (float) (0.5f * coef); cni4[i * asw + j] = 2.0f; }
+                else if (i * j == 0) { cn4[i * asw + j] = (float) (SQRT2_INV_D * coef); cni4[i * asw + j] = (float) SQRT2_D; }
+                else { cn4[i * asw + j] = (float) (1.0f * coef); cni4[i * asw + j] = 1.0f; }
             }
         T.coef4inv = 1.0f / (sqrtf((float) asw) * sqrtf((float) asw) * 2.0f);   // core:1945
     }
     for (int n = 2; n <= asw; n++) {   // core:3229-3252
         const float coef = (float) ((float) SQRT2_D / sqrt((double) n));
-        T.cnsa[n - 2][0] = (float) (SQRT2_INV_D * coef);
-        T.cnisa[n - 2][0] = (float) SQRT2_D;
-        for (int i = 1; i < n; i++) { T.cnsa[n - 2][i] = coef; T.cnisa[n - 2][i] = 1.0f; }
+        cnsa[(n - 2) * AW] = (float) (SQRT2_INV_D * coef);
+        cnisa[(n - 2) * AW] = (float) SQRT2_D;
+        for (int i = 1; i < n; i++) { cnsa[(n - 2) * AW + i] = coef; cnisa[(n - 2) * AW + i] = 1.0f; }
     }
-    for (int n = 1; n <= asw; n++) T.coefsa_inv[n] = 0.5f * (float) (SQRT2_INV_D) / sqrtf((float) n);   // core:2190, :2242
+    for (int n = 1; n <= asw; n++) coefsa_inv[n] = 0.5f * (float) (SQRT2_INV_D) / sqrtf((float) n);   // core:2190, :2242
     {   // lib_transforms.cpp:215-277
         const float coef_norm = 1.f / (sqrtf(2.f) * 128.f), sqrt2_inv = 1.f / sqrtf(2.f);
         static const float a[10] = { 3.f, -3.f, -22.f, 22.f, 128.f, 128.f, 22.f, -22.f, -3.f, 3.f };
@@ -427,27 +437,13 @@ __global__ void k_bm_identity(const int *rows, const int *cols, int nc, int w, i
 int ensure_shape_lut(lfbm5d_ctx *ctx, unsigned asw)
 {
     if (ctx->lut_asw == asw) return 0;
+    if (asw > LF_LUTASW) return 0;       // 5x5 windows: k_groups25 builds the shape of each group from its 25-bit mask
     const unsigned A = asw * asw, n = 1u << A;
     std::vector<GroupShape> lut(n);
     for (unsigned bits = 0; bits < n; bits++) {
         GroupShape &sh = lut[bits];
         memset(&sh, 0, sizeof(sh));
-        unsigned size = 0;
-        for (unsigned st = 0; st < A; st++) { sh.mask[st] = (bits >> st) & 1u; size += sh.mask[st]; }
-        sh.use_sadct = size != A;
-        unsigned mask_col[LF_MAXA] = { 0 };
-        for (unsigned s = 0; s < asw; s++) {
-            unsigned rr = 0;
-            for (unsigned t = 0; t < asw; t++) if (sh.mask[s * asw + t]) sh.idx[s * asw + rr++] = t;
-            sh.row_size[s] = rr;
-            for (unsigned t = 0; t < rr; t++) mask_col[s * asw + t] = 1;
-        }
-        for (unsigned t = 0; t < asw; t++) {
-            unsigned rr = 0;
-            for (unsigned s = 0; s < asw; s++) if (mask_col[s * asw + t]) sh.idx_col[(rr++) * asw + t] = s;
-            sh.col_size[t] = rr;
-            for (unsigned s = 0; s < rr; s++) sh.mask_dct[s * asw + t] = 1;
-        }
+        lf_shape_build(sh, bits, asw);
     }
     if (ctx->shape_lut.ensure(n * sizeof(GroupShape))) return 1;
     CK(cudaMemcpyAsync(ctx->shape_lut.p, lut.data(), n * sizeof(GroupShape), cudaMemcpyHostToDevice, ctx->stream));
@@ -724,30 +720,63 @@ int launch_stereo_argmin(lfbm5d_ctx *ctx, const PassCfg &pc, const SatPlan &P, i
     return 0;
 }
 
+// Angular shape masks of the reference patches [r0, r1) (bit st: SAI st takes part), with the SA-DCT tables their group kernel
+// reads: 16-bit masks into the host-built table for windows up to 3x3, 32-bit masks for 5x5 windows
+int launch_group_masks(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, int r0, int r1)
+{
+    const PassGeom pg = pass_geom(pc);
+    if (pc.asw > LF_LUTASW) {
+        if (ctx->gmask.ensure((size_t) pg.R * 4)) return 1;
+        LAUNCH(ctx, k_group_masks32, (r1 - r0 + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, r0, r1, (int) pc.wb,
+               (unsigned) pg.plane, (int) pc.A, pst, win, ctx->shape.as<unsigned char>(), ctx->gmask.as<unsigned>());
+        return 0;
+    }
+    if (ensure_shape_lut(ctx, pc.asw) || ctx->gmask.ensure((size_t) pg.R * 2)) return 1;
+    LAUNCH(ctx, k_group_masks, (r1 - r0 + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, r0, r1, (int) pc.wb,
+           (unsigned) pg.plane, (int) pc.A, pst, win, ctx->shape.as<unsigned char>(), ctx->gmask.as<unsigned short>());
+    return 0;
+}
+
 // Group kernel for the reference patches [r0, r1) (gather, transforms, shrinkage, inverses, staging for the aggregation)
 int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, bool partial, int r0, int r1)
 {
     if (r1 <= r0) return 0;
     const PassGeom pg = pass_geom(pc);
-    const size_t plane = pg.plane;
     const int R = pg.R;
-    GroupArgs ga{};
-    ga.gmask = ctx->gmask.as<unsigned short>(); ga.shape_lut = ctx->shape_lut.as<GroupShape>();
-    ga.act = partial ? ctx->act.as<unsigned char>() : nullptr; ga.partial = partial ? 1 : 0; ga.use_sd = (int) pc.useSD;
-    ga.C = pc.C; ga.asw = pc.asw; ga.A = pc.A; ga.k = pc.k; ga.log2k = pc.k == 8 ? 3 : 4; ga.N = pc.N; ga.w = pc.wb; ga.h = pc.hb;
-    ga.pst = pst; ga.nc = pg.nc; ga.r0 = r0;
+    GroupArgsBase gb{};
+    gb.gmask = ctx->gmask.as<unsigned short>(); gb.shape_lut = ctx->shape_lut.as<GroupShape>();
+    gb.act = partial ? ctx->act.as<unsigned char>() : nullptr; gb.partial = partial ? 1 : 0; gb.use_sd = (int) pc.useSD;
+    gb.C = pc.C; gb.asw = pc.asw; gb.A = pc.A; gb.k = pc.k; gb.log2k = pc.k == 8 ? 3 : 4; gb.N = pc.N; gb.w = pc.wb; gb.h = pc.hb;
+    gb.pst = pst; gb.nc = pg.nc; gb.r0 = r0;
     // row padding removes the shared-memory bank conflicts of the 2-D passes (3 CTAs/SM without it measured slower)
-    ga.RS = pc.tau_2D == LFBM5D_ID ? pc.k : pc.k + 1;
-    ga.PS = pc.k * ga.RS;
-    ga.tau_2D = pc.tau_2D; ga.tau_4D = pc.tau_4D; ga.tau_5D = pc.tau_5D;
-    ga.rows = ctx->rows.as<int>(); ga.cols = ctx->cols.as<int>();
-    ga.bm_count = ctx->bmcount.as<unsigned>(); ga.bm_idx = ctx->bmidx.as<unsigned>();
-    ga.first = ctx->first.as<unsigned>(); ga.shape = ctx->shape.as<unsigned char>();
-    ga.nsym = ctx->nsym.as<float>(); ga.bsym = ctx->bsym.as<float>();
-    ga.numsym = ctx->numsym.as<float>(); ga.densym = ctx->densym.as<float>();
-    ga.zbuf = ctx->zbuf.as<float>(); ga.wbuf = ctx->wbuf.as<float>(); ga.ent = ctx->spos.as<unsigned>(); ga.R = R;
-    ga.win = win;
+    gb.RS = pc.tau_2D == LFBM5D_ID ? pc.k : pc.k + 1;
+    gb.PS = pc.k * gb.RS;
+    gb.tau_2D = pc.tau_2D; gb.tau_4D = pc.tau_4D; gb.tau_5D = pc.tau_5D;
+    gb.rows = ctx->rows.as<int>(); gb.cols = ctx->cols.as<int>();
+    gb.bm_count = ctx->bmcount.as<unsigned>(); gb.bm_idx = ctx->bmidx.as<unsigned>();
+    gb.first = ctx->first.as<unsigned>(); gb.shape = ctx->shape.as<unsigned char>();
+    gb.nsym = ctx->nsym.as<float>(); gb.bsym = ctx->bsym.as<float>();
+    gb.numsym = ctx->numsym.as<float>(); gb.densym = ctx->densym.as<float>();
+    gb.zbuf = ctx->zbuf.as<float>(); gb.wbuf = ctx->wbuf.as<float>(); gb.ent = ctx->spos.as<unsigned>(); gb.R = R;
     const int nblk = r1 - r0;
+    if (pc.asw == G25_SW) {
+        // 5x5 windows: dense swizzled patches (no row padding), one CTA of 512 threads per SM; validate() bounds the group
+        GroupArgs25 g25{};
+        static_cast<GroupArgsBase &>(g25) = gb;
+        g25.RS = pc.k; g25.PS = pc.k * pc.k;
+        g25.win = win;
+        g25.gmask32 = ctx->gmask.as<unsigned>();
+        const size_t smem25 = (size_t) pc.N * pc.A * g25.PS * 4 * (pc.step == 2 ? 2 : 1);
+        void (*k25)(GroupArgs25) = pc.step == 1 ? k_groups25<1> : k_groups25<2>;
+        CK(cudaFuncSetAttribute((const void *) k25, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem25));
+        k25<<<nblk, G25_NT, smem25, ctx->stream>>>(g25);
+        ctx->stats.kernel_launches++;
+        return 0;
+    }
+    GroupArgs ga{};
+    static_cast<GroupArgsBase &>(ga) = gb;
+    for (int a = 0; a < LF_LUTA; a++) { ga.win.st[a] = win.st[a]; ga.win.mask[a] = win.mask[a]; ga.win.proc[a] = win.proc[a]; }
+    ga.win.A = win.A;
     const size_t smem = (size_t) pc.N * pc.A * ga.PS * 4 * (pc.step == 2 ? 2 : 1);
     void (*kfn)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups<1, 3> : k_groups<1, 1>)
                                           : (pc.asw == 3 ? k_groups<2, 3> : k_groups<2, 1>);
@@ -865,9 +894,7 @@ int run_pass(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, i
     if (launch_stereo_argmin(ctx, pc, P, 0, P.nslots, sB)) return 1;
     CK(cudaEventRecord(ctx->ev_join, sB));
     CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-    if (ensure_shape_lut(ctx, pc.asw) || ctx->gmask.ensure(R * 2)) return 1;
-    LAUNCH(ctx, k_group_masks, (R + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, 0, (int) R, (int) pc.wb, (unsigned) pg.plane,
-           (int) pc.A, (int) pst, win, ctx->shape.as<unsigned char>(), ctx->gmask.as<unsigned short>());
+    if (launch_group_masks(ctx, pc, win, (int) pst, 0, R)) return 1;
     if (ctx->timing) CK(cudaEventRecord(ctx->ev[1], ctx->stream));
     if (ctx->bm_only) { CK(cudaGetLastError()); return 0; }
 

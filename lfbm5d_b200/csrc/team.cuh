@@ -467,9 +467,7 @@ int team_pass_body(lfbm5d_team *T, const PassCfg &pc, bool redo)
             } else
                 LAUNCH(ctx, k_bm_identity_rows, (nown + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, wb, bd.r0, bd.r1, (int) pc.N,
                        ctx->bmcount.as<unsigned>(), ctx->bmidx.as<unsigned>());
-            if (ensure_shape_lut(ctx, pc.asw) || ctx->gmask.ensure((size_t) pg.R * 2)) return 1;
-            LAUNCH(ctx, k_group_masks, (nown + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, bd.r0, bd.r1, wb, (unsigned) plane,
-                   (int) pc.A, pst, win, ctx->shape.as<unsigned char>(), ctx->gmask.as<unsigned short>());
+            if (launch_group_masks(ctx, pc, win, pst, bd.r0, bd.r1)) return 1;
             if (clear_zero_blocks(ctx, pc) || launch_groups(ctx, pc, win, pst, partial, bd.r0, bd.r1)) return 1;
             if (launch_aggregate(ctx, pc, win, bd.pc1, bd.c1, bd.a0, bd.a1)) return 1;
         }
@@ -1197,7 +1195,9 @@ void lfbm5d_team_destroy(lfbm5d_team *T)
 int lfbm5d_team_local_ranks(lfbm5d_team *T) { return T ? (int) T->local.size() : 0; }
 
 /* Number of lanes of the team (>= 1): independent windows of a step (same level of the static plan) run concurrently, one per lane.
- * Every further lane has its own contexts (pass buffers: ~22 GB per lane at 17x17x1024^2) and exchange state. */
+ * Every further lane has its own contexts (pass buffers: ~22 GB per lane at 17x17x1024^2 with an = 1, about three times that with
+ * an = 2) and exchange state. Buffers are allocated at a lane's first pass; one that does not fit fails the step with the
+ * cudaMalloc error and its size. */
 int lfbm5d_team_set_lanes(lfbm5d_team *T, int nlanes)
 {
     if (!T || nlanes < 1 || nlanes > 8 || T->is_lane) return fail("bad lane count (1 .. 8)");
