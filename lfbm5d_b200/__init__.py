@@ -44,8 +44,7 @@ class Stats(C.Structure):
 EXPORTS = ["lfbm5d_create", "lfbm5d_destroy", "lfbm5d_last_error", "lfbm5d_reset_stats", "lfbm5d_get_stats",
            "lfbm5d_enable_timing", "lfbm5d_stream", "lfbm5d_step1", "lfbm5d_step2", "lfbm3d_run", "lfbm5d_step1_device",
            "lfbm5d_step2_device", "lfbm3d_run_device", "lfbm5d_set_max_passes", "lfbm5d_debug_pass", "lfbm5d_debug_pass_ex",
-           "lfbm5d_debug_schedule", "lfbm5d_step_begin", "lfbm5d_step_window", "lfbm5d_step_end", "lfbm5d_step_accumulators",
-           "lfbm5d_step_plan", "lfbm5d_step_force_sadct", "lfbm5d_step_window_ex", "lfbm5d_debug_block_matching", "lfbm5d_team_create_emulated", "lfbm5d_team_unique_id",
+           "lfbm5d_debug_schedule", "lfbm5d_step_plan", "lfbm5d_debug_block_matching", "lfbm5d_team_create_emulated", "lfbm5d_team_unique_id",
            "lfbm5d_team_create_nccl", "lfbm5d_team_destroy", "lfbm5d_team_local_ranks", "lfbm5d_team_step", "lfbm5d_team_band",
            "lfbm5d_team_stats", "lfbm5d_team_disable_peer_view", "lfbm5d_team_timing", "lfbm5d_team_plan_band", "lfbm5d_copy_rows", "lfbm5d_sync", "lfbm5d_team_use_peer_exchange", "lfbm5d_team_set_lanes", "lfbm5d_team_launches"]
 
@@ -247,35 +246,6 @@ class LFBM5D(object):
     def sync(self):
         if self.lib.lfbm5d_sync(self.ctx) != 0:
             raise RuntimeError("lfbm5d_sync: " + self.error())
-
-    # -- window-level entry points (see lfbm5d_b200/dist.py) -------------------------------------------
-    def step_begin(self, step, prm, d_noisy, d_basic, mask):
-        m = np.ascontiguousarray(mask, np.uint32)
-        if self.lib.lfbm5d_step_begin(self.ctx, int(step), C.byref(prm), C.c_void_p(d_noisy), C.c_void_p(d_basic or 0), _up(m)) != 0:
-            raise RuntimeError("lfbm5d_step_begin: " + self.error())
-
-    def step_window(self, ps, pt, sadct=None):
-        """sadct=None: sequential sticky rule; 0 / 1: the plan's value for this window (out-of-order drivers)."""
-        if sadct is None:
-            rc = self.lib.lfbm5d_step_window(self.ctx, int(ps), int(pt))
-        else:
-            rc = self.lib.lfbm5d_step_window_ex(self.ctx, int(ps), int(pt), int(sadct))
-        if rc != 0:
-            raise RuntimeError("lfbm5d_step_window: " + self.error())
-
-    def step_end(self, d_out):
-        if self.lib.lfbm5d_step_end(self.ctx, C.c_void_p(d_out)) != 0:
-            raise RuntimeError("lfbm5d_step_end: " + self.error())
-
-    def step_force_sadct(self):
-        self.lib.lfbm5d_step_force_sadct(self.ctx)
-
-    def step_accumulators(self):
-        """(device pointer of num, device pointer of den, floats per SAI) of the step in progress."""
-        pn, pd, each = C.c_void_p(), C.c_void_p(), C.c_size_t()
-        if self.lib.lfbm5d_step_accumulators(self.ctx, C.byref(pn), C.byref(pd), C.byref(each)) != 0:
-            raise RuntimeError("lfbm5d_step_accumulators: " + self.error())
-        return pn.value, pd.value, each.value
 
     def debug_block_matching(self, step, prm, planes):
         """planes [nplanes, hb, wb] channel-0 estimates (plane 0 = reference SAI) -> (count, idx, first, shape)."""

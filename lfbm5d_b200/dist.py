@@ -1,6 +1,6 @@
 """Host-side multi-GPU plumbing (one process per GPU, torch.distributed): SAI sharding for the per-SAI BM3D path
-(config 4: SAIs are independent, no data-path collective), light-field replicas for LFBM5D, and the max-over-ranks
-timing reduction the bench reports. Works with the gloo backend on CPU (tests) and nccl on GPUs."""
+(config 4: SAIs are independent, no data-path collective), the NCCL team that runs one LFBM5D light field on all ranks,
+and the max-over-ranks timing reduction the bench reports. Works with the gloo backend on CPU (tests) and nccl on GPUs."""
 import numpy as np
 
 
@@ -37,107 +37,6 @@ def max_over_ranks(value, dist, device="cpu"):
     t = torch.tensor([float(value)], dtype=torch.float64, device=device)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return float(t.item())
-
-
-# ---- one light field on several GPUs: window-level parallelism ---------------------------------------------------
-# The 3x3 angular windows of a step form a static schedule (lfbm5d_step_plan); windows that share no SAI commute. All ranks
-# hold the whole light field; ready windows are dealt out in rounds (plan_rounds), and before the next round the owner of
-# a window broadcasts the accumulators (num / den) of its SAIs. Every window sees exactly the accumulators it would see in the
-# sequential order, so the result is bit-identical to the single-GPU run. The dependency graph of a 17x17 light field has
-# 22 levels of width <= 4: at most 1.7x on 2 GPUs and 2.9x on >= 4 (DESIGN.md section 7).
-
-def plan_levels(plan):
-    """[[window rows of level 0], [level 1], ...] in schedule order."""
-    levels = [[] for _ in range(int(plan[:, 4].max()) + 1)] if len(plan) else []
-    for w in plan:
-        levels[int(w[4])].append(w)
-    return levels
-
-
-def plan_rounds(plan, prm, world):
-    """List scheduling of the window graph in rounds of at most `world` windows: a window is ready when every earlier window that
-    shares an SAI with it has run (in an earlier round); ready windows are taken in schedule order. 17x17: 34 rounds on 2 GPUs,
-    22 on >= 4 (level-synchronous rounds: 37 / 22)."""
-    asw = 2 * int(prm.an) + 1
-    box = [(int(w[2]), int(w[2]) + asw - 1, int(w[3]), int(w[3]) + asw - 1) for w in plan]
-
-    def overlap(a, b):
-        return not (a[1] < b[0] or b[1] < a[0] or a[3] < b[2] or b[3] < a[2])
-    deps = [[j for j in range(i) if overlap(box[i], box[j])] for i in range(len(plan))]
-    done, rounds, remaining = set(), [], list(range(len(plan)))
-    while remaining:
-        pick = [i for i in remaining if all(d in done for d in deps[i])][:max(1, int(world))]
-        rounds.append([plan[i] for i in pick])
-        done.update(pick)
-        remaining = [i for i in remaining if i not in done]
-    return rounds
-
-
-def sai_ranges(sais):
-    """Consecutive SAI indices as [lo, hi) ranges (the accumulators of consecutive SAIs are contiguous: fewer, larger broadcasts)."""
-    out = []
-    for st in sorted(sais):
-        if out and out[-1][1] == st:
-            out[-1][1] = st + 1
-        else:
-            out.append([st, st + 1])
-    return out
-
-
-def window_owner(level_windows, world):
-    """Round-robin owner rank of every window of one level."""
-    return [j % world for j in range(len(level_windows))]
-
-
-def window_sais(w, prm, mask):
-    """Global indices of the non-empty SAIs of a plan window."""
-    ROWMAJOR = 11
-    asw = 2 * int(prm.an) + 1
-    out = []
-    for s in range(int(w[2]), int(w[2]) + asw):
-        for t in range(int(w[3]), int(w[3]) + asw):
-            st = s * int(prm.awidth) + t if int(prm.ang_major) == ROWMAJOR else s + t * int(prm.aheight)
-            if mask[st]:
-                out.append(st)
-    return out
-
-
-class _DeviceArray(object):
-    def __init__(self, ptr, shape):
-        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f4", "data": (int(ptr), False), "version": 2}
-
-
-def run_step_windows(eng, step, prm, d_noisy, d_basic, mask, d_out, dist, device):
-    """One LFBM5D step of ONE light field on all ranks (NCCL). d_* are device pointers of this rank's copies of the light field
-    ([asize][C][H][W] floats, identical on all ranks on entry; d_out identical on all ranks on return)."""
-    import torch
-    from . import step_plan
-    rank, world = dist.get_rank(), dist.get_world_size()
-    mask = np.ascontiguousarray(mask, np.uint32)
-    plan = step_plan(prm, mask)
-    eng.step_begin(step, prm, d_noisy, d_basic, mask)
-    pn, pd, each = eng.step_accumulators()
-    asize = int(prm.awidth) * int(prm.aheight)
-    num = torch.as_tensor(_DeviceArray(pn, (asize, each)), device=device)
-    den = torch.as_tensor(_DeviceArray(pd, (asize, each)), device=device)
-    for wins in plan_rounds(plan, prm, world):
-        owners = window_owner(wins, world)
-        for w, o in zip(wins, owners):
-            if o == rank:
-                # the dct -> sadct switch comes from the plan entry: list scheduling runs windows out of their sequential order
-                eng.step_window(int(w[0]), int(w[1]), sadct=int(w[5]))
-        eng.step_accumulators()                      # waits for this rank's windows (the library has its own stream)
-        if world > 1:
-            works = []
-            for w, o in zip(wins, owners):
-                for lo, hi in sai_ranges(window_sais(w, prm, mask)):
-                    works.append(dist.broadcast(num[lo:hi], src=o, async_op=True))
-                    works.append(dist.broadcast(den[lo:hi], src=o, async_op=True))
-            for wk in works:
-                wk.wait()
-            torch.cuda.synchronize(device)
-    eng.step_end(d_out)
-    return plan
 
 
 # ---- one light field on several GPUs: parallelism inside a window (csrc/team.cuh) -------------------------------------------

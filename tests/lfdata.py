@@ -44,3 +44,24 @@ def synth_lf(aw, ah, H, W, C=3, disparity=1, seed=12345):
             oy, ox = pad_y + disparity * (s - cs), pad_x + disparity * (t - ct)
             out[s * aw + t] = base[:, oy:oy + H, ox:ox + W]
     return out
+
+
+def plan_levels(plan):
+    """Windows of a static plan (lfbm5d_step_plan rows) grouped by level: [[rows of level 0], [level 1], ...] in schedule order."""
+    levels = [[] for _ in range(int(plan[:, 4].max()) + 1)] if len(plan) else []
+    for w in plan:
+        levels[int(w[4])].append(w)
+    return levels
+
+
+def window_sais(w, prm, mask=None):
+    """Global indices of the SAIs of plan window w; with a mask only the non-empty ones."""
+    import lfbm5d_b200 as L
+    asw = 2 * int(prm.an) + 1
+    out = []
+    for s in range(int(w[2]), int(w[2]) + asw):
+        for t in range(int(w[3]), int(w[3]) + asw):
+            st = s * int(prm.awidth) + t if int(prm.ang_major) == L.ROWMAJOR else s + t * int(prm.aheight)
+            if mask is None or mask[st]:
+                out.append(st)
+    return out

@@ -6,15 +6,6 @@ import pytest
 import lfdata
 
 
-def _window_sais(w, prm, asw):
-    import lfbm5d_b200 as L
-    out = []
-    for s in range(int(w[2]), int(w[2]) + asw):
-        for t in range(int(w[3]), int(w[3]) + asw):
-            out.append(s * prm.awidth + t if prm.ang_major == L.ROWMAJOR else s + t * prm.aheight)
-    return out
-
-
 @pytest.mark.parametrize("aw,ah,holes,major", [
     (17, 17, (), "row"),
     (7, 7, (), "row"),
@@ -27,7 +18,6 @@ def test_step_plan_an2_matches_the_oracle_schedule(oracle, aw, ah, holes, major)
     """Same windows in the same order as the oracle's step driver at an = 2; windows of one plan level share no SAI; every SAI is
     covered; the sticky dct -> sadct switch starts at the first window that holds an empty SAI."""
     import lfbm5d_b200 as L
-    from lfbm5d_b200 import dist as D
     am = L.ROWMAJOR if major == "row" else L.COLMAJOR
     clean = lfdata.synth_lf(aw, ah, 12, 12)
     noisy = oracle.add_noise(clean, 10.0)
@@ -42,14 +32,14 @@ def test_step_plan_an2_matches_the_oracle_schedule(oracle, aw, ah, holes, major)
     if (aw, ah, holes) == (17, 17, ()):
         assert len(plan) == 25
     seen = np.zeros(aw * ah, bool)
-    for lvl in D.plan_levels(plan):
+    for lvl in lfdata.plan_levels(plan):
         used = []
         for w in lvl:
-            used += [st for st in _window_sais(w, prm, 5) if mask[st]]
+            used += lfdata.window_sais(w, prm, mask)
         assert len(used) == len(set(used))
         seen[used] = True
     assert np.array_equal(seen, mask.astype(bool))
-    with_hole = [i for i, w in enumerate(plan) if any(not mask[st] for st in _window_sais(w, prm, 5))]
+    with_hole = [i for i, w in enumerate(plan) if any(not mask[st] for st in lfdata.window_sais(w, prm))]
     expect = np.zeros(len(plan), np.uint32)
     if with_hole:
         expect[min(with_hole):] = 1

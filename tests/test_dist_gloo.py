@@ -53,7 +53,6 @@ def test_window_plan_matches_the_sequential_schedule(oracle):
     """lfbm5d_step_plan (static form of the reference's window selection) against the schedule the oracle's step driver takes
     (itself bit-identical to the reference), with and without empty SAIs; windows of one level share no SAI."""
     import lfbm5d_b200 as L
-    from lfbm5d_b200 import dist as D
     import lfdata
     for (aw, ah, holes, major) in [(5, 5, (), L.ROWMAJOR), (7, 5, (3, 17), L.ROWMAJOR), (6, 4, (23,), L.COLMAJOR)]:
         clean = lfdata.synth_lf(aw, ah, 12, 12)
@@ -67,39 +66,16 @@ def test_window_plan_matches_the_sequential_schedule(oracle):
         assert len(plan) == len(sched)
         assert np.array_equal(plan[:, 2:4], sched[:, 1:3])                       # same windows in the same order
         seen = np.zeros(aw * ah, bool)
-        for lvl in D.plan_levels(plan):
+        for lvl in lfdata.plan_levels(plan):
             used = []
             for w in lvl:
-                used += D.window_sais(w, prm, mask)
+                used += lfdata.window_sais(w, prm, mask)
             assert len(used) == len(set(used))                                   # windows of a level are disjoint
             seen[used] = True
         assert np.array_equal(seen, mask.astype(bool))
         if holes:                                                               # sticky dct -> sadct switch from the first window with a hole
-            first = min(i for i, w in enumerate(plan) if any(not mask[st] for st in _window_all(w, prm)))
+            first = min(i for i, w in enumerate(plan) if any(not mask[st] for st in lfdata.window_sais(w, prm)))
             assert np.array_equal(plan[:, 5], (np.arange(len(plan)) >= first).astype(np.uint32))
-        for world in (1, 2, 3, 8):                                                # list scheduling: every window once, dependencies first
-            order = {}
-            for ri, rnd in enumerate(D.plan_rounds(plan, prm, world)):
-                assert 1 <= len(rnd) <= world
-                for w in rnd:
-                    order[(int(w[2]), int(w[3]))] = ri
-            assert len(order) == len(plan)
-            for i, wi in enumerate(plan):
-                for wj in plan[:i]:
-                    if set(_window_all(wi, prm)) & set(_window_all(wj, prm)):
-                        assert order[(int(wj[2]), int(wj[3]))] < order[(int(wi[2]), int(wi[3]))]
-        assert D.sai_ranges([4, 5, 6, 9, 11, 12]) == [[4, 7], [9, 10], [11, 13]]
-        owners = [D.window_owner(lvl, 3) for lvl in D.plan_levels(plan)]
-        assert all(o == list(range(len(o))) or max(o) < 3 for o in owners)
-
-
-def _window_all(w, prm):
-    import lfbm5d_b200 as L
-    out = []
-    for s in range(int(w[2]), int(w[2]) + 3):
-        for t in range(int(w[3]), int(w[3]) + 3):
-            out.append(s * int(prm.awidth) + t if int(prm.ang_major) == L.ROWMAJOR else s + t * int(prm.aheight))
-    return out
 
 
 def _band_worker(rank, world, port, ret):

@@ -116,6 +116,7 @@ def test_team_lanes_run_independent_windows_concurrently(world, lanes, oracle):
     eng = L.LFBM5D(0)
     w0, b0, o0, s0 = run_single(L, eng, torch, noisy, mask, p1, p2)
     eng.close()
+    assert np.array_equal(plan[:, 2:4], s0[:, 1:3])                           # the plan's windows are the sequential schedule's
     ws, bs, outs, bands1, bands2, st = run_team(L, torch, world, noisy, mask, p1, p2, gather=1, lanes=lanes)
     for g in range(world):
         assert torch.equal(outs[g], o0), "denoised differs on rank %d" % g
