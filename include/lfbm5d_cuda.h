@@ -34,7 +34,9 @@ typedef struct lfbm5d_params {
                              * 25-SAI group in the shared memory of one CTA): k = 16 with N <= 8 / N <= 4, k = 8 with N <= 32 / N <= 16 */
     unsigned width, height, chnls;
     unsigned N;             /* NHard / NWien */
-    unsigned nSim, nDisp;
+    unsigned nSim;          /* half size of the self search window */
+    unsigned nDisp;         /* half size of the disparity search window, <= 16 ((2nDisp+1)^2 offsets per SAI of the window).
+                             * The SAIs must be at least nSim + nDisp pixels high and wide (mirror padding) */
     unsigned k;             /* kHard / kWien */
     unsigned p;             /* pHard / pWien */
     unsigned useSD;

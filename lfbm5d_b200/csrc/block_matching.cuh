@@ -847,7 +847,7 @@ __global__ void __launch_bounds__(128) k_bm_select_fast(SelGeom g, const float *
 
 // ------------------------------------------------------------------------------------------------------------
 // Disparity matching (core:3576-3608): one thread per position, walking the skewed layout k_sat2 writes so that
-// the 169 plane reads are coalesced. Only element [0] of the sorted list and the shape flag are consumed
+// the (2*nDisp+1)^2 plane reads are coalesced. Only element [0] of the sorted list and the shape flag are consumed
 // downstream (core:294, 310, 503, 510); the full std::sort is emulated only where the minimum is tied.
 // ------------------------------------------------------------------------------------------------------------
 __global__ void k_stereo_argmin(const float *__restrict__ sums, size_t plane_stride, int w, int nDisp, int lo, int row_end, int col_end,
@@ -879,11 +879,13 @@ __global__ void k_stereo_argmin(const float *__restrict__ sums, size_t plane_str
 }
 
 // Positions whose minimum distance is tied (mirror-symmetric borders, flat regions): one thread per listed position runs the
-// re-implemented libstdc++ std::sort on the (distance, index) pairs in the reference's push order (core:3590-3606).
+// re-implemented libstdc++ std::sort on the (distance, index) pairs in the reference's push order (core:3590-3606). Each thread
+// keeps its (2*nDisp+1)^2 pairs in dynamic shared memory; the host sizes the CTA to fit them.
 struct TieGeom {
     size_t plane_stride;
     int w, nDisp, lo, nstrips, SR;
     unsigned plane;                     // w * h
+    int nbuf;                           // stereo slots the sums buffer holds: slot s sits at s % nbuf
     int sai[LF_MAXA];                   // window slot of every stereo slot
 };
 __global__ void k_stereo_ties(TieGeom g, const float *__restrict__ sums, const uint2 *__restrict__ tie_list, const unsigned *__restrict__ tie_count,
@@ -899,11 +901,11 @@ __global__ void k_stereo_ties(TieGeom g, const float *__restrict__ sums, const u
         const int strip = (int) (rs / g.SR), sidx = (int) (rs - (size_t) strip * g.SR);
         const int i = g.lo + sidx - lane, j = g.lo + (strip << 5) + lane;
         const int k_r = i * g.w + j;
-        const float *sp = sums + (size_t) en.x * np * g.plane_stride + t;
+        const float *sp = sums + (size_t) (en.x % (unsigned) g.nbuf) * np * g.plane_stride + t;
         // the pairs live in shared memory: the emulated sort is a chain of dependent accesses (one thread per position, few
         // positions), its time is memory latency
         extern __shared__ LfPair s_td[];
-        LfPair *td = s_td + (size_t) threadIdx.x * LF_MAXNS2;
+        LfPair *td = s_td + (size_t) threadIdx.x * np;
         int c = 0;
         for (int djx = 0; djx < Ns; ++djx)
             for (int dix = 0; dix < Ns; ++dix, ++c) {

@@ -13,7 +13,7 @@
 #define LF_LUTASW    3
 #define LF_LUTA      (LF_LUTASW * LF_LUTASW)
 #define LF_MAXN      32      // largest number of similar patches
-#define LF_MAXNS2    169     // (2*nDisp+1)^2, nDisp <= 6
+#define LF_MAXDISP   16      // largest disparity half window nDisp: (2*nDisp+1)^2 <= 1089 disparity offsets
 #define LF_SQRT2_INV_F ((float) 0.7071067811865475)
 #define LF_SQRT2_F     ((float) 1.414213562373095)
 

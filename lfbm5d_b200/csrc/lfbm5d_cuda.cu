@@ -124,7 +124,9 @@ struct SatPlan {
     std::vector<SatPlane> planes;
     std::vector<SatGroup> groups;
     std::vector<int> stereo_sai;        // window slot of every stereo slot
-    int nself_groups = 0, nself_planes = 0, nslots = 0, groups_per_slot = 0;
+    int nself_groups = 0, nself_planes = 0, nslots = 0;
+    int groups_per_slot = 0, planes_per_slot = 0;      // Nd * ceil(Nd / 14) groups, Nd^2 planes
+    int nbuf = 0;                       // stereo slots the sums buffer holds (stereo_buffer_slots): slot s sits at s % nbuf
     int st_lo = 0, st_row_end = 0, st_col_end = 0, st_strips = 0, st_SR = 0;
     size_t st_stride = 0;
     int self_row_end = 0, self_col_end = 0, self_strips = 0, pstrips = 1;
@@ -345,6 +347,7 @@ struct lfbm5d_ctx {
     cudaStream_t stream3 = nullptr;                       // disparity matching of a pass, beside the self matching on `stream`
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_satb = nullptr;
     int num_sms = 148;
+    int smem_optin = 0;            // opt-in shared memory per block (bytes)
     DevBuf noisy, basic, out, num, den, mask;
     DevBuf nsym, bsym, numsym, densym, est0;
     DevBuf s_at, s_mir, sums, first, shape, bmcount, bmidx, bnd, progress, rowmap, colmap, rows, cols, counters,
@@ -395,7 +398,7 @@ int validate(const lfbm5d_params *p, int step)
     if (asw > LF_MAXASW) return fail("angular half window an > 2 is not supported by this build (an must be 0, 1 or 2)");
     if (p->k != 8 && p->k != 16) return fail("patch size must be 8 or 16 in this build");
     if (p->N == 0 || p->N > LF_MAXN || (p->N & (p->N - 1))) return fail("N must be a power of two <= 32");
-    if (p->nDisp > 6) return fail("nDisp > 6 is not supported by this build");
+    if (p->nDisp > LF_MAXDISP) return fail("nDisp > 16 is not supported by this build (nDisp must be <= 16)");
     if (p->nSim + p->nDisp + 1 < p->k) return fail("nSim + nDisp must be >= k - 1");
     if (p->p == 0) return fail("processing step must be >= 1");
     if (p->tau_2D != LFBM5D_ID && p->tau_2D != LFBM5D_DCT && p->tau_2D != LFBM5D_BIOR) return fail("tau_2D must be id, dct or bior");
@@ -546,6 +549,14 @@ int upload_grid(lfbm5d_ctx *ctx, const PassCfg &pc)
     return 0;
 }
 
+// Stereo slots the disparity sums buffer holds: as many as (A - 1) slots of 13^2 planes (nDisp = 6) take, at least one, at most
+// A - 1. Wider disparity windows run the slots of a pass in chunks of this many (launch_stereo).
+int stereo_buffer_slots(const PassCfg &pc)
+{
+    const int Nd = 2 * (int) pc.nDisp + 1, A1 = (int) pc.A - 1;
+    return std::min(A1, std::max(1, A1 * 169 / (Nd * Nd)));
+}
+
 int ensure_pass_buffers(lfbm5d_ctx *ctx, const PassCfg &pc)
 {
     const size_t plane = (size_t) pc.wb * pc.hb, R = pc.rows.size() * pc.cols.size();
@@ -557,9 +568,11 @@ int ensure_pass_buffers(lfbm5d_ctx *ctx, const PassCfg &pc)
     // stereo sums in the skewed layout of k_sat2: [plane][strip][SR][32]
     const size_t st_cols = pc.wb - 2 * pc.nDisp - pc.k + 1, st_rows = pc.hb - 2 * pc.nDisp - pc.k + 1;
     const size_t st_strips = (st_cols + 31) / 32, st_SR = st_rows + 31;
-    if (pc.A > 1 && ctx->sums.ensure((pc.A - 1) * Nd * Nd * st_strips * st_SR * 32 * 4)) return 1;
+    if (pc.A > 1 && ctx->sums.ensure((size_t) stereo_buffer_slots(pc) * Nd * Nd * st_strips * st_SR * 32 * 4)) return 1;
     if (ctx->first.ensure(pc.A * plane * 4) || ctx->shape.ensure(pc.A * plane)) return 1;
     if (ctx->bmcount.ensure(R * 4) || ctx->bmidx.ensure(R * (pc.N + 1) * 4)) return 1;
+    // hand-off words and first row / column are indexed by plane id, unique within a pass even where the chunks of the sums buffer
+    // reuse its memory: a word one chunk tagged under this epoch is never at an address the next chunk polls
     const size_t nplanes = nself + (pc.A - 1) * Nd * Nd;
     const size_t max_strips = std::max(st_strips, (size_t) (pc.wb - 2 * pc.n + 31) / 32);
     {   // hand-off words of k_sat2: a fresh buffer holds no valid tag (epochs start at 1)
@@ -672,24 +685,32 @@ SatPlan *sat_plan(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     P.st_col_end = partial ? std::min(st_col_full, act_xmax + (int) pc.nSim + 1) : st_col_full;
     P.st_strips = (P.st_col_end - P.st_lo + 31) / 32; P.st_SR = (P.st_row_end - P.st_lo) + 31;
     P.st_stride = (size_t) ((st_col_full - P.st_lo + 31) / 32) * ((st_row_full - P.st_lo) + 31) * 32;      // allocation: full planes
-    P.groups_per_slot = Nd;
+    // a row offset's Nd column offsets split into ngx balanced groups of <= 14 consecutive ones (one group up to nDisp = 6);
+    // plane ids stay [slot][di][dj]
+    const int ngx = (Nd + 2 * SAT_NW - 1) / (2 * SAT_NW);
+    P.groups_per_slot = Nd * ngx; P.planes_per_slot = pg.nd2;
+    P.nbuf = pc.A > 1 ? stereo_buffer_slots(pc) : 1;
     int slot = 0;
     for (int st = 0; st < (int) pc.A; st++) {
         if (st == pst || !win.mask[st]) continue;
-        for (int di = 0; di < Nd; di++) {      // core:3516: dk = (di - nDisp)*w + (dj - nDisp)
-            SatGroup G{};
-            G.img1 = ref0; G.img2 = est0 + (size_t) st * pg.plane; G.oy = di - (int) pc.nDisp; G.oxmin = -(int) pc.nDisp;
-            G.z1 = pst; G.z2 = st;
-            G.first_plane = (int) P.planes.size();
-            for (int dj = 0; dj < Nd; dj++) {
-                SatPlane Q{};
-                Q.ox = dj - (int) pc.nDisp;
-                Q.out_skew = ctx->sums.as<float>() + ((size_t) slot * pg.nd2 + (size_t) di * Nd + dj) * P.st_stride;
-                P.planes.push_back(Q);
-                G.nplanes++;
+        const size_t bslot = (size_t) (slot % P.nbuf);
+        for (int di = 0; di < Nd; di++)      // core:3516: dk = (di - nDisp)*w + (dj - nDisp)
+            for (int gx = 0, dj0 = 0; gx < ngx; gx++) {
+                const int dj1 = dj0 + Nd / ngx + (gx < Nd % ngx ? 1 : 0);
+                SatGroup G{};
+                G.img1 = ref0; G.img2 = est0 + (size_t) st * pg.plane; G.oy = di - (int) pc.nDisp; G.oxmin = dj0 - (int) pc.nDisp;
+                G.z1 = pst; G.z2 = st;
+                G.first_plane = (int) P.planes.size();
+                for (int dj = dj0; dj < dj1; dj++) {
+                    SatPlane Q{};
+                    Q.ox = dj - (int) pc.nDisp;
+                    Q.out_skew = ctx->sums.as<float>() + (bslot * pg.nd2 + (size_t) di * Nd + dj) * P.st_stride;
+                    P.planes.push_back(Q);
+                    G.nplanes++;
+                }
+                P.groups.push_back(G);
+                dj0 = dj1;
             }
-            P.groups.push_back(G);
-        }
         P.stereo_sai.push_back(st);
         slot++;
     }
@@ -855,18 +876,42 @@ int launch_stereo_argmin(lfbm5d_ctx *ctx, const PassCfg &pc, const SatPlan &P, i
     CK(cudaMemsetAsync(sc, 0, 4, strm));
     TieGeom tg{};
     tg.plane_stride = P.st_stride; tg.w = (int) pc.wb; tg.nDisp = (int) pc.nDisp; tg.lo = P.st_lo; tg.nstrips = P.st_strips; tg.SR = P.st_SR;
-    tg.plane = (unsigned) pg.plane;
+    tg.plane = (unsigned) pg.plane; tg.nbuf = P.nbuf;
     for (int s = 0; s < P.nslots; s++) tg.sai[s] = P.stereo_sai[s];
     for (int s = s0; s < s1; s++) {
         const int st = P.stereo_sai[s];
-        LAUNCH_ON(ctx, strm, k_stereo_argmin, grid_for(ctx, P.st_stride, 128), 128, 0, ctx->sums.as<float>() + (size_t) s * pg.nd2 * P.st_stride, P.st_stride,
+        LAUNCH_ON(ctx, strm, k_stereo_argmin, grid_for(ctx, P.st_stride, 128), 128, 0,
+                  ctx->sums.as<float>() + (size_t) (s % P.nbuf) * pg.nd2 * P.st_stride, P.st_stride,
                   (int) pc.wb, (int) pc.nDisp, P.st_lo, P.st_row_end, P.st_col_end, P.st_strips, P.st_SR, pg.threshold,
                   ctx->first.as<unsigned>() + (size_t) st * pg.plane, ctx->shape.as<unsigned char>() + (size_t) st * pg.plane, (unsigned) s, sl, sc);
     }
-    const size_t smem_t = (size_t) 32 * LF_MAXNS2 * sizeof(LfPair);
+    // Nd^2 pairs per thread in shared memory: 32 threads per CTA up to nDisp = 6, fewer where a CTA of 32 lists does not fit
+    const size_t pair_bytes = (size_t) pg.nd2 * sizeof(LfPair);
+    const int nt = (int) std::min<size_t>(32, (size_t) ctx->smem_optin / pair_bytes);
+    if (nt < 1) return fail("k_stereo_ties: one sort list of " + std::to_string(pair_bytes) + " bytes exceeds the shared memory of a block");
+    const size_t smem_t = (size_t) nt * pair_bytes;
     CK(cudaFuncSetAttribute((const void *) k_stereo_ties, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_t));
-    LAUNCH_ON(ctx, strm, k_stereo_ties, ctx->num_sms * 4, 32, smem_t, tg, ctx->sums.as<float>(), (const uint2 *) sl, (const unsigned *) sc,
+    LAUNCH_ON(ctx, strm, k_stereo_ties, ctx->num_sms * 4, nt, smem_t, tg, ctx->sums.as<float>(), (const uint2 *) sl, (const unsigned *) sc,
               ctx->first.as<unsigned>());
+    return 0;
+}
+
+// Disparity matching of the slots [s0, s1) on strm: planes, argmin and ties, in chunks of P.nbuf slots, the slots the sums buffer
+// holds. Each chunk's tie kernel is ordered before the next chunk's planes overwrite the buffer (same stream). between() runs once
+// the first chunk's planes are enqueued: the caller's self matching on the other stream then starts behind them. planes_done (if
+// set) is recorded on strm behind the last chunk's planes.
+template <class F>
+int launch_stereo(lfbm5d_ctx *ctx, const PassCfg &pc, const SatPlan &P, int s0, int s1, cudaStream_t strm, cudaEvent_t planes_done, F between)
+{
+    for (int c0 = s0; c0 < s1 || c0 == s0; c0 += P.nbuf) {
+        const int c1 = std::min(s1, c0 + P.nbuf);
+        // a launch on a used ticket counter hands out no work: the second and later chunks reset theirs (the pass reset the first)
+        if (c0 > s0) CK(cudaMemsetAsync(ctx->progress.as<int>() + 1, 0, 4, strm));
+        if (launch_sat_stereo(ctx, pc, P, c0, c1, strm)) return 1;
+        if (planes_done && c1 >= s1) CK(cudaEventRecord(planes_done, strm));
+        if (c0 == s0 && between()) return 1;
+        if (launch_stereo_argmin(ctx, pc, P, c0, c1, strm)) return 1;
+    }
     return 0;
 }
 
@@ -1030,18 +1075,19 @@ int run_pass(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, i
     CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
     CK(cudaStreamWaitEvent(sB, ctx->ev_fork, 0));
     // the disparity planes are launched first: they finish first and their argmin then runs under the self planes
-    if (launch_sat_stereo(ctx, pc, P, 0, P.nslots, sB)) return 1;
-    if (pg.nself > 0) {
-        LAUNCH(ctx, k_fill, grid_for(ctx, (size_t) pg.nself * R), 256, 0, ctx->s_mir.as<float>(), 2 * pg.threshold, (size_t) pg.nself * R);   // core:3317
-        if (launch_sat_self(ctx, pc, P, 0, P.nself_groups, ctx->stream)) return 1;
-    }
-    if (ctx->timing) { CK(cudaEventRecord(sat1, ctx->stream)); CK(cudaEventRecord(ctx->ev_satb, sB)); }
-    // ---- selection ----
-    if (pg.nself > 0) { if (launch_self_select(ctx, pc, ctx->stream)) return 1; }
-    else
-        LAUNCH(ctx, k_bm_identity, (R + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, (int) pc.wb, R, (int) pc.N,
-               ctx->bmcount.as<unsigned>(), ctx->bmidx.as<unsigned>());
-    if (launch_stereo_argmin(ctx, pc, P, 0, P.nslots, sB)) return 1;
+    if (launch_stereo(ctx, pc, P, 0, P.nslots, sB, ctx->timing ? ctx->ev_satb : nullptr, [&]() -> int {
+            if (pg.nself > 0) {
+                LAUNCH(ctx, k_fill, grid_for(ctx, (size_t) pg.nself * R), 256, 0, ctx->s_mir.as<float>(), 2 * pg.threshold, (size_t) pg.nself * R);   // core:3317
+                if (launch_sat_self(ctx, pc, P, 0, P.nself_groups, ctx->stream)) return 1;
+            }
+            if (ctx->timing) CK(cudaEventRecord(sat1, ctx->stream));
+            // ---- selection ----
+            if (pg.nself > 0) { if (launch_self_select(ctx, pc, ctx->stream)) return 1; }
+            else
+                LAUNCH(ctx, k_bm_identity, (R + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, (int) pc.wb, R, (int) pc.N,
+                       ctx->bmcount.as<unsigned>(), ctx->bmidx.as<unsigned>());
+            return 0;
+        })) return 1;
     CK(cudaEventRecord(ctx->ev_join, sB));
     CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
     if (launch_group_masks(ctx, pc, win, (int) pst, 0, R)) return 1;
@@ -1063,7 +1109,7 @@ int run_pass(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, i
         cudaEventElapsedTime(&a, ctx->ev[0], ctx->ev[1]);
         cudaEventElapsedTime(&b, ctx->ev[1], ctx->ev[4]);
         cudaEventElapsedTime(&c, sat0, sat1);
-        { float cb = 0.f; cudaEventElapsedTime(&cb, sat0, ctx->ev_satb); c = std::max(c, cb); }      // both plane kernels done
+        { float cb = 0.f; cudaEventElapsedTime(&cb, sat0, ctx->ev_satb); c = std::max(c, cb); }      // both plane kernels done (several chunks: the last chunk's planes, earlier chunks' argmin included)
         cudaEventElapsedTime(&d, ctx->ev[4], e2);
         ctx->stats.ms_block_matching += a; ctx->stats.ms_groups += b; ctx->stats.ms_sat += c; ctx->stats.ms_aggregate += d;
         cudaEventDestroy(e2);
@@ -1360,6 +1406,7 @@ int lfbm5d_create(lfbm5d_ctx **out, int device)
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     ctx->num_sms = prop.multiProcessorCount;
+    ctx->smem_optin = (int) prop.sharedMemPerBlockOptin;
     CK(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     CK(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
     CK(cudaStreamCreateWithFlags(&ctx->stream3, cudaStreamNonBlocking));

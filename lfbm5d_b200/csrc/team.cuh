@@ -272,12 +272,12 @@ std::vector<Band> team_bands(const PassCfg &pc, int G)
     return B;
 }
 
-// Deal the offset planes of a pass out: disparity slots evenly (whole SAIs: their argmin needs all 169 planes), then the self
+// Deal the offset planes of a pass out: disparity slots evenly (whole SAIs: their argmin needs all (2 nDisp + 1)^2 planes), then the self
 // groups in contiguous runs so that every rank ends up with about the same number of planes.
 std::vector<PlaneShare> team_planes(const SatPlan &P, int G)
 {
     std::vector<PlaneShare> S(G);
-    const int per_slot = P.groups_per_slot * P.groups_per_slot;      // planes of a disparity slot
+    const int per_slot = P.planes_per_slot;
     const double total = (double) P.nself_planes + (double) P.nslots * per_slot;
     int sg = 0;
     double cum = 0.0;
@@ -349,32 +349,33 @@ int team_pass_bm(lfbm5d_team *T, const PassCfg &pc, const LfWindow &win, int pst
         CK(cudaStreamWaitEvent(sB, ctx->ev_fork, 0));
         const bool tm = T->timing && l == 0;
         if (tm) CK(cudaEventRecord(T->bev[0], ctx->stream));
-        if (launch_sat_stereo(ctx, pc, P, sh.s0, sh.s1, sB)) return 1;
-        if (tm) CK(cudaEventRecord(T->bev[3], sB));
-        if (pg.nself > 0 && sh.pl1 > sh.pl0) {
-            LAUNCH(ctx, k_fill, grid_for(ctx, (size_t) (sh.pl1 - sh.pl0) * pg.R), 256, 0, ctx->s_mir.as<float>() + (size_t) sh.pl0 * pg.R, 2 * pg.threshold,
-                   (size_t) (sh.pl1 - sh.pl0) * pg.R);   // core:3317
-            if (launch_sat_self(ctx, pc, P, sh.sg0, sh.sg1, ctx->stream)) return 1;
-        }
-        if (tm) CK(cudaEventRecord(T->bev[1], ctx->stream));
-        if (pg.nself > 0) {
-            SelGeom sg{};
-            sg.w = pc.wb; sg.nSim = pc.nSim; sg.Ns = pg.Ns; sg.N = pc.N; sg.R = pg.R; sg.nc = pg.nc; sg.threshold = pg.threshold;
-            sg.rows = ctx->rows.as<int>(); sg.cols = ctx->cols.as<int>();
-            TeamCtxBufs *b = team_bufs(ctx);
-            void (*kp)(SelGeom, const float *, const float *, int, int, unsigned *, unsigned long long *) = nullptr;
-            switch (pc.N) {
-                case 2: kp = k_bm_partial<3>; break;
-                case 4: kp = k_bm_partial<5>; break;
-                case 8: kp = k_bm_partial<9>; break;
-                case 16: kp = k_bm_partial<17>; break;
-                default: kp = k_bm_partial<33>; break;
-            }
-            LAUNCH(ctx, kp, (pg.R + 127) / 128, 128, 0, sg, ctx->s_at.as<float>(), ctx->s_mir.as<float>(), sh.pl0, sh.pl1, b->pcnt_send.as<unsigned>(),
-                   b->pkey_send.as<unsigned long long>());
-        }
-        if (tm) CK(cudaEventRecord(T->bev[2], ctx->stream));
-        if (launch_stereo_argmin(ctx, pc, P, sh.s0, sh.s1, sB)) return 1;
+        // own disparity slots in chunks of the sums buffer, counted from sh.s0 (slot s still sits at s % nbuf)
+        if (launch_stereo(ctx, pc, P, sh.s0, sh.s1, sB, tm ? T->bev[3] : nullptr, [&]() -> int {
+                if (pg.nself > 0 && sh.pl1 > sh.pl0) {
+                    LAUNCH(ctx, k_fill, grid_for(ctx, (size_t) (sh.pl1 - sh.pl0) * pg.R), 256, 0, ctx->s_mir.as<float>() + (size_t) sh.pl0 * pg.R,
+                           2 * pg.threshold, (size_t) (sh.pl1 - sh.pl0) * pg.R);   // core:3317
+                    if (launch_sat_self(ctx, pc, P, sh.sg0, sh.sg1, ctx->stream)) return 1;
+                }
+                if (tm) CK(cudaEventRecord(T->bev[1], ctx->stream));
+                if (pg.nself > 0) {
+                    SelGeom sg{};
+                    sg.w = pc.wb; sg.nSim = pc.nSim; sg.Ns = pg.Ns; sg.N = pc.N; sg.R = pg.R; sg.nc = pg.nc; sg.threshold = pg.threshold;
+                    sg.rows = ctx->rows.as<int>(); sg.cols = ctx->cols.as<int>();
+                    TeamCtxBufs *b = team_bufs(ctx);
+                    void (*kp)(SelGeom, const float *, const float *, int, int, unsigned *, unsigned long long *) = nullptr;
+                    switch (pc.N) {
+                        case 2: kp = k_bm_partial<3>; break;
+                        case 4: kp = k_bm_partial<5>; break;
+                        case 8: kp = k_bm_partial<9>; break;
+                        case 16: kp = k_bm_partial<17>; break;
+                        default: kp = k_bm_partial<33>; break;
+                    }
+                    LAUNCH(ctx, kp, (pg.R + 127) / 128, 128, 0, sg, ctx->s_at.as<float>(), ctx->s_mir.as<float>(), sh.pl0, sh.pl1,
+                           b->pcnt_send.as<unsigned>(), b->pkey_send.as<unsigned long long>());
+                }
+                if (tm) CK(cudaEventRecord(T->bev[2], ctx->stream));
+                return 0;
+            })) return 1;
         if (tm) CK(cudaEventRecord(T->bev[4], sB));
         CK(cudaEventRecord(ctx->ev_join, sB));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
