@@ -37,7 +37,9 @@ typedef struct lfbm5d_params {
     unsigned nSim;          /* half size of the self search window */
     unsigned nDisp;         /* half size of the disparity search window, <= 16 ((2nDisp+1)^2 offsets per SAI of the window).
                              * The SAIs must be at least nSim + nDisp pixels high and wide (mirror padding) */
-    unsigned k;             /* kHard / kWien */
+    unsigned k;             /* kHard / kWien: patch side, 8, 12 or 16. k = 12 takes tau_2D = id or dct (bior needs a power of two),
+                             * an = 0 or 1, and N * A * k * (k + 1) * 4 B <= 220 KB (twice that in step 2; A = (2an+1)^2):
+                             * at an = 1, N <= 32 in step 1 and N <= 16 in step 2 */
     unsigned p;             /* pHard / pWien */
     unsigned useSD;
     unsigned tau_2D, tau_4D, tau_5D;
@@ -50,7 +52,7 @@ typedef struct lfbm3d_params {
     float    sigma;
     unsigned asize;         /* number of SAIs */
     unsigned width, height, chnls;
-    unsigned nHard, nWien, kHard, kWien, NHard, NWien, pHard, pWien;
+    unsigned nHard, nWien, kHard, kWien, NHard, NWien, pHard, pWien;     /* kHard, kWien: 8, 12 or 16; 12 with dct only */
     unsigned useSD_h, useSD_w;
     unsigned tau_2D_hard, tau_2D_wien;
     float    lambdaHard3D;

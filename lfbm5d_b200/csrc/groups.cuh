@@ -602,18 +602,28 @@ __global__ void k_group_masks32(const int *__restrict__ rows, const int *__restr
     lf_group_mask(rows, cols, nc, r0, r1, w, plane, A, pst, win, shape, gmask);
 }
 
-template <int STEP, int ASW>
-__global__ void __launch_bounds__(256) k_groups(GroupArgs g)
+// k = 12 (k_groups12): 288 threads, two patches of 144 positions per sweep. validate() keeps the group of one channel
+// (N * A * k * (k + 1) floats, twice that in step 2) within LF_G12_SMEM bytes of dynamic shared memory.
+#define LF_G12_NT 288
+#define LF_G12_SMEM (220 * 1024)
+
+// 2-D transform of the group kernels: K = 0 dispatches on g.k (8 or 16); k = 12 takes id or dct (validate())
+template <int K> __device__ __forceinline__ void lf_t2d_k(float *B, int npatch, const GroupArgs &g, bool fwd)
 {
-    extern __shared__ float smem[];
-    __shared__ GroupShape sh;
-    __shared__ float red[8];
-    __shared__ unsigned sofs[LF_MAXN * LF_LUTA];          // per gathered patch: st*C*plane + position
-    __shared__ unsigned char szero[LF_MAXN * LF_LUTA];    // patch reads as zeros (empty SAI, or column w-k: core:1697)
+    if (K == 0) lf_t2d(B, npatch, g, fwd);
+    else if (g.tau_2D == 5) lf_dct2d<K ? K : 8>(B, npatch, g.RS, g.PS, fwd);
+}
+
+// Body of the generic group kernels. K = 0: k = 8 or 16 from the arguments, 256 threads (k_groups); K = 12: LF_G12_NT threads
+// (k_groups12). The kernels declare the shared arrays (smem: the dynamic one): an extern declaration in this function would
+// move the module's first extern shared array, and with it the dynamic shared-memory base of other kernels (k_groups25).
+template <int STEP, int ASW, int K>
+__device__ __forceinline__ void lf_groups_body(const GroupArgs &g, float *smem, GroupShape &sh, float *red, unsigned *sofs, unsigned char *szero)
+{
     constexpr int A = ASW * ASW;
     const int tid = threadIdx.x;
     const int r = blockIdx.x + g.r0;
-    const int k = g.k, k2 = k * k, w = g.w;
+    const int k = K ? K : g.k, k2 = k * k, w = g.w;
     const unsigned plane = (unsigned) g.w * (unsigned) g.h;
     const int nSx = (int) g.bm_count[r];
     const int lg = 31 - __clz(nSx);
@@ -621,9 +631,9 @@ __global__ void __launch_bounds__(256) k_groups(GroupArgs g)
     float *X = smem;
     float *E = smem + (size_t) g.N * A * PS;      // step 2 only (N >= nSx except the duplicated single match: N >= 2)
     // thread <-> (sub, pq): a thread keeps its pixel/coefficient position and strides over patches
-    const int PPI = 256 >> (2 * g.log2k);          // patches handled per sweep of the block (1 for k = 16, 4 for k = 8)
-    const int sub = tid >> (2 * g.log2k), pq = tid & (k2 - 1);
-    const int p = pq >> g.log2k, q = pq & (k - 1);
+    const int PPI = K ? LF_G12_NT / (K * K) : 256 >> (2 * g.log2k);     // patches handled per sweep of the block (1 for k = 16, 2 for k = 12, 4 for k = 8)
+    const int sub = K ? tid / (K * K) : tid >> (2 * g.log2k), pq = K ? tid - sub * (K * K) : tid & (k2 - 1);
+    const int p = K ? pq / K : pq >> g.log2k, q = K ? pq - p * K : pq & (k - 1);
     const int poff = p * RS + q;
     const int npatch = nSx * A;
     if (!lf_group_setup<false>(g, r, nSx, sh, sofs, szero)) return;
@@ -651,8 +661,8 @@ __global__ void __launch_bounds__(256) k_groups(GroupArgs g)
         }
         __syncthreads();
         // ---- 2-D spatial transform; patches that read as zeros stay zero under any of the transforms ----
-        lf_t2d(X, npatch, g, true);
-        if (STEP == 2) lf_t2d(E, npatch, g, true);
+        lf_t2d_k<K>(X, npatch, g, true);
+        if (STEP == 2) lf_t2d_k<K>(E, npatch, g, true);
         // ---- angular transform (core:354-360) ----
         if (g.tau_4D != 4) {
             for (int n = sub; n < nSx; n += PPI) {
@@ -729,12 +739,34 @@ __global__ void __launch_bounds__(256) k_groups(GroupArgs g)
             __syncthreads();
         }
         // ---- inverse 2-D transform (core:489-493) ----
-        lf_t2d(Z, npatch, g, false);
+        lf_t2d_k<K>(Z, npatch, g, false);
         // ---- stage the filtered patches and the weight; k_aggregate adds them in the reference's order ----
         if (tid == 0) g.wbuf[(size_t) r * g.C + c] = wgt;
         for (int pa = sub; pa < npatch; pa += PPI) zdst[(pa * g.C + c) * k2] = Z[pa * PS + poff];
         __syncthreads();
     }
+}
+
+template <int STEP, int ASW>
+__global__ void __launch_bounds__(256) k_groups(GroupArgs g)
+{
+    extern __shared__ float smem[];
+    __shared__ GroupShape sh;
+    __shared__ float red[8];
+    __shared__ unsigned sofs[LF_MAXN * LF_LUTA];          // per gathered patch: st*C*plane + position
+    __shared__ unsigned char szero[LF_MAXN * LF_LUTA];    // patch reads as zeros (empty SAI, or column w-k: core:1697)
+    lf_groups_body<STEP, ASW, 0>(g, smem, sh, red, sofs, szero);
+}
+
+template <int STEP, int ASW>
+__global__ void __launch_bounds__(LF_G12_NT) k_groups12(GroupArgs g)
+{
+    extern __shared__ float smem[];
+    __shared__ GroupShape sh;
+    __shared__ float red[LF_G12_NT / 32];
+    __shared__ unsigned sofs[LF_MAXN * LF_LUTA];
+    __shared__ unsigned char szero[LF_MAXN * LF_LUTA];
+    lf_groups_body<STEP, ASW, 12>(g, smem, sh, red, sofs, szero);
 }
 
 // ---- packed FP32x2 versions of the 3x3 angular DCT: two independent signals per register pair ----

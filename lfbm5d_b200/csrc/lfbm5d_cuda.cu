@@ -396,7 +396,11 @@ int validate(const lfbm5d_params *p, int step)
     if (asw > p->aheight || asw > p->awidth)   // bm5d.cpp:120-124
         return fail("Wrong size of angular search window, the angular search window must be smaller than the light field angular size.");
     if (asw > LF_MAXASW) return fail("angular half window an > 2 is not supported by this build (an must be 0, 1 or 2)");
-    if (p->k != 8 && p->k != 16) return fail("patch size must be 8 or 16 in this build");
+    if (p->k != 8 && p->k != 12 && p->k != 16) return fail("patch size must be 8, 12 or 16 in this build");
+    if (p->k == 12) {
+        if (p->tau_2D == LFBM5D_BIOR) return fail("tau_2D = bior needs a power-of-two patch size (k = 8 or 16); k = 12 takes id or dct");
+        if (asw == 5) return fail("an = 2 is not supported at k = 12 (the 5x5-window group kernel needs 32 / k to be an integer); use k = 8 or 16");
+    }
     if (p->N == 0 || p->N > LF_MAXN || (p->N & (p->N - 1))) return fail("N must be a power of two <= 32");
     if (p->nDisp > LF_MAXDISP) return fail("nDisp > 16 is not supported by this build (nDisp must be <= 16)");
     if (p->nSim + p->nDisp + 1 < p->k) return fail("nSim + nDisp must be >= k - 1");
@@ -412,6 +416,10 @@ int validate(const lfbm5d_params *p, int step)
     // 5x5 windows: one channel of the group (twice that in step 2) has to fit into the shared memory of one CTA (k_groups25)
     if (asw == 5 && p->N * p->k * p->k * (step == 2 ? 2 : 1) > 2048)
         return fail("an = 2 needs N * k^2 <= 2048 in step 1 and 2 * N * k^2 <= 2048 in step 2 (k = 16: N <= 8 / N <= 4; k = 8: N <= 32 / N <= 16)");
+    // k = 12 (k_groups12): one channel of the group, rows padded to k + 1 floats (twice that in step 2), in the shared memory of one CTA
+    if (p->k == 12 && (size_t) p->N * asw * asw * 12 * 13 * 4 * (step == 2 ? 2 : 1) > LF_G12_SMEM)
+        return fail("k = 12 needs N * A * k * (k + 1) * 4 B (twice that in step 2) <= " + std::to_string(LF_G12_SMEM) +
+                    " B of shared memory per group (an = 1: N <= 32 in step 1, N <= 16 in step 2)");
     return 0;
 }
 
@@ -443,9 +451,15 @@ int setup_tables(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, unsigned tau
     {   // bm3d.cpp:1101-1169
         static const float k8[16] = { 0.1924f, 0.2989f, 0.3846f, 0.4325f, 0.2989f, 0.4642f, 0.5974f, 0.6717f,
                                       0.3846f, 0.5974f, 0.7688f, 0.8644f, 0.4325f, 0.6717f, 0.8644f, 0.9718f };
+        static const float k12[36] = { 0.1924f, 0.2615f, 0.3251f, 0.3782f, 0.4163f, 0.4362f, 0.2615f, 0.3554f, 0.4419f, 0.5139f, 0.5657f, 0.5927f,
+                                       0.3251f, 0.4419f, 0.5494f, 0.6390f, 0.7033f, 0.7369f, 0.3782f, 0.5139f, 0.6390f, 0.7433f, 0.8181f, 0.8572f,
+                                       0.4163f, 0.5657f, 0.7033f, 0.8181f, 0.9005f, 0.9435f, 0.4362f, 0.5927f, 0.7369f, 0.8572f, 0.9435f, 0.9885f };
         if (k == 8) {
             for (int i = 0; i < 8; i++)
                 for (int j = 0; j < 8; j++) T.kaiser[i * 8 + j] = k8[(i < 4 ? i : 7 - i) * 4 + (j < 4 ? j : 7 - j)];
+        } else if (k == 12) {      // the 6 x 6 quadrant, mirrored about both centre lines
+            for (int i = 0; i < 12; i++)
+                for (int j = 0; j < 12; j++) T.kaiser[i * 12 + j] = k12[(i < 6 ? i : 11 - i) * 6 + (j < 6 ? j : 11 - j)];
         } else
             for (int i = 0; i < k * k; i++) T.kaiser[i] = 1.0f;
         const float coef = 0.5f / ((float) k);
@@ -792,8 +806,10 @@ int launch_sat_self(lfbm5d_ctx *ctx, const PassCfg &pc, const SatPlan &P, int sg
     g.frow = ctx->frow.as<float>(); g.fcol = ctx->fcol.as<float>();
     const size_t smem = 2 * (128 + pc.k) * 64 * 4;
     if (ensure_tmap(ctx, pc)) return 1;
-    auto kfn = ctx->tmap_ok ? (pc.k == 8 ? k_sat2<true, 8, true> : k_sat2<true, 16, true>) : (pc.k == 8 ? k_sat2<true, 8, false> : k_sat2<true, 16, false>);
-    auto kedge = pc.k == 8 ? k_sat_edges<true, 8> : k_sat_edges<true, 16>;
+    // k = 12: cp.async ring loads (the TMA variant issues 8-row boxes and needs k to be a multiple of 8)
+    auto kfn = pc.k == 12 ? k_sat2<true, 12, false>
+             : ctx->tmap_ok ? (pc.k == 8 ? k_sat2<true, 8, true> : k_sat2<true, 16, true>) : (pc.k == 8 ? k_sat2<true, 8, false> : k_sat2<true, 16, false>);
+    auto kedge = pc.k == 8 ? k_sat_edges<true, 8> : pc.k == 12 ? k_sat_edges<true, 12> : k_sat_edges<true, 16>;
     CK(cudaFuncSetAttribute((const void *) kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     const size_t smem_e = sate_smem((int) pc.k);
     CK(cudaFuncSetAttribute((const void *) kedge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_e));
@@ -818,8 +834,9 @@ int launch_sat_stereo(lfbm5d_ctx *ctx, const PassCfg &pc, const SatPlan &P, int 
     const size_t smem = 2 * (128 + pc.k) * 64 * 4;
     const int ngroups = (s1 - s0) * P.groups_per_slot;
     if (ensure_tmap(ctx, pc)) return 1;
-    auto kfn = ctx->tmap_ok ? (pc.k == 8 ? k_sat2<false, 8, true> : k_sat2<false, 16, true>) : (pc.k == 8 ? k_sat2<false, 8, false> : k_sat2<false, 16, false>);
-    auto kedge = pc.k == 8 ? k_sat_edges<false, 8> : k_sat_edges<false, 16>;
+    auto kfn = pc.k == 12 ? k_sat2<false, 12, false>
+             : ctx->tmap_ok ? (pc.k == 8 ? k_sat2<false, 8, true> : k_sat2<false, 16, true>) : (pc.k == 8 ? k_sat2<false, 8, false> : k_sat2<false, 16, false>);
+    auto kedge = pc.k == 8 ? k_sat_edges<false, 8> : pc.k == 12 ? k_sat_edges<false, 12> : k_sat_edges<false, 16>;
     CK(cudaFuncSetAttribute((const void *) kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     const size_t smem_e = sate_smem((int) pc.k);
     CK(cudaFuncSetAttribute((const void *) kedge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_e));
@@ -975,6 +992,14 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     const size_t smem = (size_t) pc.N * pc.A * ga.PS * 4 * (pc.step == 2 ? 2 : 1);
     void (*kfn)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups<1, 3> : k_groups<1, 1>)
                                           : (pc.asw == 3 ? k_groups<2, 3> : k_groups<2, 1>);
+    if (pc.k == 12) {      // 288 threads (2 patches x 144 positions); validate() bounds the group's shared memory
+        void (*k12)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups12<1, 3> : k_groups12<1, 1>)
+                                              : (pc.asw == 3 ? k_groups12<2, 3> : k_groups12<2, 1>);
+        CK(cudaFuncSetAttribute((const void *) k12, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+        k12<<<nblk, LF_G12_NT, smem, ctx->stream>>>(ga);
+        ctx->stats.kernel_launches++;
+        return 0;
+    }
     CK(cudaFuncSetAttribute((const void *) kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     if (pc.step == 1 && pc.tau_2D == LFBM5D_ID && pc.k == 16 && pc.asw == 3 && pc.N <= 8 && pc.tau_5D != LFBM5D_DCT && !pc.useSD) {
         // register-resident path (no 2-D transform to stage); patches that contribute zeros read the zero block behind nsym
@@ -1012,8 +1037,10 @@ int launch_aggregate(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, in
     aa.ty0 = y_lo / 16;
     dim3 grid((pc.wb + 15) / 16, (y_hi + 15) / 16 - aa.ty0, pc.A);
     const bool band = !(y_lo == 0 && y_hi == (int) pc.hb && a_lo == 0 && a_hi == pg.nr);
-    void (*kagg)(AggArgs) = band ? k_aggregate<8, 1, true> : k_aggregate<8, 1, false>;         // validate(): k is 8 or 16, C is 1 or 3
+    void (*kagg)(AggArgs) = band ? k_aggregate<8, 1, true> : k_aggregate<8, 1, false>;         // validate(): k is 8, 12 or 16, C is 1 or 3
     if (pc.C == 3 && pc.k == 16) kagg = band ? k_aggregate<16, 3, true> : k_aggregate<16, 3, false>;
+    else if (pc.C == 3 && pc.k == 12) kagg = band ? k_aggregate<12, 3, true> : k_aggregate<12, 3, false>;
+    else if (pc.C == 1 && pc.k == 12) kagg = band ? k_aggregate<12, 1, true> : k_aggregate<12, 1, false>;
     else if (pc.C == 3 && pc.k == 8) kagg = band ? k_aggregate<8, 3, true> : k_aggregate<8, 3, false>;
     else if (pc.C == 1 && pc.k == 16) kagg = band ? k_aggregate<16, 1, true> : k_aggregate<16, 1, false>;
     LAUNCH(ctx, kagg, grid, 256, 0, aa);
@@ -1304,7 +1331,8 @@ int validate_bm3d(const lfbm3d_params *p)
     if (p->nHard != p->nWien) return fail("nHard must equal nWien (the reference passes the nHard-padded image to its 2nd step, bm3d.cpp:175)");
     for (int s = 0; s < 2; s++) {
         const unsigned k = s ? p->kWien : p->kHard, N = s ? p->NWien : p->NHard, t2 = s ? p->tau_2D_wien : p->tau_2D_hard;
-        if (k != 8 && k != 16) return fail("patch size must be 8 or 16 in this build");
+        if (k != 8 && k != 12 && k != 16) return fail("patch size must be 8, 12 or 16 in this build");
+        if (k == 12 && t2 == LFBM5D_BIOR) return fail("tau_2D = bior needs a power-of-two patch size (k = 8 or 16); k = 12 takes dct");
         if (N < 2 || N > LF_MAXN || (N & (N - 1))) return fail("N must be a power of two in [2, 32]");
         if (t2 != LFBM5D_DCT && t2 != LFBM5D_BIOR) return fail("tau_2D must be dct or bior for BM3D");
         if ((s ? p->pWien : p->pHard) == 0) return fail("processing step must be >= 1");
