@@ -33,11 +33,13 @@ typedef struct lfbm5d_params {
                              * an = 2 needs N * k^2 <= 2048 in step 1 and 2 * N * k^2 <= 2048 in step 2 (one channel of the
                              * 25-SAI group in the shared memory of one CTA): k = 16 with N <= 8 / N <= 4, k = 8 with N <= 32 / N <= 16 */
     unsigned width, height, chnls;
-    unsigned N;             /* NHard / NWien */
+    unsigned N;             /* NHard / NWien: a power of two <= 32. At k = 16 and an <= 1, groups whose channel does not fit into the
+                             * shared memory of one CTA (N = 32 in step 1, N >= 16 in step 2) run on 2- or 4-CTA clusters
+                             * (lfbm5d_group_cluster tells which) */
     unsigned nSim;          /* half size of the self search window */
     unsigned nDisp;         /* half size of the disparity search window, <= 16 ((2nDisp+1)^2 offsets per SAI of the window).
                              * The SAIs must be at least nSim + nDisp pixels high and wide (mirror padding) */
-    unsigned k;             /* kHard / kWien: patch side, 8, 12 or 16. k = 12 takes tau_2D = id or dct (bior needs a power of two),
+    unsigned k;             /* kHard / kWien: patch side, 8, 12 or 16 (k = 16: N <= 32 at an <= 1 in both steps). k = 12 takes tau_2D = id or dct (bior needs a power of two),
                              * an = 0 or 1, and N * A * k * (k + 1) * 4 B <= 220 KB (twice that in step 2; A = (2an+1)^2):
                              * at an = 1, N <= 32 in step 1 and N <= 16 in step 2 */
     unsigned p;             /* pHard / pWien */
@@ -99,6 +101,11 @@ int lfbm3d_run_device(lfbm5d_ctx *ctx, const lfbm3d_params *p, float *d_noisy_io
                       float *d_denoised_out);
 /* stop after this many window passes per step (0 = run to completion); for bounded measurements only */
 void lfbm5d_set_max_passes(lfbm5d_ctx *ctx, unsigned max_passes);
+/* How the group kernel of `step` runs with these parameters on the context's device: *cluster_size = 1 when one CTA holds a
+ * group, else the CTAs of the thread-block cluster that share it through distributed shared memory (2 or 4; k = 16 groups of
+ * 3x3 windows over the opt-in shared memory of one CTA), with *max_active_clusters = cudaOccupancyMaxActiveClusters of that
+ * configuration (0 for cluster_size 1). Fails, naming the cluster size and the bytes per CTA, if the device cannot run it. */
+int lfbm5d_group_cluster(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, int *cluster_size, int *max_active_clusters);
 
 /* ---- static window schedule ----------------------------------------------------------------------
  * The angular windows of a step (bm5d.cpp:171-402) in the order of the reference's schedule; windows that share no SAI commute.

@@ -43,7 +43,7 @@ class Stats(C.Structure):
 
 EXPORTS = ["lfbm5d_create", "lfbm5d_destroy", "lfbm5d_last_error", "lfbm5d_reset_stats", "lfbm5d_get_stats",
            "lfbm5d_enable_timing", "lfbm5d_stream", "lfbm5d_step1", "lfbm5d_step2", "lfbm3d_run", "lfbm5d_step1_device",
-           "lfbm5d_step2_device", "lfbm3d_run_device", "lfbm5d_set_max_passes", "lfbm5d_debug_pass", "lfbm5d_debug_pass_ex",
+           "lfbm5d_step2_device", "lfbm3d_run_device", "lfbm5d_set_max_passes", "lfbm5d_group_cluster", "lfbm5d_debug_pass", "lfbm5d_debug_pass_ex",
            "lfbm5d_debug_schedule", "lfbm5d_step_plan", "lfbm5d_debug_block_matching", "lfbm5d_team_create_emulated", "lfbm5d_team_unique_id",
            "lfbm5d_team_create_nccl", "lfbm5d_team_destroy", "lfbm5d_team_local_ranks", "lfbm5d_team_step", "lfbm5d_team_band",
            "lfbm5d_team_stats", "lfbm5d_team_disable_peer_view", "lfbm5d_team_timing", "lfbm5d_team_plan_band", "lfbm5d_copy_rows", "lfbm5d_sync", "lfbm5d_team_use_peer_exchange", "lfbm5d_team_set_lanes", "lfbm5d_team_launches"]
@@ -179,6 +179,14 @@ class LFBM5D(object):
 
     def stream(self):
         return self.lib.lfbm5d_stream(self.ctx)
+
+    def group_cluster(self, step, prm):
+        """(cluster size, cudaOccupancyMaxActiveClusters) of the group kernel of `step` with these parameters: (1, 0) when one
+        CTA holds a group."""
+        cl, occ = C.c_int(0), C.c_int(0)
+        if self.lib.lfbm5d_group_cluster(self.ctx, int(step), C.byref(prm), C.byref(cl), C.byref(occ)) != 0:
+            raise RuntimeError(self.error())
+        return cl.value, occ.value
 
     def schedule(self, max_entries=4096):
         out = np.zeros((max_entries, 4), np.uint32)

@@ -5,6 +5,8 @@
 // Restates core:277-528 (step 1) and :1054-1329 (step 2).
 #pragma once
 #include "common.cuh"
+#include <cooperative_groups.h>
+namespace cg = cooperative_groups;
 
 template <int SW> struct GroupShapeT;
 
@@ -514,7 +516,8 @@ __device__ __forceinline__ void lf_t2d(float *B, int npatch, const GroupArgs &g,
 // and the aggregation entries: (y << 16 | x) of every patch that k_aggregate has to add, LF_NOENT otherwise.
 // Returns false (after marking the group's entries empty) for reference patches the partial-window branch skips.
 // SW: window side the shared arrays are sized for; windows up to 3x3 copy their shape from the host table, 5x5 ones build it.
-template <bool ZB, int SW = LF_LUTASW, class GA = GroupArgs>
+// ENT = false: leave the aggregation entries to another CTA of the group (k_groups_cl: rank 0 writes them).
+template <bool ZB, int SW = LF_LUTASW, class GA = GroupArgs, bool ENT = true>
 __device__ __forceinline__ bool lf_group_setup(const GA &g, int r, int nSx, GroupShapeT<SW> &sh, unsigned *sofs, unsigned char *szero)
 {
     __shared__ unsigned s_yx[LF_MAXN * SW * SW];
@@ -522,10 +525,11 @@ __device__ __forceinline__ bool lf_group_setup(const GA &g, int r, int nSx, Grou
     const int tid = threadIdx.x, nt = blockDim.x;
     const unsigned plane = (unsigned) g.w * (unsigned) g.h;
     if (g.act && !g.act[r]) {        // den-aware ind_initialize (utilities_LF.cpp:1031-1099): every pixel of the patch already has a weight
-        for (int t = tid; t < g.N * A; t += nt) {
-            const int n = t / A, st = t - n * A;
-            g.ent[(size_t) st * g.R * g.N + (size_t) r * g.N + n] = LF_NOENT;
-        }
+        if constexpr (ENT)
+            for (int t = tid; t < g.N * A; t += nt) {
+                const int n = t / A, st = t - n * A;
+                g.ent[(size_t) st * g.R * g.N + (size_t) r * g.N + n] = LF_NOENT;
+            }
         return false;
     }
     if constexpr (SW == LF_LUTASW) {
@@ -546,12 +550,13 @@ __device__ __forceinline__ bool lf_group_setup(const GA &g, int r, int nSx, Grou
         s_yx[t] = (py << 16) | px;
     }
     __syncthreads();
-    for (int t = tid; t < g.N * A; t += nt) {
-        const int n = t / A, st = t - n * A;
-        // core:486, :503: which SAIs receive this group's patches
-        const bool on = n < nSx && !g.win.proc[st] && !(g.tau_4D == 6 && st != g.pst && !sh.mask[st]);
-        g.ent[(size_t) st * g.R * g.N + (size_t) r * g.N + n] = on ? s_yx[t] : LF_NOENT;
-    }
+    if constexpr (ENT)
+        for (int t = tid; t < g.N * A; t += nt) {
+            const int n = t / A, st = t - n * A;
+            // core:486, :503: which SAIs receive this group's patches
+            const bool on = n < nSx && !g.win.proc[st] && !(g.tau_4D == 6 && st != g.pst && !sh.mask[st]);
+            g.ent[(size_t) st * g.R * g.N + (size_t) r * g.N + n] = on ? s_yx[t] : LF_NOENT;
+        }
     return true;
 }
 
@@ -767,6 +772,210 @@ __global__ void __launch_bounds__(LF_G12_NT) k_groups12(GroupArgs g)
     __shared__ unsigned sofs[LF_MAXN * LF_LUTA];
     __shared__ unsigned char szero[LF_MAXN * LF_LUTA];
     lf_groups_body<STEP, ASW, 12>(g, smem, sh, red, sofs, szero);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// k = 16 groups of 3x3 windows whose channel does not fit into the shared memory of one CTA (N = 32 in step 1, N >= 16 in
+// step 2 with 2-D dct / bior): the group of one reference patch runs on a cluster of CL CTAs of 256 threads (thread <-> pixel
+// position, as k_groups at k = 16). Patch n of the group lives on CTA n % CL in local slot n / CL, with all of its SAIs, so
+// the gather, the 2-D transforms, the angular transforms and the staging stay local. The 5th dimension runs across the
+// cluster: the (st, pq) vectors are dealt out by st (CTA `rank` takes st = rank, rank + CL, ...), each thread loads its nSx
+// values from the CTAs that own them through distributed shared memory, filters them with lf_filter5d / lf_filter5d_dct and
+// stores them back. Group-wide sums (Wiener weight, useSD) are reduced per CTA and then added in rank order, so that the
+// result does not depend on scheduling. Same per-element arithmetic as k_groups: step 1 is bit-identical to it.
+// ------------------------------------------------------------------------------------------------------------
+// one (st, pq) vector whose value n sits at Xr[n % CL][(n / CL) * sstride + ofs] (Er: the basic estimate of step 2)
+template <int STEP, int CL, int NS>
+__device__ __forceinline__ float lf_filter5d_cl(float *const *Xr, float *const *Er, int ofs, int sstride, unsigned tau_5D, bool shrink, int c, int lg)
+{
+    float vo[NS], ve[NS];
+#pragma unroll
+    for (int n = 0; n < NS; ++n) {
+        vo[n] = Xr[n % CL][(n / CL) * sstride + ofs];
+        if (STEP == 2) ve[n] = Er[n % CL][(n / CL) * sstride + ofs];
+    }
+    const float wsum = lf_filter5d<STEP, NS>(vo, ve, 0, 1, tau_5D, shrink, c, lg);
+    float *const *dst = STEP == 1 ? Xr : Er;
+#pragma unroll
+    for (int n = 0; n < NS; ++n) dst[n % CL][(n / CL) * sstride + ofs] = STEP == 1 ? vo[n] : ve[n];
+    return wsum;
+}
+template <int STEP, int CL>
+__device__ __forceinline__ float lf_filter5d_dct_cl(float *const *Xr, float *const *Er, int ofs, int sstride, int ns, bool shrink, int c, int lg)
+{
+    float vo[LF_MAXN], ve[LF_MAXN];
+#pragma unroll 1
+    for (int n = 0; n < ns; ++n) {
+        vo[n] = Xr[n % CL][(n / CL) * sstride + ofs];
+        if (STEP == 2) ve[n] = Er[n % CL][(n / CL) * sstride + ofs];
+    }
+    const float wsum = lf_filter5d_dct(STEP, vo, ve, 0, 1, ns, shrink, c, lg);
+    float *const *dst = STEP == 1 ? Xr : Er;
+#pragma unroll 1
+    for (int n = 0; n < ns; ++n) dst[n % CL][(n / CL) * sstride + ofs] = STEP == 1 ? vo[n] : ve[n];
+    return wsum;
+}
+// sum of the CTAs' partial sums part[i], in rank order (the same value in every thread of the cluster)
+template <int CL>
+__device__ __forceinline__ float lf_cluster_sum(cg::cluster_group &cluster, float *part, int i)
+{
+    float s = *cluster.map_shared_rank(part + i, 0);
+#pragma unroll
+    for (int j = 1; j < CL; ++j) s += *cluster.map_shared_rank(part + i, j);
+    return s;
+}
+
+template <int STEP, int CL>
+__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(256) k_groups_cl(GroupArgs g)
+{
+    extern __shared__ float smem[];                       // this CTA's patches: N / CL slots of A patches (twice that in step 2)
+    __shared__ GroupShape sh;
+    __shared__ float red[8];
+    __shared__ float part[3];                             // this CTA's partial sums: weight, useSD's sum and sum of squares
+    __shared__ unsigned sofs[LF_MAXN * LF_LUTA];
+    __shared__ unsigned char szero[LF_MAXN * LF_LUTA];
+    constexpr int A = 9, k2 = 256;
+    cg::cluster_group cluster = cg::this_cluster();
+    const int rank = (int) cluster.block_rank();
+    const int tid = threadIdx.x;
+    const int r = blockIdx.x / CL + g.r0;
+    const int w = g.w;
+    const unsigned plane = (unsigned) g.w * (unsigned) g.h;
+    const int nSx = (int) g.bm_count[r];
+    const int lg = 31 - __clz(nSx);
+    const int PS = g.PS, RS = g.RS;
+    const int SS = A * PS;                                // slot stride (floats)
+    float *X = smem;
+    float *E = smem + (size_t) (g.N / CL) * SS;          // step 2 only
+    const int pq = tid, p = pq >> 4, q = pq & 15;
+    const int poff = p * RS + q;
+    const int nloc = (nSx - rank + CL - 1) / CL;          // patches n = rank, rank + CL, ... of the group (0 when nSx <= rank)
+    const int npl = nloc * A;
+    // every CTA of the cluster reads the same act[r] and bm_count[r]: a skipped group is skipped by all of them, before any
+    // cluster barrier
+    if (!(rank == 0 ? lf_group_setup<false>(g, r, nSx, sh, sofs, szero)
+                    : lf_group_setup<false, LF_LUTASW, GroupArgs, false>(g, r, nSx, sh, sofs, szero))) return;
+    const bool use_sadct = sh.use_sadct != 0 && g.tau_4D == 6;
+    float *zdst = g.zbuf + (size_t) r * g.N * A * g.C * k2 + pq;
+    float *Xr[CL], *Er[CL];
+#pragma unroll
+    for (int j = 0; j < CL; ++j) { Xr[j] = cluster.map_shared_rank(X, j); Er[j] = STEP == 2 ? cluster.map_shared_rank(E, j) : nullptr; }
+    float sd_w = 0.f;
+
+    for (int c = 0; c < g.C; ++c) {
+        // ---- gather (core:286-299) of this CTA's patches: local patch pl = slot * A + st is group patch (slot * CL + rank, st) ----
+        {
+            const unsigned tofs = (unsigned) c * plane + (unsigned) (p * w + q);
+            for (int pl = 0; pl < npl; ++pl) {
+                const int slot = pl / A, st = pl - slot * A;
+                const int pa = (slot * CL + rank) * A + st;
+                float *dx = &X[pl * PS + poff];
+                if (!szero[pa]) {
+                    const unsigned src = sofs[pa] + tofs;
+                    lf_cp_async4(dx, g.nsym + src);
+                    if (STEP == 2) lf_cp_async4(&E[pl * PS + poff], g.bsym + src);
+                } else {
+                    *dx = 0.f;
+                    if (STEP == 2) E[pl * PS + poff] = 0.f;
+                }
+            }
+            lf_cp_async_wait_all();
+        }
+        __syncthreads();
+        // ---- 2-D spatial transform and angular transform (core:354-360) of the local patches ----
+        lf_t2d(X, npl, g, true);
+        if (STEP == 2) lf_t2d(E, npl, g, true);
+        if (g.tau_4D != 4) {
+            for (int slot = 0; slot < nloc; ++slot) {
+                const int off = slot * SS + poff;
+                for (int rep = 0; rep < STEP; ++rep) {
+                    float *B = rep == 0 ? X : E;
+                    float v[A];
+#pragma unroll
+                    for (int st = 0; st < A; ++st) v[st] = B[off + st * PS];
+                    if (use_sadct) {
+                        float u[A];
+#pragma unroll
+                        for (int st = 0; st < A; ++st) u[st] = v[st];
+                        lf_sadct_fwd(u, sh, 3);
+#pragma unroll
+                        for (int st = 0; st < A; ++st) v[st] = u[st];
+                    } else lf_dct4_fwd<3>(v);
+#pragma unroll
+                    for (int st = 0; st < A; ++st) B[off + st * PS] = v[st];
+                }
+            }
+        }
+        cluster.sync();        // the peers read this CTA's coefficients
+        // ---- 5th dimension + shrinkage (core:371-410 / :1170-1210) across the cluster ----
+        float wpart = 0.f;
+        for (int st = rank; st < A; st += CL) {
+            const int ofs = st * PS + poff;
+            const bool shrink = !use_sadct || sh.mask_dct[st];
+            if (g.tau_5D == 5) { wpart += lf_filter5d_dct_cl<STEP, CL>(Xr, Er, ofs, SS, nSx, shrink, c, lg); continue; }
+            switch (nSx) {
+                case 1:  wpart += lf_filter5d_cl<STEP, CL, 1>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+                case 2:  wpart += lf_filter5d_cl<STEP, CL, 2>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+                case 4:  wpart += lf_filter5d_cl<STEP, CL, 4>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+                case 8:  wpart += lf_filter5d_cl<STEP, CL, 8>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+                case 16: wpart += lf_filter5d_cl<STEP, CL, 16>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+                default: wpart += lf_filter5d_cl<STEP, CL, 32>(Xr, Er, ofs, SS, g.tau_5D, shrink, c, lg); break;
+            }
+        }
+        const float wloc = lf_block_sum_f(wpart, red);
+        if (tid == 0) part[0] = wloc;
+        cluster.sync();        // the peers wrote this CTA's coefficients back; every partial weight is visible
+        // step 1: the weight is a count of coefficients, exact in any order; step 2: rank order
+        const float wsum = lf_cluster_sum<CL>(cluster, part, 0);
+        const float sg = c_tab.sigma[c];
+        float wgt = wsum > 0.0f ? (sg > 0.0f ? 1.0f / (c_tab.sigma2[c] * wsum) : 1.0f / wsum) : 1.0f;   // core:419-420
+        float *Z = STEP == 1 ? X : E;
+        if (g.use_sd) {      // sd_weighting_5d (core:3140-3173), as k_groups
+            if (g.use_sd == 1 || c == 0) {
+                float m1 = 0.f, m2 = 0.f;
+                for (int pl = 0; pl < npl; ++pl) { const float xv = Z[pl * PS + poff]; m1 += xv; m2 += xv * xv; }
+                const float s1 = lf_block_sum_f(m1, red);
+                const float s2 = lf_block_sum_f(m2, red);
+                if (tid == 0) { part[1] = s1; part[2] = s2; }
+                cluster.sync();
+                const float mean = lf_cluster_sum<CL>(cluster, part, 1);
+                const float sq = lf_cluster_sum<CL>(cluster, part, 2);
+                const float Nn = (float) (g.use_sd == 1 ? nSx * A : nSx * k2);
+                const float res = (sq - mean * mean / Nn) / (Nn - 1.0f);
+                sd_w = res > 0.0f ? 1.0f / sqrtf(res) : 0.0f;
+            }
+            wgt = sd_w;
+        }
+        // ---- inverse angular transform (core:432-451) and inverse 2-D transform (core:489-493) of the local patches ----
+        if (g.tau_4D != 4) {
+            for (int slot = 0; slot < nloc; ++slot) {
+                const int off = slot * SS + poff;
+                float v[A];
+#pragma unroll
+                for (int st = 0; st < A; ++st) v[st] = Z[off + st * PS];
+                if (use_sadct) {
+                    float u[A];
+#pragma unroll
+                    for (int st = 0; st < A; ++st) u[st] = v[st];
+                    lf_sadct_inv(u, sh, 3);
+#pragma unroll
+                    for (int st = 0; st < A; ++st) v[st] = u[st];
+                } else lf_dct4_inv<3>(v);
+#pragma unroll
+                for (int st = 0; st < A; ++st) Z[off + st * PS] = v[st];
+            }
+            __syncthreads();
+        }
+        lf_t2d(Z, npl, g, false);
+        // ---- stage the filtered patches (zbuf layout of k_groups) and, on rank 0, the weight ----
+        if (rank == 0 && tid == 0) g.wbuf[(size_t) r * g.C + c] = wgt;
+        for (int pl = 0; pl < npl; ++pl) {
+            const int slot = pl / A, st = pl - slot * A;
+            zdst[(((slot * CL + rank) * A + st) * g.C + c) * k2] = Z[pl * PS + poff];
+        }
+        __syncthreads();
+    }
+    cluster.sync();            // no CTA exits while a peer may still read its partial sums
 }
 
 // ---- packed FP32x2 versions of the 3x3 angular DCT: two independent signals per register pair ----

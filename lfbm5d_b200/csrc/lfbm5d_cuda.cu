@@ -17,6 +17,7 @@
 #include <vector>
 #include <algorithm>
 #include <array>
+#include <map>
 #include <mutex>
 #include <memory>
 
@@ -364,6 +365,7 @@ struct lfbm5d_ctx {
     unsigned max_passes = 0;
     std::vector<unsigned> sched;
     std::vector<std::unique_ptr<SatPlan>> sat_cache;     // plane tables per window shape (sat_plan)
+    std::map<std::pair<const void *, size_t>, int> cluster_occ;   // group_cluster: clusters the device holds per (kernel, smem)
     LfTables tab;                 // this context's constants; c_tab (one per device) is reloaded when it holds another context's
 };
 
@@ -949,6 +951,49 @@ int launch_group_masks(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, 
     return 0;
 }
 
+// k = 16 groups of 3x3 windows whose channel (N * A * k * RS floats, twice that in step 2) needs more than the opt-in shared memory
+// of one CTA next to k_groups' static arrays run on a cluster of CL CTAs (k_groups_cl), the smallest power of two for which
+// 1 / CL of the group fits next to that kernel's static arrays. cl = 1: k_groups' branch fits (or does not apply). Before the
+// first launch of a (kernel, shared memory) pair, the device has to be able to hold at least one such cluster at a time.
+struct GroupCluster {
+    int cl = 1;
+    void (*fn)(GroupArgs) = nullptr;
+    size_t smem = 0;                 // dynamic shared memory per CTA
+    int max_active = 0;              // cudaOccupancyMaxActiveClusters of this configuration
+};
+int group_cluster(lfbm5d_ctx *ctx, int step, unsigned k, unsigned asw, unsigned N, unsigned tau_2D, GroupCluster &gc)
+{
+    gc = GroupCluster{};
+    if (k != 16 || asw != 3) return 0;
+    const size_t smem = (size_t) N * 9 * k * (tau_2D == LFBM5D_ID ? k : k + 1) * 4 * (step == 2 ? 2 : 1);
+    cudaFuncAttributes fa;
+    CK(cudaFuncGetAttributes(&fa, (const void *) (step == 1 ? k_groups<1, 3> : k_groups<2, 3>)));
+    if (smem + fa.sharedSizeBytes <= (size_t) ctx->smem_optin) return 0;
+    void (*const fns[2][2])(GroupArgs) = { { k_groups_cl<1, 2>, k_groups_cl<1, 4> }, { k_groups_cl<2, 2>, k_groups_cl<2, 4> } };
+    for (int i = 0; i < 2 && !gc.fn; i++) {
+        void (*fn)(GroupArgs) = fns[step - 1][i];
+        CK(cudaFuncGetAttributes(&fa, (const void *) fn));
+        if (smem / (2 << i) + fa.sharedSizeBytes <= (size_t) ctx->smem_optin) { gc.cl = 2 << i; gc.fn = fn; gc.smem = smem / gc.cl; }
+    }
+    if (!gc.fn) return fail("a group of " + std::to_string(smem) + " B of shared memory per channel does not fit a cluster of 4 CTAs");
+    const auto key = std::make_pair((const void *) gc.fn, gc.smem);
+    const auto it = ctx->cluster_occ.find(key);
+    if (it != ctx->cluster_occ.end()) { gc.max_active = it->second; return 0; }
+    CK(cudaFuncSetAttribute((const void *) gc.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) gc.smem));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned) gc.cl); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = gc.smem; cfg.stream = ctx->stream;
+    cudaLaunchAttribute at;
+    at.id = cudaLaunchAttributeClusterDimension;
+    at.val.clusterDim.x = (unsigned) gc.cl; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
+    cfg.attrs = &at; cfg.numAttrs = 1;
+    CK(cudaOccupancyMaxActiveClusters(&gc.max_active, (const void *) gc.fn, &cfg));
+    if (gc.max_active <= 0)
+        return fail("the group kernel needs clusters of " + std::to_string(gc.cl) + " CTAs with " + std::to_string(gc.smem + fa.sharedSizeBytes) +
+                    " B of shared memory per CTA, and this device cannot run one");
+    ctx->cluster_occ[key] = gc.max_active;
+    return 0;
+}
+
 // Group kernel for the reference patches [r0, r1) (gather, transforms, shrinkage, inverses, staging for the aggregation)
 int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, bool partial, int r0, int r1)
 {
@@ -997,6 +1042,14 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
                                               : (pc.asw == 3 ? k_groups12<2, 3> : k_groups12<2, 1>);
         CK(cudaFuncSetAttribute((const void *) k12, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
         k12<<<nblk, LF_G12_NT, smem, ctx->stream>>>(ga);
+        ctx->stats.kernel_launches++;
+        return 0;
+    }
+    GroupCluster gc;
+    if (group_cluster(ctx, pc.step, pc.k, pc.asw, pc.N, pc.tau_2D, gc)) return 1;
+    if (gc.cl > 1) {       // distributed over a cluster: CTA blockIdx.x % cl of the cluster of reference patch blockIdx.x / cl + r0
+        CK(cudaFuncSetAttribute((const void *) gc.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) gc.smem));
+        gc.fn<<<nblk * gc.cl, 256, gc.smem, ctx->stream>>>(ga);
         ctx->stats.kernel_launches++;
         return 0;
     }
@@ -1476,6 +1529,19 @@ void lfbm5d_get_stats(lfbm5d_ctx *ctx, lfbm5d_stats *out) { if (ctx && out) *out
 void lfbm5d_enable_timing(lfbm5d_ctx *ctx, int on) { if (ctx) ctx->timing = on != 0; }
 void *lfbm5d_stream(lfbm5d_ctx *ctx) { return ctx ? (void *) ctx->stream : nullptr; }
 void lfbm5d_set_max_passes(lfbm5d_ctx *ctx, unsigned m) { if (ctx) ctx->max_passes = m; }
+
+int lfbm5d_group_cluster(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, int *cluster_size, int *max_active_clusters)
+{
+    if (!ctx || !cluster_size || !max_active_clusters) return fail("null argument");
+    if (step != 1 && step != 2) return fail("step must be 1 or 2");
+    if (validate(p, step)) return 1;
+    CK(cudaSetDevice(ctx->device));
+    GroupCluster gc;
+    if (group_cluster(ctx, step, p->k, 2 * p->an + 1, p->N, p->tau_2D, gc)) return 1;
+    *cluster_size = gc.cl;
+    *max_active_clusters = gc.max_active;
+    return 0;
+}
 
 int lfbm5d_step1_device(lfbm5d_ctx *ctx, const lfbm5d_params *p, float *d_noisy_io, const unsigned *sai_mask, float *d_basic_out)
 {
