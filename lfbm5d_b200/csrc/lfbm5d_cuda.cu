@@ -951,6 +951,15 @@ int launch_group_masks(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, 
     return 0;
 }
 
+// Dynamic shared memory of one channel of a group on one CTA: N patches of A SAIs (twice that in step 2), k rows of RS floats.
+// Row padding removes the shared-memory bank conflicts of the 2-D passes (3 CTAs/SM without it measured slower); 5x5 windows
+// store their patches densely (LfSwizzled).
+static int group_rs(unsigned k, unsigned asw, unsigned tau_2D) { return asw > LF_LUTASW || tau_2D == LFBM5D_ID ? (int) k : (int) k + 1; }
+static size_t group_smem(int step, unsigned k, unsigned asw, unsigned N, unsigned tau_2D)
+{
+    return (size_t) N * asw * asw * k * group_rs(k, asw, tau_2D) * 4 * (step == 2 ? 2 : 1);
+}
+
 // k = 16 groups of 3x3 windows whose channel (N * A * k * RS floats, twice that in step 2) needs more than the opt-in shared memory
 // of one CTA next to k_groups' static arrays run on a cluster of CL CTAs (k_groups_cl), the smallest power of two for which
 // 1 / CL of the group fits next to that kernel's static arrays. cl = 1: k_groups' branch fits (or does not apply). Before the
@@ -965,7 +974,7 @@ int group_cluster(lfbm5d_ctx *ctx, int step, unsigned k, unsigned asw, unsigned 
 {
     gc = GroupCluster{};
     if (k != 16 || asw != 3) return 0;
-    const size_t smem = (size_t) N * 9 * k * (tau_2D == LFBM5D_ID ? k : k + 1) * 4 * (step == 2 ? 2 : 1);
+    const size_t smem = group_smem(step, k, asw, N, tau_2D);
     cudaFuncAttributes fa;
     CK(cudaFuncGetAttributes(&fa, (const void *) (step == 1 ? k_groups<1, 3> : k_groups<2, 3>)));
     if (smem + fa.sharedSizeBytes <= (size_t) ctx->smem_optin) return 0;
@@ -1005,9 +1014,9 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     gb.act = partial ? ctx->act.as<unsigned char>() : nullptr; gb.partial = partial ? 1 : 0; gb.use_sd = (int) pc.useSD;
     gb.C = pc.C; gb.asw = pc.asw; gb.A = pc.A; gb.k = pc.k; gb.log2k = pc.k == 8 ? 3 : 4; gb.N = pc.N; gb.w = pc.wb; gb.h = pc.hb;
     gb.pst = pst; gb.nc = pg.nc; gb.r0 = r0;
-    // row padding removes the shared-memory bank conflicts of the 2-D passes (3 CTAs/SM without it measured slower)
-    gb.RS = pc.tau_2D == LFBM5D_ID ? pc.k : pc.k + 1;
+    gb.RS = group_rs(pc.k, pc.asw, pc.tau_2D);
     gb.PS = pc.k * gb.RS;
+    const size_t smem = group_smem(pc.step, pc.k, pc.asw, pc.N, pc.tau_2D);
     gb.tau_2D = pc.tau_2D; gb.tau_4D = pc.tau_4D; gb.tau_5D = pc.tau_5D;
     gb.rows = ctx->rows.as<int>(); gb.cols = ctx->cols.as<int>();
     gb.bm_count = ctx->bmcount.as<unsigned>(); gb.bm_idx = ctx->bmidx.as<unsigned>();
@@ -1020,13 +1029,11 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
         // 5x5 windows: dense swizzled patches (no row padding), one CTA of 512 threads per SM; validate() bounds the group
         GroupArgs25 g25{};
         static_cast<GroupArgsBase &>(g25) = gb;
-        g25.RS = pc.k; g25.PS = pc.k * pc.k;
         g25.win = win;
         g25.gmask32 = ctx->gmask.as<unsigned>();
-        const size_t smem25 = (size_t) pc.N * pc.A * g25.PS * 4 * (pc.step == 2 ? 2 : 1);
         void (*k25)(GroupArgs25) = pc.step == 1 ? k_groups25<1> : k_groups25<2>;
-        CK(cudaFuncSetAttribute((const void *) k25, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem25));
-        k25<<<nblk, G25_NT, smem25, ctx->stream>>>(g25);
+        CK(cudaFuncSetAttribute((const void *) k25, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+        k25<<<nblk, G25_NT, smem, ctx->stream>>>(g25);
         ctx->stats.kernel_launches++;
         return 0;
     }
@@ -1034,7 +1041,6 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     static_cast<GroupArgsBase &>(ga) = gb;
     for (int a = 0; a < LF_LUTA; a++) { ga.win.st[a] = win.st[a]; ga.win.mask[a] = win.mask[a]; ga.win.proc[a] = win.proc[a]; }
     ga.win.A = win.A;
-    const size_t smem = (size_t) pc.N * pc.A * ga.PS * 4 * (pc.step == 2 ? 2 : 1);
     void (*kfn)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups<1, 3> : k_groups<1, 1>)
                                           : (pc.asw == 3 ? k_groups<2, 3> : k_groups<2, 1>);
     if (pc.k == 12) {      // 288 threads (2 patches x 144 positions); validate() bounds the group's shared memory
