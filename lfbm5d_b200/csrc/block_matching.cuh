@@ -845,6 +845,15 @@ __global__ void __launch_bounds__(128) k_bm_select_fast(SelGeom g, const float *
     if (nSx == 1) { dst[1] = idx_of((unsigned) (top[0] & 0xffffffffu)); out_count[r] = 2; } else out_count[r] = nSx;
 }
 
+// N = 1 has no self search: every reference patch r in [r0, r1) is its own only match (core:3448-3460)
+__global__ void k_bm_identity(const int *rows, const int *cols, int nc, int w, int r0, int r1, int N, unsigned *out_count, unsigned *out_idx)
+{
+    const int r = r0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= r1) return;
+    out_count[r] = 1;
+    out_idx[(size_t) r * (N + 1)] = (unsigned) (rows[r / nc] * w + cols[r % nc]);
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // Disparity matching (core:3576-3608): one thread per position, walking the skewed layout k_sat2 writes so that
 // the (2*nDisp+1)^2 plane reads are coalesced. Only element [0] of the sorted list and the shape flag are consumed

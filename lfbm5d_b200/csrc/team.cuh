@@ -358,9 +358,6 @@ int team_pass_bm(lfbm5d_team *T, const PassCfg &pc, const LfWindow &win, int pst
                 }
                 if (tm) CK(cudaEventRecord(T->bev[1], ctx->stream));
                 if (pg.nself > 0) {
-                    SelGeom sg{};
-                    sg.w = pc.wb; sg.nSim = pc.nSim; sg.Ns = pg.Ns; sg.N = pc.N; sg.R = pg.R; sg.nc = pg.nc; sg.threshold = pg.threshold;
-                    sg.rows = ctx->rows.as<int>(); sg.cols = ctx->cols.as<int>();
                     TeamCtxBufs *b = team_bufs(ctx);
                     void (*kp)(SelGeom, const float *, const float *, int, int, unsigned *, unsigned long long *) = nullptr;
                     switch (pc.N) {
@@ -370,7 +367,7 @@ int team_pass_bm(lfbm5d_team *T, const PassCfg &pc, const LfWindow &win, int pst
                         case 16: kp = k_bm_partial<17>; break;
                         default: kp = k_bm_partial<33>; break;
                     }
-                    LAUNCH(ctx, kp, (pg.R + 127) / 128, 128, 0, sg, ctx->s_at.as<float>(), ctx->s_mir.as<float>(), sh.pl0, sh.pl1,
+                    LAUNCH(ctx, kp, (pg.R + 127) / 128, 128, 0, sel_geom(ctx, pc), ctx->s_at.as<float>(), ctx->s_mir.as<float>(), sh.pl0, sh.pl1,
                            b->pcnt_send.as<unsigned>(), b->pkey_send.as<unsigned long long>());
                 }
                 if (tm) CK(cudaEventRecord(T->bev[2], ctx->stream));
@@ -436,9 +433,7 @@ int team_pass_body(lfbm5d_team *T, const PassCfg &pc, bool redo)
         const int nown = bd.r1 - bd.r0;
         if (nown > 0) {
             if (pg.nself > 0 && !redo) {
-                SelGeom sg{};
-                sg.w = pc.wb; sg.nSim = pc.nSim; sg.Ns = pg.Ns; sg.N = pc.N; sg.R = pg.R; sg.nc = pg.nc; sg.threshold = pg.threshold;
-                sg.rows = ctx->rows.as<int>(); sg.cols = ctx->cols.as<int>();
+                const SelGeom sg = sel_geom(ctx, pc);
                 void (*km)(SelGeom, int, int, int, const unsigned *, const unsigned long long *, unsigned *, unsigned *, unsigned *, unsigned *) = nullptr;
                 switch (pc.N) {
                     case 2: km = k_bm_merge<3>; break;
@@ -466,7 +461,7 @@ int team_pass_body(lfbm5d_team *T, const PassCfg &pc, bool redo)
             } else if (pg.nself > 0) {      // ties somewhere: every rank now holds the complete sums, the reference's selection as on one GPU
                 if (launch_self_select(ctx, pc, ctx->stream)) return 1;
             } else
-                LAUNCH(ctx, k_bm_identity_rows, (nown + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, wb, bd.r0, bd.r1, (int) pc.N,
+                LAUNCH(ctx, k_bm_identity, (nown + 255) / 256, 256, 0, ctx->rows.as<int>(), ctx->cols.as<int>(), pg.nc, wb, bd.r0, bd.r1, (int) pc.N,
                        ctx->bmcount.as<unsigned>(), ctx->bmidx.as<unsigned>());
             if (launch_group_masks(ctx, pc, win, pst, bd.r0, bd.r1)) return 1;
             if (clear_zero_blocks(ctx, pc) || launch_groups(ctx, pc, win, pst, partial, bd.r0, bd.r1)) return 1;
@@ -583,10 +578,7 @@ int team_pass_finish(lfbm5d_team *T, const PassCfg &pc, unsigned long long *cov)
         lfbm5d_ctx *ctx = T->local[l];
         const Band &bd = T->bands[T->local_rank[l]];
         CK(cudaSetDevice(ctx->device));
-        if (bd.c1 > bd.y0)
-            LAUNCH(ctx, k_pad_rows, grid_for(ctx, (size_t) pc.A * (bd.c1 - bd.y0) * pc.wb), 256, 0, T->d_noisy[l], pc.step == 2 ? T->d_basic[l] : (const float *) nullptr,
-                   ctx->num.as<float>(), ctx->den.as<float>(), ctx->nsym.as<float>(), ctx->bsym.as<float>(), ctx->numsym.as<float>(),
-                   ctx->densym.as<float>(), ctx->est0.as<float>(), win, (int) pc.W, (int) pc.H, (int) pc.C, (int) pc.n, bd.y0, bd.c1 - bd.y0, bd.y1);
+        launch_pad(ctx, pc, win, T->d_noisy[l], pc.step == 2 ? T->d_basic[l] : nullptr, bd.y0, bd.c1, bd.y1);
     }
     if (team_pass_body(T, pc, true) || team_pass_read(T, cov, &ties)) return 1;
     return 0;
@@ -623,13 +615,10 @@ int team_count_zero(lfbm5d_team *T, const std::vector<unsigned> &items, bool pad
         unsigned long long *cnts = reinterpret_cast<unsigned long long *>(team_bufs(ctx)->counters.as<char>() + cslot(T, g));
         CK(cudaMemsetAsync(cnts, 0, 64 * 8, ctx->stream));
         for (int i = 0; i < nit; i++) {
-            if (padded) {      // padded weights of window slot items[i], all channels, own rows [y0, y1)
-                if (bd.y1 > bd.y0)
-                    LAUNCH(ctx, k_count_zero_rows, grid_for(ctx, (size_t) pc.C * (bd.y1 - bd.y0) * pc.wb), 256, 0,
-                           ctx->densym.as<float>() + (size_t) items[i] * pc.C * pc.wb * pc.hb, (int) pc.C, (size_t) pc.wb * pc.hb, (int) pc.wb, bd.y0, bd.y1 - bd.y0, cnts + i);
-            } else if (bd.i1 > bd.i0)
-                LAUNCH(ctx, k_count_zero_rows, grid_for(ctx, (size_t) pc.C * (bd.i1 - bd.i0) * pc.W), 256, 0,
-                       ctx->den.as<float>() + (size_t) items[i] * pc.C * pc.W * pc.H, (int) pc.C, (size_t) pc.W * pc.H, (int) pc.W, bd.i0, bd.i1 - bd.i0, cnts + i);
+            if (padded)      // padded weights of window slot items[i], all channels, own rows [y0, y1)
+                launch_count_zero(ctx, ctx->densym.as<float>() + (size_t) items[i] * pc.C * pc.wb * pc.hb, (int) pc.C, (int) pc.wb, (int) pc.hb, bd.y0, bd.y1, cnts + i);
+            else
+                launch_count_zero(ctx, ctx->den.as<float>() + (size_t) items[i] * pc.C * pc.W * pc.H, (int) pc.C, (int) pc.W, (int) pc.H, bd.i0, bd.i1, cnts + i);
         }
     }
     std::vector<TeamSeg> segs;
@@ -840,12 +829,10 @@ int team_step_begin(lfbm5d_team *T, int step, const lfbm5d_params *p_, float *co
         ctx->sched.clear();
         if (ctx->mask.ensure(asize * 4) || ctx->num.ensure(asize * each * 4) || ctx->den.ensure(asize * each * 4)) return 1;
         CK(cudaMemcpyAsync(ctx->mask.p, S.mask.data(), asize * 4, cudaMemcpyHostToDevice, ctx->stream));
-        if (S.docolor && bd.j1 > bd.j0) {      // only the rows this rank's groups read (own band + the rows it shares with the next rank)
-            LAUNCH(ctx, k_color_rows, grid_for(ctx, (size_t) asize * (bd.j1 - bd.j0) * p->width), 256, 0, T->d_noisy[l], ctx->mask.as<unsigned>(), asize,
-                   (int) p->width, (int) p->height, p->color_space, 1, bd.j0, bd.j1 - bd.j0);
+        if (S.docolor) {      // only the rows this rank's groups read (own band + the rows it shares with the next rank)
+            launch_color(ctx, ctx->stream, T->d_noisy[l], T->d_noisy[l], ctx->mask.as<unsigned>(), asize, p->width, p->height, p->color_space, 1, bd.j0, bd.j1);
             if (step == 2 && !late_gather)
-                LAUNCH(ctx, k_color_rows, grid_for(ctx, (size_t) asize * (bd.j1 - bd.j0) * p->width), 256, 0, T->d_basic[l], ctx->mask.as<unsigned>(), asize,
-                       (int) p->width, (int) p->height, p->color_space, 1, bd.j0, bd.j1 - bd.j0);
+                launch_color(ctx, ctx->stream, T->d_basic[l], T->d_basic[l], ctx->mask.as<unsigned>(), asize, p->width, p->height, p->color_space, 1, bd.j0, bd.j1);
         }
         CK(cudaMemsetAsync(ctx->num.p, 0, asize * each * 4, ctx->stream));
         CK(cudaMemsetAsync(ctx->den.p, 0, asize * each * 4, ctx->stream));
@@ -858,9 +845,8 @@ int team_step_begin(lfbm5d_team *T, int step, const lfbm5d_params *p_, float *co
             lfbm5d_ctx *ctx = T->local[l];
             const Band &bd = T->bands[T->local_rank[l]];
             CK(cudaSetDevice(ctx->device));
-            if (S.docolor && bd.j1 > bd.j0)
-                LAUNCH(ctx, k_color_rows, grid_for(ctx, (size_t) asize * (bd.j1 - bd.j0) * p->width), 256, 0, T->d_basic[l], ctx->mask.as<unsigned>(), asize,
-                       (int) p->width, (int) p->height, p->color_space, 1, bd.j0, bd.j1 - bd.j0);
+            if (S.docolor)
+                launch_color(ctx, ctx->stream, T->d_basic[l], T->d_basic[l], ctx->mask.as<unsigned>(), asize, p->width, p->height, p->color_space, 1, bd.j0, bd.j1);
         }
     }
     for (int l = 0; l < nl; l++) {
@@ -913,11 +899,10 @@ int team_select(lfbm5d_team *T, unsigned &ps, unsigned &pt)
 int team_window_prepass(lfbm5d_team *T)
 {
     StepState &S = T->ss;
-    const int step = S.step, nl = (int) T->local.size();
+    const int nl = (int) T->local.size();
     const PassCfg &pc = S.pc;
     WindowRun &wf = T->wf;
     const LfWindow &win = wf.win;
-    const unsigned Aw = (unsigned) win.A, C = S.p.chnls;
     if (window_next(wf, [&](const std::vector<unsigned> &slots, std::vector<unsigned long long> &zeros) {
             return team_count_zero(T, slots, true, pc, zeros);
         })) return 1;
@@ -926,9 +911,7 @@ int team_window_prepass(lfbm5d_team *T)
             lfbm5d_ctx *ctx = T->local[l];
             const Band &bd = T->bands[T->local_rank[l]];
             CK(cudaSetDevice(ctx->device));
-            if (bd.y1 > bd.y0)
-                LAUNCH(ctx, k_est0_rows, grid_for(ctx, (size_t) Aw * (bd.y1 - bd.y0) * pc.wb), 256, 0, step == 1 ? ctx->nsym.as<float>() : ctx->bsym.as<float>(),
-                       ctx->numsym.as<float>(), ctx->densym.as<float>(), ctx->est0.as<float>(), win, (int) pc.wb, (int) pc.hb, (int) C, bd.y0, bd.y1 - bd.y0);
+            launch_est0(ctx, pc, win, bd.y0, bd.y1);
         }
     TMARK(1);
     if (team_est0_exchange(T, pc, win)) return 1;
@@ -942,7 +925,6 @@ int team_window_begin(lfbm5d_team *T, unsigned ps, unsigned pt, int force_sadct)
     const lfbm5d_params *p = &S.p;
     const int step = S.step, nl = (int) T->local.size();
     const PassCfg &pc = S.pc;
-    const unsigned C = p->chnls, W = p->width, H = p->height;
     if (window_open(S, T->wf, ps, pt, force_sadct))
         for (int l = 0; l < nl; l++) { CK(cudaSetDevice(T->local[l]->device)); if (setup_tables(T->local[l], step, p, S.tau_4D)) return 1; }
     const LfWindow &win = T->wf.win;
@@ -951,10 +933,7 @@ int team_window_begin(lfbm5d_team *T, unsigned ps, unsigned pt, int force_sadct)
         lfbm5d_ctx *ctx = T->local[l];
         const Band &bd = T->bands[T->local_rank[l]];
         CK(cudaSetDevice(ctx->device));
-        if (bd.c1 > bd.y0)
-            LAUNCH(ctx, k_pad_rows, grid_for(ctx, (size_t) win.A * (bd.c1 - bd.y0) * pc.wb), 256, 0, T->d_noisy[l], step == 2 ? T->d_basic[l] : (const float *) nullptr,
-                   ctx->num.as<float>(), ctx->den.as<float>(), ctx->nsym.as<float>(), ctx->bsym.as<float>(), ctx->numsym.as<float>(),
-                   ctx->densym.as<float>(), ctx->est0.as<float>(), win, (int) W, (int) H, (int) C, (int) pc.n, bd.y0, bd.c1 - bd.y0, bd.y1);
+        launch_pad(ctx, pc, win, T->d_noisy[l], step == 2 ? T->d_basic[l] : nullptr, bd.y0, bd.c1, bd.y1);
     }
     if (!T->wf.n_unproc) return 0;
     return team_window_prepass(T);
@@ -963,13 +942,10 @@ int team_window_begin(lfbm5d_team *T, unsigned ps, unsigned pt, int force_sadct)
 int team_window_finish(lfbm5d_team *T, lfbm5d_team *sched_to)
 {
     StepState &S = T->ss;
-    const lfbm5d_params *p = &S.p;
     const int nl = (int) T->local.size();
     const PassCfg &pc = S.pc;
-    const unsigned C = p->chnls, W = p->width, H = p->height;
     WindowRun &wf = T->wf;
     const LfWindow &win = wf.win;
-    const unsigned Aw = (unsigned) win.A;
     while (wf.n_unproc) {
         unsigned long long cnt = 0;
         if (team_pass_finish(T, pc, &cnt)) return 1;
@@ -979,9 +955,7 @@ int team_window_finish(lfbm5d_team *T, lfbm5d_team *sched_to)
             lfbm5d_ctx *ctx = T->local[l];
             const Band &bd = T->bands[T->local_rank[l]];
             CK(cudaSetDevice(ctx->device));
-            if (bd.j1 > bd.j0)
-                LAUNCH(ctx, k_unpad_rows, grid_for(ctx, (size_t) Aw * C * (bd.j1 - bd.j0) * W), 256, 0, ctx->num.as<float>(), ctx->den.as<float>(),
-                       ctx->numsym.as<float>(), ctx->densym.as<float>(), win, (int) W, (int) H, (int) C, (int) pc.n, bd.j0, bd.j1 - bd.j0);
+            launch_unpad(ctx, pc, win, bd.j0, bd.j1, nullptr);
         }
         if (!window_after_call(S, wf, cnt)) break;
         if (team_window_prepass(T)) return 1;
@@ -1005,25 +979,20 @@ int team_step_end(lfbm5d_team *T, float *const *d_out, int gather)
     StepState &S = T->ss;
     const lfbm5d_params *p = &S.p;
     const int nl = (int) T->local.size(), G = T->world;
-    const unsigned asize = S.asize(), C = p->chnls;
+    const unsigned asize = S.asize();
     const int W = (int) p->width, H = (int) p->height;
     for (int l = 0; l < nl; l++) {
         lfbm5d_ctx *ctx = T->local[l];
         const Band &bd = T->bands[T->local_rank[l]];
         CK(cudaSetDevice(ctx->device));
-        if (bd.j1 > bd.j0)
-            LAUNCH(ctx, k_final_rows, grid_for(ctx, (size_t) asize * (bd.j1 - bd.j0) * W), 256, 0, ctx->num.as<float>(), ctx->den.as<float>(), T->d_noisy[l],
-                   T->d_basic[l], d_out[l], ctx->mask.as<unsigned>(), asize, W, H, (int) C, S.step, p->color_space, S.docolor ? 1 : 0, bd.j0, bd.j1 - bd.j0);
+        launch_final(ctx, S, T->d_noisy[l], T->d_basic[l], d_out[l], 0, asize, 1, bd.j0, bd.j1);
         if (S.docolor) {      // rows this rank never transformed: leave them as the reference leaves its inputs (colour round trip)
             const int lo[2] = { 0, bd.j1 }, hi[2] = { bd.j0, H };
-            for (int q = 0; q < 2; q++)
-                if (hi[q] > lo[q]) {
-                    LAUNCH(ctx, k_color_rows, grid_for(ctx, (size_t) asize * (hi[q] - lo[q]) * W), 256, 0, T->d_noisy[l], ctx->mask.as<unsigned>(), asize, W, H,
-                           p->color_space, 2, lo[q], hi[q] - lo[q]);
-                    if (S.step == 2)
-                        LAUNCH(ctx, k_color_rows, grid_for(ctx, (size_t) asize * (hi[q] - lo[q]) * W), 256, 0, T->d_basic[l], ctx->mask.as<unsigned>(), asize, W, H,
-                               p->color_space, 2, lo[q], hi[q] - lo[q]);
-                }
+            for (int q = 0; q < 2; q++) {
+                launch_color(ctx, ctx->stream, T->d_noisy[l], T->d_noisy[l], ctx->mask.as<unsigned>(), asize, W, H, p->color_space, 2, lo[q], hi[q]);
+                if (S.step == 2)
+                    launch_color(ctx, ctx->stream, T->d_basic[l], T->d_basic[l], ctx->mask.as<unsigned>(), asize, W, H, p->color_space, 2, lo[q], hi[q]);
+            }
         }
         CK(cudaGetLastError());
     }
