@@ -1763,94 +1763,29 @@ unsigned lfbm5d_debug_schedule(lfbm5d_ctx *ctx, unsigned *out, unsigned max_entr
     return n;
 }
 
-int lfbm5d_debug_pass(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *noisy_sym, const float *basic_sym,
-                      float *num_sym_io, float *den_sym_io, const unsigned *mask_asw, const unsigned *procSAI_asw, unsigned pst,
-                      unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
+// Set-up shared by the two debug exports: the parameters are validated as one window of (2 an + 1)^2 SAIs, the tables and buffers of
+// a pass are made ready, and `win` becomes the identity window (window SAI a is plane a); the caller sets its mask and proc flags.
+static int debug_setup(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, PassCfg &pc, LfWindow &win)
 {
-    return lfbm5d_debug_pass_ex(ctx, step, p, noisy_sym, basic_sym, num_sym_io, den_sym_io, mask_asw, procSAI_asw, pst, pst, out_count, out_idx,
-                                out_first, out_shape);
-}
-
-int lfbm5d_debug_pass_ex(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *noisy_sym, const float *basic_sym,
-                         float *num_sym_io, float *den_sym_io, const unsigned *mask_asw, const unsigned *procSAI_asw, unsigned cst, unsigned pst,
-                         unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
-{
-    if (!ctx || !noisy_sym || !num_sym_io || !den_sym_io || !mask_asw || !procSAI_asw) return fail("null argument");
-    if (step != 1 && step != 2) return fail("step must be 1 or 2");
-    if (step == 2 && !basic_sym) return fail("step 2 needs the basic estimate");
     lfbm5d_params q = *p;
     if (q.awidth < 2 * q.an + 1) q.awidth = 2 * q.an + 1;
     if (q.aheight < 2 * q.an + 1) q.aheight = 2 * q.an + 1;
     if (validate(&q, step)) return 1;
     CK(cudaSetDevice(ctx->device));
-    PassCfg pc;
     if (make_passcfg(pc, step, p, p->tau_4D) || setup_tables(ctx, step, p, p->tau_4D) || ensure_pass_buffers(ctx, pc) || upload_grid(ctx, pc))
         return 1;
-    if (pst >= pc.A) return fail("pst out of range");
-    const size_t plane = (size_t) pc.wb * pc.hb, bytes = pc.A * pc.C * plane * 4;
-    LfWindow win{};
     win.A = (int) pc.A;
-    for (unsigned a = 0; a < pc.A; a++) { win.st[a] = (int) a; win.mask[a] = mask_asw[a]; win.proc[a] = procSAI_asw[a]; }
-    CK(cudaMemcpyAsync(ctx->nsym.p, noisy_sym, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    if (step == 2) CK(cudaMemcpyAsync(ctx->bsym.p, basic_sym, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->numsym.p, num_sym_io, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->densym.p, den_sym_io, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemsetAsync(ctx->first.p, 0xFF, pc.A * plane * 4, ctx->stream));
-    CK(cudaMemsetAsync(ctx->shape.p, 0, pc.A * plane, ctx->stream));
-    launch_est0(ctx, pc, win, 0, (int) pc.hb);
-    if (cst >= pc.A) return fail("cst out of range");
-    if (run_pass(ctx, pc, win, (int) pst, (int) cst)) return 1;
-    CK(cudaMemcpyAsync(num_sym_io, ctx->numsym.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(den_sym_io, ctx->densym.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    const size_t R = pc.rows.size() * pc.cols.size(), nc = pc.cols.size();
-    if (out_count && out_idx) {
-        std::vector<unsigned> cnt(R), idx(R * (pc.N + 1));
-        CK(cudaMemcpy(cnt.data(), ctx->bmcount.p, R * 4, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(idx.data(), ctx->bmidx.p, R * (pc.N + 1) * 4, cudaMemcpyDeviceToHost));
-        memset(out_count, 0, plane * 4);
-        for (size_t r = 0; r < R; r++) {
-            const size_t k_r = (size_t) pc.rows[r / nc] * pc.wb + pc.cols[r % nc];
-            out_count[k_r] = cnt[r];
-            for (unsigned n = 0; n < cnt[r]; n++) out_idx[k_r * (pc.N + 1) + n] = idx[r * (pc.N + 1) + n];
-        }
-    }
-    if (out_first) CK(cudaMemcpy(out_first, ctx->first.p, pc.A * plane * 4, cudaMemcpyDeviceToHost));
-    if (out_shape) {
-        std::vector<unsigned char> s(pc.A * plane);
-        CK(cudaMemcpy(s.data(), ctx->shape.p, pc.A * plane, cudaMemcpyDeviceToHost));
-        for (size_t i = 0; i < s.size(); i++) out_shape[i] = s[i];
-    }
+    for (unsigned a = 0; a < pc.A; a++) win.st[a] = (int) a;
     return 0;
 }
 
-
-int lfbm5d_debug_block_matching(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *planes, unsigned nplanes,
-                                unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
+// Read-back shared by the two debug exports, after the stream has drained: the match lists scattered onto the padded positions of
+// their reference patches, and the disparity argmin and shape flags of the first `nplanes` planes.
+static int debug_readback(lfbm5d_ctx *ctx, const PassCfg &pc, unsigned nplanes, unsigned *out_count, unsigned *out_idx, unsigned *out_first,
+                          unsigned *out_shape)
 {
-    if (!ctx || !p || !planes) return fail("null argument");
-    if (step != 1 && step != 2) return fail("step must be 1 or 2");
-    lfbm5d_params q = *p;
-    if (q.awidth < 2 * q.an + 1) q.awidth = 2 * q.an + 1;
-    if (q.aheight < 2 * q.an + 1) q.aheight = 2 * q.an + 1;
-    if (validate(&q, step)) return 1;
-    CK(cudaSetDevice(ctx->device));
-    PassCfg pc;
-    if (make_passcfg(pc, step, p, p->tau_4D) || setup_tables(ctx, step, p, p->tau_4D) || ensure_pass_buffers(ctx, pc) || upload_grid(ctx, pc))
-        return 1;
-    if (nplanes < 1 || nplanes > pc.A) return fail("1 <= nplanes <= (2*an+1)^2");
-    const size_t plane = (size_t) pc.wb * pc.hb;
-    LfWindow win{};
-    win.A = (int) pc.A;
-    for (unsigned a = 0; a < pc.A; a++) { win.st[a] = (int) a; win.mask[a] = a < nplanes; win.proc[a] = a >= nplanes; }
-    CK(cudaMemcpyAsync(ctx->est0.p, planes, nplanes * plane * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemsetAsync(ctx->first.p, 0xFF, pc.A * plane * 4, ctx->stream));
-    CK(cudaMemsetAsync(ctx->shape.p, 0, pc.A * plane, ctx->stream));
-    ctx->bm_only = true;
-    const int rc = run_pass(ctx, pc, win, 0, 0);
-    ctx->bm_only = false;
-    if (rc) return 1;
     CK(cudaStreamSynchronize(ctx->stream));
+    const size_t plane = (size_t) pc.wb * pc.hb;
     const size_t R = pc.rows.size() * pc.cols.size(), nc = pc.cols.size();
     if (out_count && out_idx) {
         std::vector<unsigned> cnt(R), idx(R * (pc.N + 1));
@@ -1870,6 +1805,63 @@ int lfbm5d_debug_block_matching(lfbm5d_ctx *ctx, int step, const lfbm5d_params *
         for (size_t i = 0; i < sh.size(); i++) out_shape[i] = sh[i];
     }
     return 0;
+}
+
+int lfbm5d_debug_pass(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *noisy_sym, const float *basic_sym,
+                      float *num_sym_io, float *den_sym_io, const unsigned *mask_asw, const unsigned *procSAI_asw, unsigned pst,
+                      unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
+{
+    return lfbm5d_debug_pass_ex(ctx, step, p, noisy_sym, basic_sym, num_sym_io, den_sym_io, mask_asw, procSAI_asw, pst, pst, out_count, out_idx,
+                                out_first, out_shape);
+}
+
+int lfbm5d_debug_pass_ex(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *noisy_sym, const float *basic_sym,
+                         float *num_sym_io, float *den_sym_io, const unsigned *mask_asw, const unsigned *procSAI_asw, unsigned cst, unsigned pst,
+                         unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
+{
+    if (!ctx || !noisy_sym || !num_sym_io || !den_sym_io || !mask_asw || !procSAI_asw) return fail("null argument");
+    if (step != 1 && step != 2) return fail("step must be 1 or 2");
+    if (step == 2 && !basic_sym) return fail("step 2 needs the basic estimate");
+    PassCfg pc;
+    LfWindow win{};
+    if (debug_setup(ctx, step, p, pc, win)) return 1;
+    if (pst >= pc.A) return fail("pst out of range");
+    const size_t plane = (size_t) pc.wb * pc.hb, bytes = pc.A * pc.C * plane * 4;
+    for (unsigned a = 0; a < pc.A; a++) { win.mask[a] = mask_asw[a]; win.proc[a] = procSAI_asw[a]; }
+    CK(cudaMemcpyAsync(ctx->nsym.p, noisy_sym, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (step == 2) CK(cudaMemcpyAsync(ctx->bsym.p, basic_sym, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->numsym.p, num_sym_io, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->densym.p, den_sym_io, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(ctx->first.p, 0xFF, pc.A * plane * 4, ctx->stream));
+    CK(cudaMemsetAsync(ctx->shape.p, 0, pc.A * plane, ctx->stream));
+    launch_est0(ctx, pc, win, 0, (int) pc.hb);
+    if (cst >= pc.A) return fail("cst out of range");
+    if (run_pass(ctx, pc, win, (int) pst, (int) cst)) return 1;
+    CK(cudaMemcpyAsync(num_sym_io, ctx->numsym.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(den_sym_io, ctx->densym.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    return debug_readback(ctx, pc, pc.A, out_count, out_idx, out_first, out_shape);
+}
+
+
+int lfbm5d_debug_block_matching(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, const float *planes, unsigned nplanes,
+                                unsigned *out_count, unsigned *out_idx, unsigned *out_first, unsigned *out_shape)
+{
+    if (!ctx || !p || !planes) return fail("null argument");
+    if (step != 1 && step != 2) return fail("step must be 1 or 2");
+    PassCfg pc;
+    LfWindow win{};
+    if (debug_setup(ctx, step, p, pc, win)) return 1;
+    if (nplanes < 1 || nplanes > pc.A) return fail("1 <= nplanes <= (2*an+1)^2");
+    const size_t plane = (size_t) pc.wb * pc.hb;
+    for (unsigned a = 0; a < pc.A; a++) { win.mask[a] = a < nplanes; win.proc[a] = a >= nplanes; }
+    CK(cudaMemcpyAsync(ctx->est0.p, planes, nplanes * plane * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(ctx->first.p, 0xFF, pc.A * plane * 4, ctx->stream));
+    CK(cudaMemsetAsync(ctx->shape.p, 0, pc.A * plane, ctx->stream));
+    ctx->bm_only = true;
+    const int rc = run_pass(ctx, pc, win, 0, 0);
+    ctx->bm_only = false;
+    if (rc) return 1;
+    return debug_readback(ctx, pc, nplanes, out_count, out_idx, out_first, out_shape);
 }
 
 } // extern "C"

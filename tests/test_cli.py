@@ -8,9 +8,7 @@ import numpy as np
 import pytest
 
 import lfdata
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIBDIR = os.path.join(ROOT, "lfbm5d_b200", "_lib")
+from gpucheck import LIBDIR, check_pngs, run_cli, write_lf
 
 
 def test_cli_binary_and_host_library_exist():
@@ -28,23 +26,14 @@ def test_cli_binary_and_host_library_exist():
 def test_cli_readme_command(tmp_path):
     from PIL import Image
     clean = lfdata.synth_lf(3, 3, 64, 72)
-    src = tmp_path / "sourceLF"
-    for d in ("sourceLF", "noisyLF", "basicLF", "denoisedLF", "diffLF"):
-        (tmp_path / d).mkdir()
-    for s in range(3):
-        for t in range(3):
-            img = np.clip(np.floor(clean[s * 3 + t] + 0.5), 0, 255).astype(np.uint8).transpose(1, 2, 0)
-            Image.fromarray(img).save(str(src / ("SAI_%02d_%02d.png" % (s + 1, t + 1))))
+    src = write_lf(tmp_path, clean, 3)
     report = tmp_path / "objectiveResults.txt"
     # README.md:50 command line
     args = [os.path.join(LIBDIR, "LFBM5Ddenoising"), str(src), "SAI", "_", "3", "3", "1", "1", "1", "1", "row", "25", "2.7",
             str(tmp_path / "noisyLF"), str(tmp_path / "basicLF"), str(tmp_path / "denoisedLF"), str(tmp_path / "diffLF"),
             "8", "18", "6", "16", "4", "id", "sadct", "haar", "0", "16", "18", "6", "8", "4", "dct", "sadct", "haar", "0",
             "opp", "0", str(report)]
-    env = dict(os.environ, LFBM5D_SEED="20171016")
-    p = subprocess.run(args, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, env=env, timeout=300)
-    out = p.stdout.decode()
-    assert p.returncode == 0, out[-2000:]
+    out = run_cli(args)
     assert "Step 1 done in" in out and "Step 2 done in" in out and "THIS IS THE END" in out
     for d in ("noisyLF", "basicLF", "denoisedLF", "diffLF"):
         assert len(os.listdir(str(tmp_path / d))) == 9
@@ -66,15 +55,7 @@ def test_cli_readme_command(tmp_path):
     basic, n1 = eng.step1(p1, noisy, mask)
     out, b2, n2 = eng.step2(p2, n1, basic, mask)
     eng.close()
-
-    def as_png(x):
-        return np.clip(np.floor(x + np.float32(0.5)), 0, 255).astype(np.uint8)
-    for s in range(3):
-        for t in range(3):
-            st = s * 3 + t
-            for d, arr in (("noisyLF", noisy), ("basicLF", basic), ("denoisedLF", out)):      # basic is saved before step 2 round-trips it
-                img = np.asarray(Image.open(str(tmp_path / d / ("SAI_%02d_%02d.png" % (s + 1, t + 1))))).transpose(2, 0, 1)
-                assert np.array_equal(img, as_png(arr[st])), (d, st)
+    check_pngs(tmp_path, (("noisyLF", noisy), ("basicLF", basic), ("denoisedLF", out)), 3)      # basic is saved before step 2 round-trips it
     blocks = re.findall(r"-> Average PSNR (\w+) = ([0-9.]+)\n-> Standard deviation PSNR \w+ = ([0-9.e+-]+)\nPSNR for all \w+ SAIs:\n((?:[0-9. ]+\n){3})", txt)
     assert [b[0] for b in blocks] == ["noisy", "basic", "denoised"]
     for (name, avg, std, rows), arr in zip(blocks, (noisy, basic, out)):
@@ -82,10 +63,8 @@ def test_cli_readme_command(tmp_path):
         got = [float(v) for v in rows.split()]
         assert np.allclose(got, want, rtol=0, atol=1e-4) and abs(float(avg) - np.mean(want)) < 2e-4, (name, got, want)   # 6 significant digits printed
     # second mode: no ground truth, noisy light field read back from disk (utilities_LF.cpp:1187)
-    args2 = list(args)
-    args2[1] = "none"
-    p = subprocess.run(args2, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, env=env, timeout=300)
-    assert p.returncode == 0 and b"Loading noisy LF elapsed time" in p.stdout
+    args[1] = "none"
+    assert "Loading noisy LF elapsed time" in run_cli(args)
 
 
 @pytest.mark.gpu

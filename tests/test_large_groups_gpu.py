@@ -2,45 +2,24 @@
 clusters of 2 or 4 CTAs that share the group through distributed shared memory (k_groups_cl). GPU against the CPU oracle through
 the C ABI. The oracle is generic in N but pinned against the reference only at the N values of the other tests, so these results
 are checked GPU vs oracle: match lists, disparity argmin and shape flags bit-exact; step 1 accumulators and LF_basic bit-identical;
-complete runs within 0.01 dB; step 2 within the rounding bound of the oracle's group sums (wiener_tol below)."""
+complete runs within 0.01 dB; step 2 within the rounding bound of the oracle's group sums (gpucheck.wiener_tol)."""
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import golden_inputs as gi
 import lfdata
-from test_gpu_parity import estimate
-from test_patch12_gpu import check_files, psnr_on, write_lf
+from gpucheck import (LIBDIR, assert_team_matches_single, check_complete_run, check_pass, check_pngs, eng, estimate, psnr_on,
+                      run_cli, wiener_tol, write_lf)  # noqa: F401 (eng is the engine fixture)
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIBDIR = os.path.join(ROOT, "lfbm5d_b200", "_lib")
 K = 16
-
-
-@pytest.fixture(scope="module")
-def eng():
-    import lfbm5d_b200 as L
-    e = L.LFBM5D(0)
-    yield e
-    e.close()
 
 
 def expected_cluster(step, N):
     """CTAs per group: one channel of the group is N * 9 * 16 * RS * 4 B (RS = 16 for id, 17 otherwise), twice that in step 2."""
     return {(1, 32): 2, (2, 16): 2, (2, 32): 4}[(step, N)]
-
-
-def wiener_tol(N, useSD):
-    """Relative tolerance of a step-2 pass. Like the reference, the oracle adds the N * 9 * 256 Wiener coefficients of a group
-    (and useSD's sums) one by one in float; the error of such a sum of n non-negative terms is bounded by (n - 1) * 2^-24 of the
-    sum, which grows with the group and is far above the 2e-5 of test_gpu_parity.py at these N. Measured on one B200 on the
-    inputs below: switching the oracle's weight sum to double moves the oracle by up to 2.1e-4 at N = 32 (5e-5 already at N = 8
-    on the one-CTA k_groups), while the GPU, which sums in blocks and then in rank order, stays within 3e-6 of the double sum.
-    A wrong patch, coefficient or weight gives errors of order 1e-1 and more."""
-    return max(1e-4 if useSD else 2e-5, N * 9 * 256 * 2.0 ** -24)
 
 
 def spread_inputs(H=40, W=48):
@@ -54,35 +33,19 @@ def spread_inputs(H=40, W=48):
 
 
 def check_pass_cl(eng, oracle, step, sym, basic, num0, den0, mask, proc, N, t2, t4, t5, lam=2.7, useSD=0, pst=4, cst=None, spread=False):
+    """check_pass at k = 16 on the cluster size the group needs, step 2 and useSD within wiener_tol."""
     import lfbm5d_b200 as L
     A, C, hb, wb = sym.shape
-    H, W = hb - 48, wb - 48
-    oracle.lib().orc_set_use_sd(int(useSD))
-    try:
-        on, od, odbg = oracle.run_pass(step, sym, basic, num0, den0, mask, proc, pst, 3, 25.0, lam, 18, 6, K, N, 4, t2, t4, t5, debug=True,
-                                       cst=cst)
-    finally:
-        oracle.lib().orc_set_use_sd(0)
-    prm = L.make_params(25.0, lam, 3, 3, 1, W, H, C, N, 18, 6, K, 4, t2, t4, t5, useSD=int(useSD))
+    prm = L.make_params(25.0, lam, 3, 3, 1, wb - 48, hb - 48, C, N, 18, 6, K, 4, t2, t4, t5, useSD=int(useSD))
     cl, occ = eng.group_cluster(step, prm)
     assert cl == expected_cluster(step, N) and occ > 0, (cl, occ)
-    gn, gd, gdbg = eng.debug_pass(step, prm, sym, basic, num0, den0, mask, proc, pst, debug=True, cst=cst)
-    assert np.array_equal(odbg[0], gdbg[0]), "self-match counts differ"
-    m = np.arange(N + 1)[None, :] < odbg[0][:, None]
-    assert np.array_equal(odbg[1] * m, gdbg[1] * m), "self-match lists differ"
-    assert np.array_equal(odbg[2], gdbg[2]), "disparity argmin differs"
-    assert np.array_equal(odbg[3], gdbg[3]), "shape flags differ"
-    assert np.array_equal(od != 0, gd != 0)
+    on, od, gn, gd, gdbg = check_pass(eng, oracle, step, sym, basic, num0, den0, mask, proc, K, N, t2, t4, t5, pst=pst, cst=cst, lam=lam,
+                                      useSD=useSD, rel=wiener_tol(N, useSD), est=False)
     if spread:
         # every CTA of the cluster holds patches (nSx = N), and the CTAs hold one patch each or, on 4-CTA clusters, two of them
         # hold none (nSx = 2, the smallest group: a single match is duplicated)
         cnt = gdbg[0][gdbg[0] > 0]
         assert (cnt == N).any() and (cnt == 2).any(), np.unique(cnt)
-    if step == 1 and not useSD:
-        assert np.array_equal(gn, on) and np.array_equal(gd, od)                     # step 1: bit-identical
-    else:
-        tol = wiener_tol(N, useSD)
-        assert np.abs(gn - on).max() <= tol * np.abs(on).max() and np.abs(gd - od).max() <= tol * np.abs(od).max()
     return on, od, gn, gd
 
 
@@ -137,8 +100,8 @@ def test_single_passes_cluster_masked_processed_and_partial(eng, oracle):
     num, den = gi.partial_holes(num, den)
     proc[4] = 1
     for pst in (1, 6):
-        gn, _, _, _ = check_pass_cl(eng, oracle, 1, sym, None, num, den, mask, proc, 32, oracle.ID, oracle.SADCT, oracle.HAAR, pst=pst, cst=4)
-        assert not np.array_equal(gn, num)
+        pon, _, _, _ = check_pass_cl(eng, oracle, 1, sym, None, num, den, mask, proc, 32, oracle.ID, oracle.SADCT, oracle.HAAR, pst=pst, cst=4)
+        assert not np.array_equal(pon, num)
         for N in (16, 32):
             check_pass_cl(eng, oracle, 2, sym, basic, num, den, mask, proc, N, oracle.DCT, oracle.SADCT, oracle.HAAR, lam=0.0, pst=pst, cst=4)
 
@@ -147,61 +110,31 @@ def test_single_passes_cluster_masked_processed_and_partial(eng, oracle):
 def test_complete_runs_cluster(eng, oracle, aw, C, masked, N1, N2):
     """Both steps with the group sizes `8 / 16` and `32 / 32` at k = 16 (an = 1) through the host-buffer and the device-resident
     entry points, with the oracle's window schedule; grayscale with an empty centre SAI takes the partial-window branch."""
-    import torch
     import lfbm5d_b200 as L
     H, W = 32, 36
     clean = np.ascontiguousarray(lfdata.synth_lf(aw, aw, H, W)[:, :C])
-    noisy = oracle.add_noise(clean, 25.0)
     m = np.ones(aw * aw, np.uint32)
     if masked:
         m[(aw * aw) // 2] = 0
     p1 = L.make_params(25.0, 2.7, aw, aw, 1, W, H, C, N1, 18, 6, K, 4, L.ID, L.SADCT, L.HAAR)
     p2 = L.make_params(25.0, 0.0, aw, aw, 1, W, H, C, N2, 18, 6, K, 4, L.DCT, L.SADCT, L.HAAR)
     assert eng.group_cluster(1, p1)[0] == (1 if N1 == 8 else 2) and eng.group_cluster(2, p2)[0] == expected_cluster(2, N2)
-    b, nrt = eng.step1(p1, noisy, m)
-    ob, onrt, sched = oracle.run_step1(noisy, m, 25.0, 2.7, aw, aw, 1, N1, 18, 6, K, 4, oracle.ID, oracle.SADCT, oracle.HAAR)
-    assert np.array_equal(eng.schedule(), sched)
+    noisy, sched, _, d, _, _ = check_complete_run(eng, oracle, clean, m, p1, p2)
     if masked:
         assert sched[:, 3].max() > 1
-    assert np.array_equal(nrt[m == 1], onrt[m == 1])
-    assert np.array_equal(b[m == 1], ob[m == 1])                                  # step 1 is bit-identical
-    d, _, _ = eng.step2(p2, nrt, b, m)
-    od, _, _, sched2 = oracle.run_step2(nrt, ob, m, 25.0, aw, aw, 1, N2, 18, 6, K, 4, oracle.DCT, oracle.SADCT, oracle.HAAR)
-    assert np.array_equal(eng.schedule(), sched2)
     psnr = psnr_on(clean, m)
-    assert abs(psnr(d) - psnr(od)) <= 0.01, (psnr(d), psnr(od))
     assert psnr(d) > psnr(noisy) + 3.0
-    dev = torch.device("cuda", 0)
-    w = torch.from_numpy(noisy.copy()).to(dev)
-    bd, dd = torch.zeros_like(w), torch.zeros_like(w)
-    eng.step1_device(p1, w.data_ptr(), m, bd.data_ptr())
-    torch.cuda.synchronize()
-    assert np.array_equal(bd.cpu().numpy()[m == 1], ob[m == 1])
-    eng.step2_device(p2, w.data_ptr(), bd.data_ptr(), m, dd.data_ptr())
-    assert abs(psnr(dd.cpu().numpy()) - psnr(od)) <= 0.01
 
 
 @pytest.mark.parametrize("world,H,W", [(2, 200, 72), (3, 330, 64)])
-def test_team_bit_identical_to_single_cluster(oracle, world, H, W):
+def test_team_bit_identical_to_single_cluster(eng, oracle, world, H, W):
     """Emulated teams run the cluster kernel on their row bands; its sums are reduced in a fixed order, so the results are
     bit-identical to one GPU."""
-    import torch
     import lfbm5d_b200 as L
-    from test_team_gpu import run_single, run_team
-    dev = torch.device("cuda", 0)
-    clean = lfdata.synth_lf(3, 3, H, W)
-    noisy = torch.from_numpy(oracle.add_noise(np.ascontiguousarray(clean), 15.0)).to(dev)
-    mask = np.ones(9, np.uint32)
     p1 = L.make_params(15.0, 2.7, 3, 3, 1, W, H, 3, 32, 18, 6, K, 4, L.ID, L.SADCT, L.HAAR)
     p2 = L.make_params(15.0, 0.0, 3, 3, 1, W, H, 3, 32, 18, 6, K, 4, L.DCT, L.SADCT, L.HAAR)
-    e = L.LFBM5D(0)
-    assert e.group_cluster(1, p1)[0] == 2 and e.group_cluster(2, p2)[0] == 4
-    w0, b0, o0, s0 = run_single(L, e, torch, noisy, mask, p1, p2)
-    e.close()
-    ws, bs, outs, bands1, bands2, st = run_team(L, torch, world, noisy, mask, p1, p2, gather=1)
-    assert st["bytes_exchanged"] > 0
-    for g in range(world):
-        assert torch.equal(bs[g], b0) and torch.equal(outs[g], o0) and torch.equal(ws[g], w0)
+    assert eng.group_cluster(1, p1)[0] == 2 and eng.group_cluster(2, p2)[0] == 4
+    assert_team_matches_single(oracle, world, p1, p2)
 
 
 def test_command_line_cluster(tmp_path):
@@ -213,11 +146,7 @@ def test_command_line_cluster(tmp_path):
     dirs = [str(tmp_path / d) for d in ("noisyLF", "basicLF", "denoisedLF", "diffLF")]
     head = [os.path.join(LIBDIR, "LFBM5Ddenoising"), str(src), "SAI", "_", "3", "3", "1", "1", "1", "1", "row", "25", "2.7"] + dirs
     tail = ["8", "18", "6", "16", "4", "id", "sadct", "haar", "0", "16", "18", "6", "16", "4", "dct", "sadct", "haar", "0"]
-    args = head + tail + ["opp", "0", str(tmp_path / "objectiveResults.txt")]
-    env = dict(os.environ, LFBM5D_SEED="20171016")
-    p = subprocess.run(args, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, env=env, timeout=300)
-    out = p.stdout.decode()
-    assert p.returncode == 0, out[-2000:]
+    run_cli(head + tail + ["opp", "0", str(tmp_path / "objectiveResults.txt")])
     src8 = np.clip(np.floor(clean + 0.5), 0, 255).astype(np.float32)
     noisy = L.add_noise(src8, 25.0, seed0=20171016)
     mask = np.ones(9, np.uint32)
@@ -228,7 +157,7 @@ def test_command_line_cluster(tmp_path):
     basic, n1 = e.step1(p1, noisy, mask)
     den, _, _ = e.step2(p2, n1, basic, mask)
     e.close()
-    check_files(tmp_path, (("noisyLF", noisy), ("basicLF", basic), ("denoisedLF", den)), 3)
+    check_pngs(tmp_path, (("noisyLF", noisy), ("basicLF", basic), ("denoisedLF", den)), 3)
 
 
 def test_group_cluster_query(eng):

@@ -6,36 +6,9 @@ import numpy as np
 import pytest
 
 import lfdata
+from gpucheck import run_single, run_team
 
 pytestmark = pytest.mark.gpu
-
-
-def run_single(L, eng, torch, noisy, mask, p1, p2):
-    w, b, o = noisy.clone(), torch.zeros_like(noisy), torch.zeros_like(noisy)
-    eng.step1_device(p1, w.data_ptr(), mask, b.data_ptr())
-    s1 = eng.schedule().copy()
-    eng.step2_device(p2, w.data_ptr(), b.data_ptr(), mask, o.data_ptr())
-    torch.cuda.synchronize()
-    return w, b, o, s1
-
-
-def run_team(L, torch, world, noisy, mask, p1, p2, gather, peer_view=True, lanes=1):
-    team = L.Team.emulated(0, world)
-    if lanes > 1:
-        team.set_lanes(lanes)
-    if not peer_view:
-        team.disable_peer_view()
-    ws = [noisy.clone() for _ in range(world)]
-    bs = [torch.zeros_like(noisy) for _ in range(world)]
-    outs = [torch.zeros_like(noisy) for _ in range(world)]
-    team.step(1, p1, [t.data_ptr() for t in ws], None, mask, [t.data_ptr() for t in bs], gather=gather)
-    bands1 = [team.band(g) for g in range(world)]
-    team.step(2, p2, [t.data_ptr() for t in ws], [t.data_ptr() for t in bs], mask, [t.data_ptr() for t in outs], gather=gather)
-    bands2 = [team.band(g) for g in range(world)]
-    torch.cuda.synchronize()
-    st = team.stats()
-    team.close()
-    return ws, bs, outs, bands1, bands2, st
 
 
 @pytest.mark.parametrize("world,aw,ah,H,W,C,masked", [(2, 3, 3, 200, 72, 3, False), (3, 4, 3, 330, 64, 3, True), (4, 3, 3, 340, 56, 3, False),

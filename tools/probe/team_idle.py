@@ -7,7 +7,7 @@ sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import torch
 import lfbm5d_b200 as L
 import lfdata
-import test_team_gpu as T
+import gpucheck as T
 
 dev = torch.device("cuda", 0)
 def psnr(a, b): return float(10 * torch.log10(255.0 ** 2 / torch.mean((a - b) ** 2)))
