@@ -106,6 +106,10 @@ void lfbm5d_set_max_passes(lfbm5d_ctx *ctx, unsigned max_passes);
  * 3x3 windows over the opt-in shared memory of one CTA), with *max_active_clusters = cudaOccupancyMaxActiveClusters of that
  * configuration (0 for cluster_size 1). Fails, naming the cluster size and the bytes per CTA, if the device cannot run it. */
 int lfbm5d_group_cluster(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, int *cluster_size, int *max_active_clusters);
+/* Debug: the name of the group kernel a window pass of `step` launches with these parameters on the context's device, as
+ * "k_groups<2,3>", "k_groups_w8<1>", "k_groups_cl<2,4>", ..., written NUL-terminated into name[cap] (truncated to fit).
+ * Fails like lfbm5d_group_cluster on parameters the library rejects. */
+int lfbm5d_group_kernel(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, char *name, unsigned cap);
 
 /* ---- static window schedule ----------------------------------------------------------------------
  * The angular windows of a step (bm5d.cpp:171-402) in the order of the reference's schedule; windows that share no SAI commute.

@@ -1003,10 +1003,69 @@ int group_cluster(lfbm5d_ctx *ctx, int step, unsigned k, unsigned asw, unsigned 
     return 0;
 }
 
+// The group kernel a pass runs, chosen from (step, k, asw, N, C, tau_2D, tau_5D, useSD), with its launch shape. Exactly one of
+// fn / fn_nz / fn25 is set: fn_nz kernels take the zero-block marker as a second argument. cl > 1: a cluster of cl CTAs per group.
+struct GroupKernel {
+    const char *name = nullptr;
+    void (*fn)(GroupArgs) = nullptr;                                  // k_groups, k_groups12, k_groups_cl
+    void (*fn_nz)(GroupArgs, unsigned long long) = nullptr;           // k_groups_id16, k_groups_w8
+    void (*fn25)(GroupArgs25) = nullptr;                              // k_groups25
+    int threads = 256, cl = 1;
+    size_t smem = 0;                                                  // dynamic shared memory per CTA
+    const void *func() const { return fn ? (const void *) fn : fn_nz ? (const void *) fn_nz : (const void *) fn25; }
+};
+int group_kernel(lfbm5d_ctx *ctx, int step, unsigned k, unsigned asw, unsigned N, unsigned C, unsigned tau_2D, unsigned tau_5D,
+                 unsigned useSD, GroupKernel &gk)
+{
+    gk = GroupKernel{};
+    gk.smem = group_smem(step, k, asw, N, tau_2D);
+    const bool s1 = step == 1, c3 = C == 3;        // validate(): C is 1 or 3
+    if (asw == G25_SW) {
+        // 5x5 windows: dense swizzled patches (no row padding), one CTA of 512 threads per SM; validate() bounds the group
+        gk.fn25 = s1 ? k_groups25<1> : k_groups25<2>;
+        gk.name = s1 ? "k_groups25<1>" : "k_groups25<2>";
+        gk.threads = G25_NT;
+        return 0;
+    }
+    if (k == 12) {         // 288 threads (2 patches x 144 positions); validate() bounds the group's shared memory
+        gk.fn = s1 ? (asw == 3 ? k_groups12<1, 3> : k_groups12<1, 1>) : (asw == 3 ? k_groups12<2, 3> : k_groups12<2, 1>);
+        gk.name = s1 ? (asw == 3 ? "k_groups12<1,3>" : "k_groups12<1,1>") : (asw == 3 ? "k_groups12<2,3>" : "k_groups12<2,1>");
+        gk.threads = LF_G12_NT;
+        return 0;
+    }
+    GroupCluster gc;
+    if (group_cluster(ctx, step, k, asw, N, tau_2D, gc)) return 1;
+    if (gc.cl > 1) {       // distributed over a cluster: CTA blockIdx.x % cl of the cluster of reference patch blockIdx.x / cl + r0
+        gk.fn = gc.fn; gk.cl = gc.cl; gk.smem = gc.smem;
+        gk.name = s1 ? (gc.cl == 2 ? "k_groups_cl<1,2>" : "k_groups_cl<1,4>") : (gc.cl == 2 ? "k_groups_cl<2,2>" : "k_groups_cl<2,4>");
+        return 0;
+    }
+    if (s1 && tau_2D == LFBM5D_ID && k == 16 && asw == 3 && N <= 8 && tau_5D != LFBM5D_DCT && !useSD) {
+        // register-resident path (no 2-D transform to stage); patches that contribute zeros read the zero block behind nsym
+        gk.fn_nz = c3 ? k_groups_id16<3> : k_groups_id16<1>;
+        gk.name = c3 ? "k_groups_id16<3>" : "k_groups_id16<1>";
+        gk.smem = 0;
+        return 0;
+    }
+    if (!s1 && tau_2D == LFBM5D_DCT && k == 8 && asw == 3 && N <= 16 && tau_5D == LFBM5D_HAAR && !useSD) {
+        // packed X/E path: FP32x2 forward transforms, two rows per lane in the inverses
+        gk.fn_nz = c3 ? k_groups_w8<3> : k_groups_w8<1>;
+        gk.name = c3 ? "k_groups_w8<3>" : "k_groups_w8<1>";
+        gk.threads = W8_NT;
+        gk.smem = (size_t) 16 * 9 * W8_PS * 8;
+        return 0;
+    }
+    gk.fn = s1 ? (asw == 3 ? k_groups<1, 3> : k_groups<1, 1>) : (asw == 3 ? k_groups<2, 3> : k_groups<2, 1>);
+    gk.name = s1 ? (asw == 3 ? "k_groups<1,3>" : "k_groups<1,1>") : (asw == 3 ? "k_groups<2,3>" : "k_groups<2,1>");
+    return 0;
+}
+
 // Group kernel for the reference patches [r0, r1) (gather, transforms, shrinkage, inverses, staging for the aggregation)
 int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int pst, bool partial, int r0, int r1)
 {
     if (r1 <= r0) return 0;
+    GroupKernel gk;
+    if (group_kernel(ctx, pc.step, pc.k, pc.asw, pc.N, pc.C, pc.tau_2D, pc.tau_5D, pc.useSD, gk)) return 1;
     const PassGeom pg = pass_geom(pc);
     const int R = pg.R;
     GroupArgsBase gb{};
@@ -1016,7 +1075,6 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     gb.pst = pst; gb.nc = pg.nc; gb.r0 = r0;
     gb.RS = group_rs(pc.k, pc.asw, pc.tau_2D);
     gb.PS = pc.k * gb.RS;
-    const size_t smem = group_smem(pc.step, pc.k, pc.asw, pc.N, pc.tau_2D);
     gb.tau_2D = pc.tau_2D; gb.tau_4D = pc.tau_4D; gb.tau_5D = pc.tau_5D;
     gb.rows = ctx->rows.as<int>(); gb.cols = ctx->cols.as<int>();
     gb.bm_count = ctx->bmcount.as<unsigned>(); gb.bm_idx = ctx->bmidx.as<unsigned>();
@@ -1025,55 +1083,21 @@ int launch_groups(lfbm5d_ctx *ctx, const PassCfg &pc, const LfWindow &win, int p
     gb.numsym = ctx->numsym.as<float>(); gb.densym = ctx->densym.as<float>();
     gb.zbuf = ctx->zbuf.as<float>(); gb.wbuf = ctx->wbuf.as<float>(); gb.ent = ctx->spos.as<unsigned>(); gb.R = R;
     const int nblk = r1 - r0;
-    if (pc.asw == G25_SW) {
-        // 5x5 windows: dense swizzled patches (no row padding), one CTA of 512 threads per SM; validate() bounds the group
+    if (gk.smem) CK(cudaFuncSetAttribute(gk.func(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int) gk.smem));
+    if (gk.fn25) {
         GroupArgs25 g25{};
         static_cast<GroupArgsBase &>(g25) = gb;
         g25.win = win;
         g25.gmask32 = ctx->gmask.as<unsigned>();
-        void (*k25)(GroupArgs25) = pc.step == 1 ? k_groups25<1> : k_groups25<2>;
-        CK(cudaFuncSetAttribute((const void *) k25, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        k25<<<nblk, G25_NT, smem, ctx->stream>>>(g25);
-        ctx->stats.kernel_launches++;
-        return 0;
+        gk.fn25<<<nblk, gk.threads, gk.smem, ctx->stream>>>(g25);
+    } else {
+        GroupArgs ga{};
+        static_cast<GroupArgsBase &>(ga) = gb;
+        for (int a = 0; a < LF_LUTA; a++) { ga.win.st[a] = win.st[a]; ga.win.mask[a] = win.mask[a]; ga.win.proc[a] = win.proc[a]; }
+        ga.win.A = win.A;
+        if (gk.fn_nz) gk.fn_nz<<<nblk, gk.threads, gk.smem, ctx->stream>>>(ga, 0x8000000080000000ull);
+        else gk.fn<<<nblk * gk.cl, gk.threads, gk.smem, ctx->stream>>>(ga);
     }
-    GroupArgs ga{};
-    static_cast<GroupArgsBase &>(ga) = gb;
-    for (int a = 0; a < LF_LUTA; a++) { ga.win.st[a] = win.st[a]; ga.win.mask[a] = win.mask[a]; ga.win.proc[a] = win.proc[a]; }
-    ga.win.A = win.A;
-    void (*kfn)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups<1, 3> : k_groups<1, 1>)
-                                          : (pc.asw == 3 ? k_groups<2, 3> : k_groups<2, 1>);
-    if (pc.k == 12) {      // 288 threads (2 patches x 144 positions); validate() bounds the group's shared memory
-        void (*k12)(GroupArgs) = pc.step == 1 ? (pc.asw == 3 ? k_groups12<1, 3> : k_groups12<1, 1>)
-                                              : (pc.asw == 3 ? k_groups12<2, 3> : k_groups12<2, 1>);
-        CK(cudaFuncSetAttribute((const void *) k12, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        k12<<<nblk, LF_G12_NT, smem, ctx->stream>>>(ga);
-        ctx->stats.kernel_launches++;
-        return 0;
-    }
-    GroupCluster gc;
-    if (group_cluster(ctx, pc.step, pc.k, pc.asw, pc.N, pc.tau_2D, gc)) return 1;
-    if (gc.cl > 1) {       // distributed over a cluster: CTA blockIdx.x % cl of the cluster of reference patch blockIdx.x / cl + r0
-        CK(cudaFuncSetAttribute((const void *) gc.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) gc.smem));
-        gc.fn<<<nblk * gc.cl, 256, gc.smem, ctx->stream>>>(ga);
-        ctx->stats.kernel_launches++;
-        return 0;
-    }
-    CK(cudaFuncSetAttribute((const void *) kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-    if (pc.step == 1 && pc.tau_2D == LFBM5D_ID && pc.k == 16 && pc.asw == 3 && pc.N <= 8 && pc.tau_5D != LFBM5D_DCT && !pc.useSD) {
-        // register-resident path (no 2-D transform to stage); patches that contribute zeros read the zero block behind nsym
-        if (pc.C == 3) k_groups_id16<3><<<nblk, 256, 0, ctx->stream>>>(ga, 0x8000000080000000ull);
-        else k_groups_id16<1><<<nblk, 256, 0, ctx->stream>>>(ga, 0x8000000080000000ull);       // validate(): C is 1 or 3
-    }
-    else if (pc.step == 2 && pc.tau_2D == LFBM5D_DCT && pc.k == 8 && pc.asw == 3 && pc.N <= 16 && pc.tau_5D == LFBM5D_HAAR && !pc.useSD) {
-        // packed X/E path: FP32x2 forward transforms, two rows per lane in the inverses
-        void (*k8)(GroupArgs, unsigned long long) = pc.C == 3 ? k_groups_w8<3> : k_groups_w8<1>;       // validate(): C is 1 or 3
-        const size_t smem8 = (size_t) 16 * 9 * W8_PS * 8;
-        CK(cudaFuncSetAttribute((const void *) k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem8));
-        k8<<<nblk, W8_NT, smem8, ctx->stream>>>(ga, 0x8000000080000000ull);
-    }
-    else
-        kfn<<<nblk, 256, smem, ctx->stream>>>(ga);
     ctx->stats.kernel_launches++;
     return 0;
 }
@@ -1581,6 +1605,18 @@ int lfbm5d_group_cluster(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, int 
     if (group_cluster(ctx, step, p->k, 2 * p->an + 1, p->N, p->tau_2D, gc)) return 1;
     *cluster_size = gc.cl;
     *max_active_clusters = gc.max_active;
+    return 0;
+}
+
+int lfbm5d_group_kernel(lfbm5d_ctx *ctx, int step, const lfbm5d_params *p, char *name, unsigned cap)
+{
+    if (!ctx || !name || cap == 0) return fail("null argument");
+    if (step != 1 && step != 2) return fail("step must be 1 or 2");
+    if (validate(p, step)) return 1;
+    CK(cudaSetDevice(ctx->device));
+    GroupKernel gk;
+    if (group_kernel(ctx, step, p->k, 2 * p->an + 1, p->N, p->chnls, p->tau_2D, p->tau_5D, p->useSD ? 1 : 0, gk)) return 1;
+    snprintf(name, cap, "%s", gk.name);
     return 0;
 }
 

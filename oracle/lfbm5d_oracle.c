@@ -21,9 +21,11 @@
 
 static int g_dct_mode = 0;
 static int g_use_sd = 0;    /* useSD of the next orc_pass / orc_run_* calls (test infrastructure; see orc_set_use_sd) */
+static int g_sum_mode = 0;  /* 1: group weight sums in double (test infrastructure; see orc_set_sum_mode) */
 static int g_bm3d = 0;      /* set while orc_run_bm3d_LF drives orc_pass: BM3D thresholds (bm3d.cpp:340, :532, :940) */
 static int g_threads = 0;
 void orc_set_dct_mode(int mode) { g_dct_mode = mode; }
+void orc_set_sum_mode(int mode) { g_sum_mode = mode; }
 void orc_set_threads(int n) { g_threads = n; }
 static int nthreads(void)
 {
@@ -1001,6 +1003,7 @@ static void process_group(const pass_ctx *cx, int step, const float *noisy, cons
 
     /* 5th dimension: per pq, vectors along n for each (c, st); core:2281-2505 / :2706-2925 */
     float wt[3] = { 0.0f, 0.0f, 0.0f };
+    double wtd[3] = { 0.0, 0.0, 0.0 };           /* step-2 weight sums of sum mode 1 */
     float vo[64], ve[64];
     const float hcoef = 1.0f / (float) nSx;
     float cn5[64], cni5[64];                     /* preProcess_5d, core:3262-3276 */
@@ -1057,7 +1060,7 @@ static void process_group(const pass_ctx *cx, int step, const float *noisy, cons
                             value /= (value + sg * sg);
                             *e = (*g) * value * hcoef;
                         }
-                        wt[c] += value;
+                        if (g_sum_mode) wtd[c] += value; else wt[c] += value;
                     }
                 }
             }
@@ -1082,6 +1085,8 @@ static void process_group(const pass_ctx *cx, int step, const float *noisy, cons
                 }
             }
     }
+    if (g_sum_mode && step == 2)                 /* rounded to float once; the weight below is the same float expression */
+        for (unsigned c = 0; c < C; c++) wt[c] = (float) wtd[c];
     for (unsigned c = 0; c < C; c++) {
         const float sg = cx->sigma_table[c];
         go->w[c] = wt[c] > 0.0f ? (sg > 0.0 ? 1.0f / (float) (sg * sg * wt[c]) : 1.0f / (float) (wt[c])) : 1.0f;
@@ -1092,13 +1097,15 @@ static void process_group(const pass_ctx *cx, int step, const float *noisy, cons
         for (unsigned c = 0; c < C; c++) {
             const unsigned cc = g_bm3d ? 0 : c;
             float mean = 0.0f, std = 0.0f;
+            double meand = 0.0, stdd = 0.0;      /* sum mode 1 */
             for (unsigned pq = 0; pq < k2; pq++)
                 for (unsigned st = 0; st < A; st++)
                     for (unsigned n = 0; n < nSx; n++) {
                         const float x = X[((size_t) (n * C + cc) * k2 + pq) * A + st];
-                        mean += x;
-                        std += x * x;
+                        if (g_sum_mode) { meand += x; stdd += x * x; }
+                        else { mean += x; std += x * x; }
                     }
+            if (g_sum_mode) { mean = (float) meand; std = (float) stdd; }
             const float res = (std - mean * mean / (float) Nn) / (float) (Nn - 1);
             go->w[c] = res > 0.0f ? 1.0f / sqrtf(res) : 0.0f;
         }

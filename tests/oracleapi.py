@@ -1,4 +1,5 @@
 """ctypes bindings for oracle/liblfbm5d_oracle.so (CPU restatement). TEST INFRASTRUCTURE ONLY."""
+import contextlib
 import ctypes as C
 import os
 import subprocess
@@ -44,6 +45,17 @@ def u32(a):
 
 def set_dct_mode(m):
     lib().orc_set_dct_mode(int(m))
+
+
+@contextlib.contextmanager
+def sum_mode(m):
+    """Runs the block with orc_set_sum_mode(m) (1: the group's Wiener weight and useSD sums added in double and rounded to
+    float once, 0: term by term in float as the reference does) and restores mode 0 however it ends."""
+    lib().orc_set_sum_mode(int(m))
+    try:
+        yield
+    finally:
+        lib().orc_set_sum_mode(0)
 
 
 def add_noise(clean, sigma, seed0=20171016):

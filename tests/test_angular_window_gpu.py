@@ -18,6 +18,9 @@ pytestmark = pytest.mark.gpu
 
 
 def test_an2_single_passes(eng, oracle):
+    import lfbm5d_b200 as L
+    prm = L.make_params(25.0, 0.0, 5, 5, 2, 48, 40, 3, 16, 18, 6, 8, 4, L.DCT, L.SADCT, L.HAAR)
+    assert eng.group_kernel(1, prm) == "k_groups25<1>" and eng.group_kernel(2, prm) == "k_groups25<2>"
     sym = pad_inputs5(oracle, 40, 48, 25.0)
     z = np.zeros_like(sym)
     mask, proc = np.ones(25, np.uint32), np.zeros(25, np.uint32)

@@ -2,7 +2,7 @@
 clusters of 2 or 4 CTAs that share the group through distributed shared memory (k_groups_cl). GPU against the CPU oracle through
 the C ABI. The oracle is generic in N but pinned against the reference only at the N values of the other tests, so these results
 are checked GPU vs oracle: match lists, disparity argmin and shape flags bit-exact; step 1 accumulators and LF_basic bit-identical;
-complete runs within 0.01 dB; step 2 within the rounding bound of the oracle's group sums (gpucheck.wiener_tol)."""
+complete runs within 0.01 dB; step 2 within STEP2_REL (STEP2_REL_SD with useSD) of the exact-sum oracle, as on one CTA."""
 import os
 
 import numpy as np
@@ -11,7 +11,7 @@ import pytest
 import golden_inputs as gi
 import lfdata
 from gpucheck import (LIBDIR, assert_team_matches_single, check_complete_run, check_pass, check_pngs, eng, estimate, psnr_on,
-                      run_cli, wiener_tol, write_lf)  # noqa: F401 (eng is the engine fixture)
+                      run_cli, spread_inputs, write_lf)  # noqa: F401 (eng is the engine fixture)
 
 pytestmark = pytest.mark.gpu
 K = 16
@@ -22,25 +22,16 @@ def expected_cluster(step, N):
     return {(1, 32): 2, (2, 16): 2, (2, 32): 4}[(step, N)]
 
 
-def spread_inputs(H=40, W=48):
-    """Noisy padded SAIs with a flat region (every candidate matches, with exact distance ties: groups of N patches) and a region
-    of strong noise (only the reference patch matches: the duplicated single match, groups of 2 patches)."""
-    _, _, sym = gi.pad_inputs(H, W, 25.0)
-    rng = np.random.default_rng(7)
-    sym[:, :, 24:44, 24:56] = 100.0
-    sym[:, :, 44:64, 40:72] += rng.normal(0.0, 120.0, (9, 3, 20, 32)).astype(np.float32)
-    return sym
-
-
 def check_pass_cl(eng, oracle, step, sym, basic, num0, den0, mask, proc, N, t2, t4, t5, lam=2.7, useSD=0, pst=4, cst=None, spread=False):
-    """check_pass at k = 16 on the cluster size the group needs, step 2 and useSD within wiener_tol."""
+    """check_pass at k = 16 on the cluster size the group needs, and on k_groups_cl of that size."""
     import lfbm5d_b200 as L
     A, C, hb, wb = sym.shape
     prm = L.make_params(25.0, lam, 3, 3, 1, wb - 48, hb - 48, C, N, 18, 6, K, 4, t2, t4, t5, useSD=int(useSD))
     cl, occ = eng.group_cluster(step, prm)
     assert cl == expected_cluster(step, N) and occ > 0, (cl, occ)
+    assert eng.group_kernel(step, prm) == "k_groups_cl<%d,%d>" % (step, cl)
     on, od, gn, gd, gdbg = check_pass(eng, oracle, step, sym, basic, num0, den0, mask, proc, K, N, t2, t4, t5, pst=pst, cst=cst, lam=lam,
-                                      useSD=useSD, rel=wiener_tol(N, useSD), est=False)
+                                      useSD=useSD)
     if spread:
         # every CTA of the cluster holds patches (nSx = N), and the CTAs hold one patch each or, on 4-CTA clusters, two of them
         # hold none (nSx = 2, the smallest group: a single match is duplicated)

@@ -31,11 +31,14 @@ def test_block_matching_k12(eng, oracle, nDisp):
 
 def test_single_passes_k12(eng, oracle):
     """Every 2-D / angular / 1-D transform combination at k = 12, both steps, and a second pass on top of the first's accumulators."""
+    import lfbm5d_b200 as L
     _, _, sym = gi.pad_inputs(40, 48, 25.0)
     z = np.zeros_like(sym)
     mask, proc = np.ones(9, np.uint32), np.zeros(9, np.uint32)
     on, od, _, _, _ = check_pass(eng, oracle, 1, sym, None, z, z, mask, proc, K, 16, oracle.ID, oracle.SADCT, oracle.HAAR)
     basic = estimate(on, od, sym)
+    prm = L.make_params(25.0, 0.0, 3, 3, 1, 48, 40, 3, 16, 18, 6, K, 4, L.DCT, L.SADCT, L.HAAR)
+    assert eng.group_kernel(1, prm) == "k_groups12<1,3>" and eng.group_kernel(2, prm) == "k_groups12<2,3>"
     for t2 in (oracle.ID, oracle.DCT):
         for t4 in (oracle.DCT, oracle.SADCT, oracle.ID):
             for t5 in (oracle.HAAR, oracle.HADAMARD, oracle.DCT):
@@ -106,7 +109,8 @@ def test_lfbm3d_k12(eng, oracle):
     noisy = oracle.add_noise(clean, 10.0)
     mask = np.ones(4, np.uint32)
     mask[3] = 0
-    ob, od, on = oracle.run_bm3d_lf(noisy, mask, 10.0, 16, 16, K, K, 16, 32, 3, 3, L.DCT, L.DCT, 2.7)
+    with oracle.sum_mode(1):
+        ob, od, on = oracle.run_bm3d_lf(noisy, mask, 10.0, 16, 16, K, K, 16, 32, 3, 3, L.DCT, L.DCT, 2.7)
     prm = L.make_params3d(10.0, 4, 48, 40, 3, 16, 16, K, K, 16, 32, 3, 3, L.DCT, L.DCT, 2.7)
     gb, gd, gn = eng.bm3d(prm, noisy, mask)
     assert np.array_equal(gn, on)
