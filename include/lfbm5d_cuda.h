@@ -99,6 +99,18 @@ int lfbm5d_step2_device(lfbm5d_ctx *ctx, const lfbm5d_params *p, float *d_noisy_
                         const unsigned *sai_mask, float *d_denoised_out);
 int lfbm3d_run_device(lfbm5d_ctx *ctx, const lfbm3d_params *p, float *d_noisy_io, const unsigned *sai_mask, float *d_basic_out,
                       float *d_denoised_out);
+/* ---- noise level of a light field without ground truth (an extension; the reference has no estimator) ----------------------
+ * Donoho's estimator on the input as given (RGB or grey, before any colour transform): for every non-masked SAI, channel and 2 x 2
+ * block at (2i, 2j), i < height/2, j < width/2 (an odd last row / column is dropped), the key |((x00 - x01) - (x10 - x11)) * 0.5f|
+ * (float, no contraction); sigma = (lower median of the keys, rank (n - 1) / 2) / 0.6744897501960817f. *sigma pools all keys;
+ * sigma_chnl[chnls] (may be NULL) takes the keys of each channel, sigma_sai[asize] (may be NULL) those of each SAI (masked SAIs: 0).
+ * Integer-valued input (8-bit PNGs) gives keys that are multiples of 0.5, so sigma is then a multiple of 0.7413. The input is not
+ * modified. Fails (before any launch) on chnls other than 1 or 3, width or height < 2, asize 0, or every SAI masked.
+ * lfbm5d_estimate_sigma: noisy[st] host arrays as for lfbm5d_step1; _device: d_noisy is [asize][chnls][height][width] on the device. */
+int lfbm5d_estimate_sigma(lfbm5d_ctx *ctx, float *const *noisy, const unsigned *sai_mask, unsigned asize, unsigned chnls, unsigned width,
+                          unsigned height, float *sigma, float *sigma_chnl, float *sigma_sai);
+int lfbm5d_estimate_sigma_device(lfbm5d_ctx *ctx, const float *d_noisy, const unsigned *sai_mask, unsigned asize, unsigned chnls, unsigned width,
+                                 unsigned height, float *sigma, float *sigma_chnl, float *sigma_sai);
 /* stop after this many window passes per step (0 = run to completion); for bounded measurements only */
 void lfbm5d_set_max_passes(lfbm5d_ctx *ctx, unsigned max_passes);
 /* How the group kernel of `step` runs with these parameters on the context's device: *cluster_size = 1 when one CTA holds a

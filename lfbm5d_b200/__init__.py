@@ -46,7 +46,8 @@ EXPORTS = ["lfbm5d_create", "lfbm5d_destroy", "lfbm5d_last_error", "lfbm5d_reset
            "lfbm5d_step2_device", "lfbm3d_run_device", "lfbm5d_set_max_passes", "lfbm5d_group_cluster", "lfbm5d_group_kernel", "lfbm5d_debug_pass", "lfbm5d_debug_pass_ex",
            "lfbm5d_debug_schedule", "lfbm5d_step_plan", "lfbm5d_debug_block_matching", "lfbm5d_team_create_emulated", "lfbm5d_team_unique_id",
            "lfbm5d_team_create_nccl", "lfbm5d_team_destroy", "lfbm5d_team_local_ranks", "lfbm5d_team_step", "lfbm5d_team_band",
-           "lfbm5d_team_stats", "lfbm5d_team_disable_peer_view", "lfbm5d_team_timing", "lfbm5d_team_plan_band", "lfbm5d_copy_rows", "lfbm5d_sync", "lfbm5d_team_use_peer_exchange", "lfbm5d_team_set_lanes", "lfbm5d_team_launches"]
+           "lfbm5d_team_stats", "lfbm5d_team_disable_peer_view", "lfbm5d_team_timing", "lfbm5d_team_plan_band", "lfbm5d_copy_rows", "lfbm5d_sync", "lfbm5d_team_use_peer_exchange", "lfbm5d_team_set_lanes", "lfbm5d_team_launches",
+           "lfbm5d_estimate_sigma", "lfbm5d_estimate_sigma_device"]
 
 HOST_LIB_PATH = os.path.join(_HERE, "_lib", "liblfbm5d_host.so")
 HOST_EXPORTS = ["lfio_add_noise", "lfio_psnr", "lfio_png_read", "lfio_png_write", "lfio_psnr_LF", "lfio_diff_LF", "lfio_write_psnr_LF", "lfio_load_LF", "lfio_save_LF"]      # include/lfbm5d_host_c.h
@@ -237,6 +238,37 @@ class LFBM5D(object):
         m = np.ascontiguousarray(mask, np.uint32)
         if self.lib.lfbm3d_run_device(self.ctx, C.byref(prm3), C.c_void_p(d_noisy), _up(m), C.c_void_p(d_basic), C.c_void_p(d_out)) != 0:
             raise RuntimeError("lfbm3d_run_device: " + self.error())
+
+    def estimate_sigma(self, noisy, mask):
+        """Noise level of a light field without ground truth (lfbm5d_estimate_sigma): noisy [asize, C, H, W] as given (RGB or grey)
+        -> (sigma pooled over all SAIs and channels, sigma per channel [C], sigma per SAI [asize], 0 for masked SAIs). The pooled
+        value is the one to denoise with; the per-SAI values show whether one sigma fits the light field."""
+        n = np.ascontiguousarray(noisy, np.float32)
+        if n.ndim != 4:
+            raise ValueError("noisy must be [asize, C, H, W]")
+        asize, chnls, h, w = n.shape
+        m = self._mask(mask, asize)
+        sig, sc, ss = C.c_float(), np.zeros(chnls, np.float32), np.zeros(asize, np.float32)
+        if self.lib.lfbm5d_estimate_sigma(self.ctx, self._ptrs(n), _up(m), asize, chnls, w, h, C.byref(sig), _fp(sc), _fp(ss)) != 0:
+            raise RuntimeError("lfbm5d_estimate_sigma: " + self.error())
+        return sig.value, sc, ss
+
+    def estimate_sigma_device(self, d_lf, mask, asize, chnls, width, height):
+        """estimate_sigma of a device light field [asize][chnls][height][width] (raw pointer, e.g. a torch tensor's data_ptr()),
+        on the engine's stream; returns when the result is on the host."""
+        m = self._mask(mask, asize)
+        sig, sc, ss = C.c_float(), np.zeros(max(int(chnls), 1), np.float32), np.zeros(max(int(asize), 1), np.float32)
+        if self.lib.lfbm5d_estimate_sigma_device(self.ctx, C.c_void_p(d_lf), _up(m), int(asize), int(chnls), int(width), int(height),
+                                                 C.byref(sig), _fp(sc), _fp(ss)) != 0:
+            raise RuntimeError("lfbm5d_estimate_sigma_device: " + self.error())
+        return sig.value, sc[:chnls], ss[:asize]
+
+    @staticmethod
+    def _mask(mask, asize):
+        m = np.ascontiguousarray(mask, np.uint32)
+        if m.shape != (int(asize),):
+            raise ValueError("mask must hold one entry per SAI")
+        return m
 
     # -- device-resident entry points (raw device pointers, e.g. torch tensors' data_ptr()) -------
     def step1_device(self, prm, d_noisy, mask, d_basic):

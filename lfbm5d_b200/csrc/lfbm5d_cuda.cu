@@ -8,6 +8,7 @@
 #include "groups.cuh"
 #include "groups_wiener8.cuh"
 #include "groups25.cuh"
+#include "noise_estimate.cuh"
 
 #include <cmath>
 #include <cstdio>
@@ -353,6 +354,7 @@ struct lfbm5d_ctx {
     DevBuf nsym, bsym, numsym, densym, est0;
     DevBuf s_at, s_mir, sums, first, shape, bmcount, bmidx, bnd, progress, rowmap, colmap, rows, cols, counters,
            zbuf, wbuf, spos, arange, brange, gmask, shape_lut, tielist, stielist, act, rt_noisy, rt_basic, frow, fcol;
+    DevBuf nehist, neseg;          // noise estimate: 64-bit histograms and selection state per segment (noise_estimate.cuh)
     unsigned lut_asw = 0;
     lfbm5d_stats stats{};
     bool timing = false;
@@ -1533,6 +1535,50 @@ int download_lf(lfbm5d_ctx *ctx, const DevBuf &buf, float *const *host, const un
     return 0;
 }
 
+// lfbm5d_estimate_sigma: arguments checked before anything is uploaded or launched
+int validate_estimate(const void *lf, const unsigned *mask, unsigned asize, unsigned chnls, unsigned width, unsigned height,
+                      const float *sigma)
+{
+    if (chnls != 1 && chnls != 3) return fail("chnls must be 1 or 3");
+    if (width < 2 || height < 2) return fail("the noise estimate needs SAIs of at least 2 x 2 pixels");
+    if (asize == 0) return fail("empty light field (asize = 0)");
+    if (!lf || !mask || !sigma) return fail("null argument");
+    for (unsigned st = 0; st < asize; st++) if (mask[st]) return 0;
+    return fail("every SAI is masked: nothing to estimate the noise from");
+}
+
+// Noise estimate of the device light field d_lf [asize][chnls][height][width] (noise_estimate.cuh): three histogram passes, each
+// followed by the selection of one digit per segment, then the 1 + chnls + asize medians come back to the host.
+int noise_estimate(lfbm5d_ctx *ctx, const float *d_lf, const unsigned *mask, unsigned asize, unsigned chnls, unsigned width, unsigned height,
+                   float *sigma, float *sigma_chnl, float *sigma_sai)
+{
+    const unsigned nseg = 1 + chnls + asize, W2 = width / 2, H2 = height / 2;
+    if (ctx->nehist.ensure((size_t) nseg * NE_BINS * 8) || ctx->neseg.ensure(nseg * sizeof(NeSeg)) || ctx->mask.ensure(asize * 4)) return 1;
+    CK(cudaMemcpyAsync(ctx->mask.p, mask, asize * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(ctx->nehist.p, 0, (size_t) nseg * NE_BINS * 8, ctx->stream));     // k_ne_select clears what it has read
+    const unsigned rows = std::max(1u, NE_TILE_KEYS / W2);
+    const dim3 grid((H2 + rows - 1) / rows, chnls, asize);
+    for (int pass = 0; pass < 3; pass++) {
+        LAUNCH(ctx, k_ne_hist, grid, NE_THREADS, 0, d_lf, ctx->mask.as<unsigned>(), (int) width, (int) height, (int) rows, pass,
+               ctx->neseg.as<NeSeg>(), ctx->nehist.as<unsigned long long>());
+        LAUNCH(ctx, k_ne_select, nseg, NE_THREADS, 0, ctx->nehist.as<unsigned long long>(), ctx->neseg.as<NeSeg>(), pass);
+    }
+    CK(cudaGetLastError());
+    std::vector<NeSeg> seg(nseg);
+    CK(cudaMemcpyAsync(seg.data(), ctx->neseg.p, nseg * sizeof(NeSeg), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    auto value = [&](unsigned s) {
+        if (seg[s].empty) return 0.0f;
+        float m;
+        memcpy(&m, &seg[s].prefix, 4);
+        return m / NE_SIGMA_DIV;      // one IEEE float division (no fast-math in this build)
+    };
+    *sigma = value(0);
+    for (unsigned c = 0; c < chnls && sigma_chnl; c++) sigma_chnl[c] = value(1 + c);
+    for (unsigned st = 0; st < asize && sigma_sai; st++) sigma_sai[st] = value(1 + chnls + st);
+    return 0;
+}
+
 } // namespace
 
 extern "C" {
@@ -1573,7 +1619,8 @@ void lfbm5d_destroy(lfbm5d_ctx *ctx)
     DevBuf *all[] = { &ctx->noisy, &ctx->basic, &ctx->out, &ctx->num, &ctx->den, &ctx->mask, &ctx->nsym, &ctx->bsym, &ctx->numsym,
                       &ctx->densym, &ctx->est0, &ctx->s_at, &ctx->s_mir, &ctx->sums, &ctx->first, &ctx->shape, &ctx->bmcount,
                       &ctx->bmidx, &ctx->bnd, &ctx->progress, &ctx->rowmap, &ctx->colmap, &ctx->rows, &ctx->cols, &ctx->counters,
-                      &ctx->zbuf, &ctx->wbuf, &ctx->spos, &ctx->arange, &ctx->brange, &ctx->gmask, &ctx->shape_lut, &ctx->tielist, &ctx->stielist, &ctx->act, &ctx->rt_noisy, &ctx->rt_basic, &ctx->frow, &ctx->fcol };
+                      &ctx->zbuf, &ctx->wbuf, &ctx->spos, &ctx->arange, &ctx->brange, &ctx->gmask, &ctx->shape_lut, &ctx->tielist, &ctx->stielist, &ctx->act, &ctx->rt_noisy, &ctx->rt_basic, &ctx->frow, &ctx->fcol,
+                      &ctx->nehist, &ctx->neseg };
     for (auto b : all) b->release();
     for (auto &e : ctx->sat_cache) { e->d_planes.release(); e->d_groups.release(); }
     for (auto &ev : ctx->ev) if (ev) cudaEventDestroy(ev);
@@ -1739,6 +1786,26 @@ int lfbm3d_run_device(lfbm5d_ctx *ctx, const lfbm3d_params *p, float *d_noisy_io
 {
     if (!ctx || !d_noisy_io || !sai_mask || !d_basic_out || !d_denoised_out) return fail("null argument");
     return bm3d_device(ctx, p, d_noisy_io, sai_mask, d_basic_out, d_denoised_out);
+}
+
+int lfbm5d_estimate_sigma(lfbm5d_ctx *ctx, float *const *noisy, const unsigned *sai_mask, unsigned asize, unsigned chnls, unsigned width,
+                          unsigned height, float *sigma, float *sigma_chnl, float *sigma_sai)
+{
+    if (!ctx) return fail("null argument");
+    if (validate_estimate(noisy, sai_mask, asize, chnls, width, height, sigma)) return 1;
+    CK(cudaSetDevice(ctx->device));
+    const size_t each = (size_t) width * height * chnls;
+    if (upload_lf(ctx, ctx->noisy, noisy, sai_mask, asize, each)) return 1;
+    return noise_estimate(ctx, ctx->noisy.as<float>(), sai_mask, asize, chnls, width, height, sigma, sigma_chnl, sigma_sai);
+}
+
+int lfbm5d_estimate_sigma_device(lfbm5d_ctx *ctx, const float *d_noisy, const unsigned *sai_mask, unsigned asize, unsigned chnls, unsigned width,
+                                 unsigned height, float *sigma, float *sigma_chnl, float *sigma_sai)
+{
+    if (!ctx) return fail("null argument");
+    if (validate_estimate(d_noisy, sai_mask, asize, chnls, width, height, sigma)) return 1;
+    CK(cudaSetDevice(ctx->device));
+    return noise_estimate(ctx, d_noisy, sai_mask, asize, chnls, width, height, sigma, sigma_chnl, sigma_sai);
 }
 
 unsigned lfbm5d_step_plan(const lfbm5d_params *p, const unsigned *sai_mask, unsigned *out, unsigned max_entries)

@@ -119,6 +119,26 @@ int run_bm3d_LF(const float sigma, std::vector<std::vector<float> > &LF_noisy, s
     return EXIT_SUCCESS;
 }
 
+int estimate_sigma_LF(const std::vector<std::vector<float> > &LF, const std::vector<unsigned> &mask, unsigned width, unsigned height,
+                      unsigned chnls, float *sigma, std::vector<float> *sigma_chnl, std::vector<float> *sigma_sai)
+{
+    lfbm5d_ctx *ctx = context();
+    if (!ctx) return EXIT_FAILURE;
+    const unsigned asize = (unsigned) LF.size();
+    const size_t each = (size_t) width * height * chnls;
+    if (check_sizes(LF, mask, asize, each, "LF")) return EXIT_FAILURE;
+    std::vector<float *> p(asize, nullptr);      // read only: the C ABI takes the pointer type of the step entry points
+    for (unsigned st = 0; st < asize; st++) if (mask[st]) p[st] = const_cast<float *>(LF[st].data());
+    std::vector<float> sc(chnls), ss(asize);
+    if (lfbm5d_estimate_sigma(ctx, p.data(), mask.data(), asize, chnls, width, height, sigma, sc.data(), ss.data()) != 0) {
+        std::cout << lfbm5d_last_error() << std::endl;
+        return EXIT_FAILURE;
+    }
+    if (sigma_chnl) *sigma_chnl = sc;
+    if (sigma_sai) *sigma_sai = ss;
+    return EXIT_SUCCESS;
+}
+
 // ---- C exports of the host-side noise / metric helpers of the command lines (include/lfbm5d_host_c.h) ----
 extern "C" {
 

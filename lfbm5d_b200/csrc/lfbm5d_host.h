@@ -44,3 +44,9 @@ int run_bm3d_LF(const float sigma, std::vector<std::vector<float> > &LF_noisy, s
                 const unsigned kWien, const unsigned NHard, const unsigned NWien, const unsigned pHard, const unsigned pWien,
                 const bool useSD_h, const bool useSD_w, const unsigned tau_2D_hard, const unsigned tau_2D_wien,
                 const float lambdaHard3D, const unsigned color_space, const unsigned nb_threads, char *sub_img_name);
+
+//! Noise level of a light field without ground truth (lfbm5d_estimate_sigma, include/lfbm5d_cuda.h; not in the reference): LF[st] of
+//! width*height*chnls floats (planar, as given: RGB or grey), SAIs with mask[st] == 0 ignored. *sigma pools every SAI and channel;
+//! sigma_chnl / sigma_sai, when given, receive the value per channel and per SAI (0 for masked SAIs). The input is not modified.
+int estimate_sigma_LF(const std::vector<std::vector<float> > &LF, const std::vector<unsigned> &mask, unsigned width, unsigned height,
+                      unsigned chnls, float *sigma, std::vector<float> *sigma_chnl = nullptr, std::vector<float> *sigma_sai = nullptr);

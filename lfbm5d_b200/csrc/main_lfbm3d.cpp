@@ -33,7 +33,15 @@ int main(int argc, char **argv)
     i += 2;      // asw sizes: parsed and unused by the BM3D driver
     const unsigned ang_major = pick(argv[++i], { { "row", ROWMAJOR }, { "col", COLMAJOR } });
     if (ang_major == NONE) { cout << "ang_major is not known. Choice is :" << endl << " -row" << endl << " -col" << endl; return EXIT_FAILURE; }
-    const float fSigma = atof(argv[++i]), lambdaHard3D = atof(argv[++i]);
+    // sigma = auto: estimated from the noisy light field read back from disk (estimate_sigma_LF), so only without ground truth
+    const bool sigma_auto = strcmp(argv[++i], "auto") == 0;
+    float fSigma = sigma_auto ? 0.0f : atof(argv[i]);
+    const float lambdaHard3D = atof(argv[++i]);
+    if (sigma_auto && gt_exists) {
+        cout << "sigma = auto needs LF_dir = none: with a ground-truth light field, noise of the given sigma is added to it. "
+                "Give sigma as a number, or LF_dir = none to denoise the light field in LF_dir_noisy." << endl;
+        return EXIT_FAILURE;
+    }
     const char *LF_noisy_name = argv[++i], *LF_basic_name = argv[++i], *LF_denoised_name = argv[++i], *LF_diff_name = argv[++i];
     unsigned N[2], n[2], k[2], p[2], t2[2];
     bool useSD[2];
@@ -74,6 +82,14 @@ int main(int argc, char **argv)
     const size_t whc = (size_t) width * height * chnls;
     LF_diff.assign(awh, vector<float>(whc, 0.0f)); LF_basic.assign(awh, vector<float>(whc, 0.0f)); LF_denoised.assign(awh, vector<float>(whc, 0.0f));
     for (unsigned st = 0; st < awh; st++) if (LF_noisy[st].size() != whc) LF_noisy[st].resize(whc, 0.0f);
+    if (sigma_auto) {
+        vector<float> sigma_chnl;
+        if (estimate_sigma_LF(LF_noisy, LF_SAI_mask, width, height, chnls, &fSigma, &sigma_chnl) != EXIT_SUCCESS) return EXIT_FAILURE;
+        char line[160];
+        int n = snprintf(line, sizeof(line), "Estimated noise level: sigma = %.9g (per channel:", fSigma);
+        for (float s : sigma_chnl) n += snprintf(line + n, sizeof(line) - n, " %.9g", s);
+        cout << endl << line << ")" << endl;
+    }
     vector<float> psnr_noisy, rmse_noisy, psnr_basic, rmse_basic, psnr, rmse;
     float apn = 0, arn = 0, spn = 0, srn = 0, apb = 0, arb = 0, spb = 0, srb = 0, ap = 0, ar = 0, sp = 0, sr = 0;
     if (gt_exists) {
